@@ -1,13 +1,17 @@
 #!/usr/bin/env python
 """bench.py -- guided filter Mpix/s (BASELINE.json metric) on N B200s of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 A step = one pass of the fused guided filter over one synthetic 3840x2160 float32 gray frame,
 r=8, eps=1e-2 (BASELINE.json configs[1]).  Frames rotate over 6 distinct buffer sets (597 MB,
 > the 126 MB L2) so no step finds its input in L2.  With N>1 every rank filters its own frames
 (batch sharding, no collective; weak scaling) and `value` is the sum over ranks / max time.
+
+--dump-outputs DIR writes the q plane of the last timed step (rank 0) to DIR/q.npy, float32
+3840x2160.  The frames are seeded, so two builds run with the same arguments can be compared
+output for output.
 
 JSON keys beyond the base contract:
   roofline     the fused kernel against the HBM roofline: 12 B/px algorithmic (read I, read p,
@@ -212,7 +216,12 @@ def main():
     ap.add_argument("--no-scaling", action="store_true", help="skip the config-3 / config-5 legs (scaling_configs)")
     ap.add_argument("--frames", type=int, default=256, help="config 3: frames in the batch (sharded over the ranks)")
     ap.add_argument("--giga", type=int, default=32768, help="config 5: side of the square image (sharded by row strips)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's q to DIR/q.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU path; --impl reference times a band whose height depends on its speed")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -269,6 +278,8 @@ def main():
     ev1.record(stream)
     barrier()
     t_wall1 = time.perf_counter()
+    # copied now: the steps below reuse the buffer
+    last_q = frames[(args.steps - 1) % NSETS][2].cpu().numpy() if args.dump_outputs and rank == 0 else None
     launches = api.launch_count() - n0
     kernel_name = api.last_kernel()
     ms = ev0.elapsed_time(ev1)
@@ -440,6 +451,9 @@ def main():
             line["cpu_baseline"] = {k: res[k] for k in ("value", "unit", "cores", "kind", "sample")}
         if ref_gpu:
             line["reference_gpu"] = ref_gpu
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "q.npy"), last_q)
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
