@@ -988,18 +988,12 @@ static const char* gf_ws_try(const Job& j, bool* done, const char** name)
     if (j.r == RR && (force_k == 0 || force_k == KK) && j.width >= GfWsGeom<RR, KK, NN>::WOUT && (KK % 8 != 0 || in32)) { \
         *done = true; *name = NAME; return gf_ws_launch<RR, KK, NN>(j);              \
     }
-#ifdef GF_CPU_EMU
-    GF_WS_CASE(8, 12, 4, "ws_r8_k12")
-    GF_WS_CASE(8, 8, 6, "ws_r8_k8")
-    GF_WS_CASE(4, 8, 4, "ws_r4_k8")
-    GF_WS_CASE(16, 12, 2, "ws_r16_k12")
-#else
+    // (the emulator build compiles the same list: every instantiation that ships is under its tests)
     GF_WS_CASE(8, 12, 4, "ws_r8_k12")
     GF_WS_CASE(8, 8, 6, "ws_r8_k8")
     GF_WS_CASE(7, 12, 4, "ws_r7_k12")
     GF_WS_CASE(4, 8, 6, "ws_r4_k8")
     GF_WS_CASE(16, 12, 2, "ws_r16_k12")
-#endif
 #undef GF_WS_CASE
     return nullptr;
 }

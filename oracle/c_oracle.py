@@ -71,14 +71,17 @@ def guided_gray_f32(I, p, r, eps, border=0, nthreads=1, return_ab=False):
     return (q, A, B) if return_ab else q
 
 
-def guided_gray_f64(I, p, r, eps, border=0, nthreads=1):
+def guided_gray_f64(I, p, r, eps, border=0, nthreads=1, return_ab=False):
     I = np.ascontiguousarray(I, dtype=np.float64)
     p = np.ascontiguousarray(p, dtype=np.float64)
     h, w = I.shape
     q = np.empty_like(I)
-    rc = lib().gf_oracle_guided_gray_f64(_dp(I), _dp(p), _dp(q), None, None, w, h, w, r, eps, border, nthreads)
+    A = np.empty_like(I) if return_ab else None
+    B = np.empty_like(I) if return_ab else None
+    rc = lib().gf_oracle_guided_gray_f64(_dp(I), _dp(p), _dp(q), _dp(A) if return_ab else None,
+                                         _dp(B) if return_ab else None, w, h, w, r, eps, border, nthreads)
     assert rc == 0, rc
-    return q
+    return (q, A, B) if return_ab else q
 
 
 def guided_color_f32(I3, p, r, eps, border=0, nthreads=1):

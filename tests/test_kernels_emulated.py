@@ -347,6 +347,21 @@ def test_class_run_planar_path(be, knob):
     ((200, 704), 4, 0, 8),      # r = 4: window narrower than two lanes
     ((210, 400), 16, 0, 12),    # r = 16: windows reach two lanes to either side, two streams
     ((100, 800), 16, 2, 12),
+    # r = 7 (every r = 7 a/b job, hGuidedFilter's demo call) and r = 4 (six streams), at the widths of each strip edge mode:
+    # one strip over both edges, two strips with the last one not pulled back, pulled back exactly to column 0, two
+    # overlapping strips, two whole strips, interior strips; heights at the minimum 4r+2 and around the 4-/6-stream plans
+    ((36, 352), 7, 0, 12),
+    ((35, 356), 7, 1, 12),
+    ((30, 368), 7, 2, 12),
+    ((90, 700), 7, 0, 12),
+    ((60, 704), 7, 2, 12),
+    ((50, 1064), 7, 1, 12),
+    ((34, 240), 4, 2, 8),
+    ((33, 244), 4, 0, 8),
+    ((18, 248), 4, 1, 8),
+    ((120, 476), 4, 2, 8),
+    ((60, 480), 4, 1, 8),
+    ((40, 728), 4, 0, 8),
 ])
 @pytest.mark.parametrize("split", [0, 1])
 def test_gray_ws(be, shape, r, border, k, split, knob):
@@ -355,12 +370,13 @@ def test_gray_ws(be, shape, r, border, k, split, knob):
     knob(be, "GF_WS_K", k)
     knob(be, "GF_WS_SPLIT1", split)
     I, p = synth_pair(*shape, seed=81, kind="structured")
-    q, A, B = be.guided_gray(I, p, r, 1e-2, border, want_ab=True)
+    w = shape[1]
+    q, A, B = be.guided_gray(I, p, r, 1e-2, border, want_ab=True, pad=(-w) % 8 if k % 8 == 0 else 0)   # K = 8: 32-byte rows
     assert be.api.last_kernel() == f"ws_r{r}_k{k}"
     rq, ra, rb = O.guided_filter_gray(I, p, r, 1e-2, border, np.float64, return_ab=True)
     assert np.abs(q - rq).max() <= TOL
     assert np.abs(A - ra).max() <= TOL and np.abs(B - rb).max() <= TOL
-    q2 = be.guided_gray(I, p, r, 1e-2, border)              # without the A / B planes: the same q
+    q2 = be.guided_gray(I, p, r, 1e-2, border, pad=(-w) % 8 if k % 8 == 0 else 0)      # without the A / B planes: the same q
     assert np.array_equal(q, q2)
 
 

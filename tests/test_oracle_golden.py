@@ -53,9 +53,11 @@ def test_kat_crops(crop):
                                      ((64, 48), 16), ((129, 257), 7)])
 def test_c_vs_numpy(shape, r, mode):
     I, p = synth_pair(*shape, seed=3)
-    qn = O.guided_filter_gray(I, p, r, 1e-2, mode, np.float64)
+    qn, an, bn = O.guided_filter_gray(I, p, r, 1e-2, mode, np.float64, return_ab=True)
     qc = C.guided_gray_f64(I, p, r, 1e-2, mode, nthreads=3)
     assert np.abs(qn - qc).max() < 1e-10
+    qc, ac, bc = C.guided_gray_f64(I, p, r, 1e-2, mode, nthreads=3, return_ab=True)
+    assert np.abs(qn - qc).max() < 1e-10 and np.abs(an - ac).max() < 1e-10 and np.abs(bn - bc).max() < 1e-10
     qf = C.guided_gray_f32(I, p, r, 1e-2, mode, nthreads=2)
     assert np.abs(qn - qf).max() < 2e-5
 
