@@ -22,11 +22,12 @@
 #ifdef GF_HAVE_FAST
 #include "gf_fast.cuh"
 #include "gf_wp.cuh"
-// the three big kernel families live in their own translation units (gf_tu_s8.cu, gf_tu_ws.cu, gf_tu_c4.cu) so that the
-// library builds in parallel
+// the big kernel families live in their own translation units (gf_tu_s8.cu, gf_tu_ws.cu, gf_tu_c4.cu, gf_tu_c4u8.cu) so
+// that the library builds in parallel
 const char* gf_s8_try_x(const Job& j, bool* done, const char** name, bool u8);
 const char* gf_ws_try_x(const Job& j, bool* done, const char** name);
 const char* gf_c4_try_x(const Job& j, bool* done, const char** name);
+const char* gf_c4u8_try_x(const Job& j, bool* done, const char** name);
 static inline const char* gf_s8_try(const Job& j, bool* done, const char** name, bool u8 = false) { return gf_s8_try_x(j, done, name, u8); }
 static inline const char* gf_ws_try(const Job& j, bool* done, const char** name) { return gf_ws_try_x(j, done, name); }
 static inline const char* gf_c4_try(const Job& j, bool* done, const char** name) { return gf_c4_try_x(j, done, name); }
@@ -635,6 +636,44 @@ int gf_guided_color(const float* guide3, const float* src, float* dst, int width
         js[c].dst = Plane{dst, or_packed(dst_stride, width, src_channels), 0, src_channels, c};
     }
     return run_jobs(js, src_channels);
+}
+
+int gf_guided_color_u8(const unsigned char* guide3, const unsigned char* src, unsigned char* dst, int width, int height,
+                       int src_channels, int64_t guide_stride, int64_t src_stride, int64_t dst_stride, int r, float eps,
+                       int border, void* stream)
+{
+#ifdef GF_HAVE_FAST
+    if (src_channels != 1 && src_channels != 3) return fail(GF_ERR_UNSUPPORTED, "Do not support channel: 3, %d", src_channels);
+    Job j;
+    j.count = src_channels;                 // one launch: the frames of the c4 kernel are the source channels
+    j.width = width; j.height = height; j.buf_rows = height; j.out_rows = height;
+    j.r = r; j.eps = eps; j.border = border; j.stream = stream; j.color = true;
+    // Plane carries float*: the u8 planes are reinterpreted, every stride is in ELEMENTS (= bytes here)
+    j.guide = Plane{reinterpret_cast<const float*>(guide3), or_packed(guide_stride, width, 3), 0, 3, 0};
+    j.src = Plane{reinterpret_cast<const float*>(src), or_packed(src_stride, width, src_channels), 0, src_channels, 0};
+    j.dst = Plane{reinterpret_cast<const float*>(dst), or_packed(dst_stride, width, src_channels), 0, src_channels, 0};
+    j.A = j.B = Plane{nullptr, 0, 0, 1, 0};
+    if (int rc = check_common(j)) return rc;
+    {   // any overlap of the output with an input, not just equal pointers (byte ranges: the planes hold unsigned char)
+        auto ov = [&](const unsigned char* a, int64_t sa, const unsigned char* b, int64_t sb) {
+            return a < b + (int64_t)height * sb && b < a + (int64_t)height * sa;
+        };
+        if (ov(dst, j.dst.stride, guide3, j.guide.stride) || ov(dst, j.dst.stride, src, j.src.stride))
+            return fail(GF_ERR_UNSUPPORTED, "gf_guided_color_u8: in-place filtering is not supported");
+    }
+    bool done = false;
+    const char* name = nullptr;
+    const char* e = gf_c4u8_try_x(j, &done, &name);
+    if (!done)
+        return fail(GF_ERR_UNSUPPORTED, "gf_guided_color_u8 needs r in {4,8,12,16}, width %% 4 == 0, width >= 128, height >= 4r+2, "
+                                        "rows x stride < 2^31 and 4-byte aligned planes and row strides");
+    if (e) return fail(GF_ERR_CUDA, "%s launch: %s", name, e);
+    g_launches++;
+    g_kernel = name;
+    return GF_OK;
+#else
+    return fail(GF_ERR_UNSUPPORTED, "gf_guided_color_u8: built without the tuned kernels");
+#endif
 }
 
 int gf_guided_batch(const float* guide, const float* src, float* dst, int count, int width, int height, int guide_channels,

@@ -20,6 +20,13 @@
 //     (the class API's border, guided_filter.cpp:22-60) -- rows and lanes outside the image are zeros and every
 //     mean divides by its own in-image pixel count; any other width uses the generic kernel.
 // R must be a multiple of 4 and <= 16 (M <= 4 halo lanes per side and stage).
+//
+// T = unsigned char: the same kernel on 8-bit planes (gf_guided_color_u8), in the integer domain of the gray
+// uint8 build (gf_s8.cuh): I' = 255 I and p' = 255 p are the bytes as floats 0..255, the host passes
+// eps' = 255^2 eps, and q' = 255 q is rounded and saturated by the store.  The stage-1 column sums are then
+// integers below 33 x 255^2 < 2^24, exact in float32.  A row is kept raw (3 guide words, 1 or 3 src words)
+// and expanded where it is consumed.  The frames of a launch are the source channels (count = 1 or 3,
+// frame strides 0): frame f reads and writes byte f of every interleaved src / dst pixel.
 #pragma once
 #include "gf_s8.cuh"
 
@@ -62,9 +69,9 @@ __device__ __forceinline__ void gf_c4_window(const float (&x)[4], float (&w)[4])
     w[0] = l0 + r0; w[1] = l1 + r1; w[2] = l2 + r2; w[3] = l3 + r3;
 }
 
-template <int R>
+template <int R, class T = float>
 struct GfC4Ctx {
-    const float* gI; const float* gP; float* gQ;     // frame bases at this lane's first column (gI: 3 floats per column)
+    const T* gI; const T* gP; T* gQ;                 // frame bases at this lane's first column (gI: 3 elements per column)
     int gs, ss, ds;
     float4* ring;
     int lane, x0, width, height, border, buf_y0, buf_ylast, out_y0, yi0;
@@ -77,13 +84,57 @@ struct GfC4Ctx {
     float sa[4][4];                                  // stage-2 running sums (a_r, a_g, a_b, b)
     float va[4][4];                                  // a, b of the row produced by the previous iteration
     float nI[12], nP[4], oI[12], oP[4];              // newest row / row leaving the window (= guide row of the output)
+    bool p3;                                         // uint8 only: 3-channel src / dst (gQ then points at channel ch)
+    unsigned selA, selB;                             // uint8 only: byte selectors of the src words (gf_c4_expand)
 };
+
+// Byte permute (PRMT): byte n of the result is byte (s >> 4n) & 7 of the 8 bytes y:x.
+__device__ __forceinline__ unsigned gf_prmt(unsigned x, unsigned y, unsigned s)
+{
+#ifdef GF_CPU_EMU
+    const unsigned long long v = ((unsigned long long)y << 32) | x;
+    unsigned r = 0;
+    for (int n = 0; n < 4; ++n) r |= (unsigned)((v >> (8 * ((s >> (4 * n)) & 7))) & 255u) << (8 * n);
+    return r;
+#else
+    return __byte_perm(x, y, s);
+#endif
+}
+
+// uint8 build: a raw row (vi[0..2]: the 12 guide bytes; vp[0..2]: the src words, as float bit patterns) -> floats 0..255.
+// The src pixels are gathered into one word first: 1 channel: bytes 0..3 of vp[0] (= vp[1]); 3 channels: pixel j,
+// channel ch is byte 3j + ch of the 12 bytes, i.e. byte ch, 3 + ch of (vp[0], vp[1]) and 2 + ch, 5 + ch of (vp[1], vp[2]).
+template <int R, class T>
+__device__ __forceinline__ void gf_c4_expand(const GfC4Ctx<R, T>& c, float (&vi)[12], float (&vp)[4])
+{
+    const unsigned g0 = gf_f_bits(vi[0]), g1 = gf_f_bits(vi[1]), g2 = gf_f_bits(vi[2]);
+    const unsigned w0 = gf_f_bits(vp[0]), w1 = gf_f_bits(vp[1]), w2 = gf_f_bits(vp[2]);
+    const unsigned pw = gf_prmt(gf_prmt(w0, w1, c.selA), gf_prmt(w1, w2, c.selB), 0x7610u);
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+        vi[k] = gf_u8_to_f(g0, k); vi[4 + k] = gf_u8_to_f(g1, k); vi[8 + k] = gf_u8_to_f(g2, k);
+        vp[k] = gf_u8_to_f(pw, k);
+    }
+}
 
 // Raw loads of one row: 12 guide floats (3 x LDG.128) and 4 src floats.  A lane outside the image
 // loads its mirror lane's address instead (any valid address would do) and is patched by gf_c4_mirror.
-template <int R>
-__device__ __forceinline__ void gf_c4_ld(const GfC4Ctx<R>& c, int row_ofs_I, int row_ofs_P, float (&vi)[12], float (&vp)[4])
+// uint8: 12 guide bytes (3 x LDG.32) and 4 (1 x LDG.32) or 12 src bytes, kept raw for gf_c4_expand.
+template <int R, class T>
+__device__ __forceinline__ void gf_c4_ld(const GfC4Ctx<R, T>& c, int row_ofs_I, int row_ofs_P, float (&vi)[12], float (&vp)[4])
 {
+    if constexpr (sizeof(T) == 1) {
+        const unsigned* pi = reinterpret_cast<const unsigned*>(c.gI + row_ofs_I);
+        const unsigned* pp = reinterpret_cast<const unsigned*>(c.gP + row_ofs_P);
+        vi[0] = gf_bits_f(pi[0]); vi[1] = gf_bits_f(pi[1]); vi[2] = gf_bits_f(pi[2]);
+        vp[0] = gf_bits_f(pp[0]);
+        vp[1] = vp[0]; vp[2] = 0.f;
+        if (c.p3) { vp[1] = gf_bits_f(pp[1]); vp[2] = gf_bits_f(pp[2]); }
+#pragma unroll
+        for (int i = 3; i < 12; ++i) vi[i] = 0.f;
+        vp[3] = 0.f;
+        return;
+    }
     const float4* pi = reinterpret_cast<const float4*>(c.gI + row_ofs_I);
     const float4 t0 = pi[0], t1 = pi[1], t2 = pi[2];
     const float4 tp = *reinterpret_cast<const float4*>(c.gP + row_ofs_P);
@@ -97,8 +148,8 @@ __device__ __forceinline__ void gf_c4_ld(const GfC4Ctx<R>& c, int row_ofs_I, int
 //   right: column W+4m+j <- column W-2-4m-j = {col2, col1, col0 of lane s1(=s0), col3 of lane s2}
 // REFLECT (edge pixel repeated): column -4k+j <- 4k-1-j and W+4m+j <- W-1-4m-j: the four columns of ONE lane (s0), reversed.
 // TRUNCATE: zeros.  A warp overhangs at most one side (width >= 128), so all its lanes publish that side's pattern.
-template <int R, int BM>
-__device__ __forceinline__ void gf_c4_mirror(const GfC4Ctx<R>& c, float (&vi)[12], float (&vp)[4], bool zero_row = false)
+template <int R, int BM, class T>
+__device__ __forceinline__ void gf_c4_mirror(const GfC4Ctx<R, T>& c, float (&vi)[12], float (&vp)[4], bool zero_row = false)
 {
     const unsigned full = 0xffffffffu;
     const bool out = c.out_l || c.out_r;
@@ -143,8 +194,8 @@ __device__ __forceinline__ void gf_c4_mirror(const GfC4Ctx<R>& c, float (&vi)[12
 
 // Returns true when the row stands for zeros (TRUNCATE, row outside the image or past the resident rows): the loads are
 // issued anyway, from a clamped row, so that the load schedule has no branch; gf_c4_mirror<.., 2> clears the values.
-template <int R, bool MIRROR, int BM>
-__device__ __forceinline__ bool gf_c4_load_row(const GfC4Ctx<R>& c, int y, float (&vi)[12], float (&vp)[4])
+template <int R, bool MIRROR, int BM, class T>
+__device__ __forceinline__ bool gf_c4_load_row(const GfC4Ctx<R, T>& c, int y, float (&vi)[12], float (&vp)[4])
 {
     int rn = BM == 2 ? (y < 0 ? 0 : y) : gf_s8_map_y(y, c.height, c.border);
     const bool zero = BM == 2 && (y < 0 || y > c.buf_ylast);
@@ -168,13 +219,14 @@ __device__ __forceinline__ void gf_c4_accum(float (&c)[13][4], int j, float i0, 
 }
 
 // Iteration t >= 2R (see gf_s8_iter for the schedule: ramp-up is data, not code).
-template <int R, bool MIRROR, int BM>
-__device__ __forceinline__ void gf_c4_iter(GfC4Ctx<R>& c, int t, int slot, bool full)
+template <int R, bool MIRROR, int BM, class T>
+__device__ __forceinline__ void gf_c4_iter(GfC4Ctx<R, T>& c, int t, int slot, bool full)
 {
     using G = GfC4Geom<R>;
     constexpr int KW = G::KW, VL = G::VL;
     const int yi = c.yi0 + t;
 
+    if constexpr (sizeof(T) == 1) { gf_c4_expand(c, c.nI, c.nP); gf_c4_expand(c, c.oI, c.oP); }
     if (MIRROR || BM == 2) { gf_c4_mirror<R, BM>(c, c.nI, c.nP, c.nz); gf_c4_mirror<R, BM>(c, c.oI, c.oP, c.oz); }
     // ---- stage 1, vertical: add row yi, drop row yi - KW (its guide pixels are kept for the output)
     float gI[12];
@@ -218,7 +270,20 @@ __device__ __forceinline__ void gf_c4_iter(GfC4Ctx<R>& c, int t, int slot, bool 
                 const float v = fmaf(c.sa[0][j], gI[3 * j], fmaf(c.sa[1][j], gI[3 * j + 1], fmaf(c.sa[2][j], gI[3 * j + 2], c.sa[3][j])));
                 qv[j] = v * (BM == 2 ? c.icx[j] * icy : inv);
             }
-            if (c.out_lane) *reinterpret_cast<float4*>(c.gQ + (yo - c.out_y0) * c.ds) = make_float4(qv[0], qv[1], qv[2], qv[3]);
+            if (c.out_lane) {
+                T* q = c.gQ + (yo - c.out_y0) * c.ds;
+                if constexpr (sizeof(T) == 1) {             // q' = 255 q: round half to even, saturate
+                    if (c.p3) {                             // byte stores: the other channels are other warps' frames
+#pragma unroll
+                        for (int j = 0; j < 4; ++j) q[3 * j] = (unsigned char)gf_f_to_u8(qv[j]);
+                    } else {
+                        *reinterpret_cast<unsigned*>(q) =
+                            gf_f_to_u8(qv[0]) | (gf_f_to_u8(qv[1]) << 8) | (gf_f_to_u8(qv[2]) << 16) | (gf_f_to_u8(qv[3]) << 24);
+                    }
+                } else {
+                    *reinterpret_cast<float4*>(q) = make_float4(qv[0], qv[1], qv[2], qv[3]);
+                }
+            }
         }
     }
 
@@ -253,8 +318,8 @@ __device__ __forceinline__ void gf_c4_iter(GfC4Ctx<R>& c, int t, int slot, bool 
     }
 }
 
-template <int R, bool MIRROR, int BM>
-__device__ __forceinline__ void gf_c4_band(GfC4Ctx<R>& c, int steps)
+template <int R, bool MIRROR, int BM, class T>
+__device__ __forceinline__ void gf_c4_band(GfC4Ctx<R, T>& c, int steps)
 {
     constexpr int KW = 2 * R + 1;
     // warm-up rows t in [0, 2R): vertical accumulation only; rows are loaded four at a time so that
@@ -268,6 +333,7 @@ __device__ __forceinline__ void gf_c4_band(GfC4Ctx<R>& c, int steps)
             for (int k = 0; k < 4; ++k) bz[k] = gf_c4_load_row<R, MIRROR, BM>(c, c.yi0 + t + 1 + k, bI[k], bP[k]);
 #pragma unroll
             for (int k = 0; k < 4; ++k) {
+                if constexpr (sizeof(T) == 1) gf_c4_expand(c, c.nI, c.nP);
                 if (MIRROR || BM == 2) gf_c4_mirror<R, BM>(c, c.nI, c.nP, c.nz);
                 c.nz = bz[k];
 #pragma unroll
@@ -290,14 +356,14 @@ __device__ __forceinline__ void gf_c4_band(GfC4Ctx<R>& c, int steps)
     }
 }
 
-template <int R, int MINB, int BM>
+template <int R, int MINB, int BM, class T = float>
 __global__ void __launch_bounds__(32, MINB) gf_c4_color_kernel(const GF_GRID_CONSTANT GfWpArgs a)
 {
     using G = GfC4Geom<R>;
     constexpr int M = G::M, VL = G::VL;
     GF_DYN_SMEM(float, smem);
     auto run = [&](int64_t f, int strip, int yo0, int yo1) {
-    GfC4Ctx<R> c;
+    GfC4Ctx<R, T> c;
     c.lane = threadIdx.x & 31;
     const int xl = strip * G::WOUT - 2 * M * 4;
     c.x0 = xl + 4 * c.lane;
@@ -322,7 +388,18 @@ __global__ void __launch_bounds__(32, MINB) gf_c4_color_kernel(const GF_GRID_CON
     }
     // lanes outside the image load from a valid address (their mirror lane's); the data is replaced
     const int xa = (c.out_l || c.out_r) ? 4 * c.s0 + xl : c.x0;
-    c.gI = a.guide + f * a.gfs + (int64_t)3 * xa; c.gP = a.src + f * a.sfs + xa; c.gQ = a.dst + f * a.dfs + c.x0;
+    // (GfWpArgs carries the planes as float*; the uint8 build reinterprets them, strides are in elements)
+    const int pch = sizeof(T) == 1 ? a.count : 1;   // interleaved src / dst channels: uint8 frames are the channels
+    c.gI = reinterpret_cast<const T*>(a.guide) + f * a.gfs + (int64_t)3 * xa;
+    c.gP = reinterpret_cast<const T*>(a.src) + f * a.sfs + (int64_t)pch * xa;
+    c.gQ = reinterpret_cast<T*>(a.dst) + f * a.dfs + (int64_t)pch * c.x0;
+    if constexpr (sizeof(T) == 1) {
+        const unsigned ch = (unsigned)f;
+        c.p3 = pch == 3;
+        c.gQ += c.p3 ? ch : 0u;
+        c.selA = c.p3 ? ch | (3 + ch) << 4 : 0x3210u;
+        c.selB = c.p3 ? (2 + ch) << 8 | (5 + ch) << 12 : 0x3210u;
+    }
     c.gs = (int)a.gs; c.ss = (int)a.ss; c.ds = (int)a.ds;
     c.ring_lane = c.lane >= 2 * M && c.lane < 32 - 2 * M;
     c.out_lane = c.ring_lane && c.x0 < a.width;
@@ -364,7 +441,7 @@ __global__ void __launch_bounds__(32, MINB) gf_c4_color_kernel(const GF_GRID_CON
 
 // ---- host side ------------------------------------------------------------------------------------
 #ifndef GF_NO_HOST   // (stand-alone SASS builds of one kernel define GF_NO_HOST)
-template <int R>
+template <int R, class T>
 static const char* gf_c4_launch(const Job& j)
 {
     using G = GfC4Geom<R>;
@@ -376,7 +453,8 @@ static const char* gf_c4_launch(const Job& j)
     a.gs = j.guide.stride; a.ss = j.src.stride; a.ds = j.dst.stride; a.abs_ = 0;
     a.gfs = j.guide.frame_stride; a.sfs = j.src.frame_stride; a.dfs = j.dst.frame_stride; a.abfs = 0;
     a.width = j.width; a.height = j.height; a.buf_y0 = j.buf_y0; a.buf_rows = j.buf_rows; a.out_y0 = j.out_y0;
-    a.out_rows = j.out_rows; a.border = j.border; a.eps = j.eps; a.count = j.count;
+    a.out_rows = j.out_rows; a.border = j.border; a.count = j.count;
+    a.eps = sizeof(T) == 1 ? j.eps * 65025.0f : j.eps;       // uint8 build: integer domain, eps scales with 255^2
     a.tape_piece = 0; a.tape_rho = 0; a.tape_we = 100;
     a.nstrips = (j.width + G::WOUT - 1) / G::WOUT;
     a.hb_e = 0; a.nbands_e = 0;
@@ -409,29 +487,42 @@ static const char* gf_c4_launch(const Job& j)
         GF_LAUNCH(k, grid, block, smem, j.stream, a);
         return gf_rt_launch_error();
     };
-    if (j.border == GF_REFLECT) return go(gf_c4_color_kernel<R, MINB, 1>);
-    if (j.border == GF_TRUNCATE) return go(gf_c4_color_kernel<R, MINB, 2>);
-    return go(gf_c4_color_kernel<R, MINB, 0>);
+    if (j.border == GF_REFLECT) return go(gf_c4_color_kernel<R, MINB, 1, T>);
+    if (j.border == GF_TRUNCATE) return go(gf_c4_color_kernel<R, MINB, 2, T>);
+    return go(gf_c4_color_kernel<R, MINB, 0, T>);
 }
 
+// T = unsigned char (gf_guided_color_u8): the planes hold unsigned char (Plane::ptr reinterpreted, strides in
+// elements), the frames are the src_channels (1 or 3) interleaved source channels: count = src.channels = dst.channels,
+// every frame stride 0.  Each kernel family is instantiated in its own translation unit (gf_tu_c4.cu, gf_tu_c4u8.cu).
+template <class T>
 static const char* gf_c4_try(const Job& j, bool* done, const char** name)
 {
+    constexpr bool u8 = sizeof(T) == 1;
     *done = false;
     if (!j.color || j.A.ptr) return nullptr;
     if (j.border != GF_REFLECT101 && j.border != GF_REFLECT && j.border != GF_TRUNCATE) return nullptr;
-    if (GF_KNOB("GF_DISABLE_C4", 0) || GF_KNOB("GF_DISABLE_FAST", 0)) return nullptr;
-    if (j.guide.channels != 3 || j.guide.coff != 0 || j.src.channels != 1 || j.src.coff != 0 || j.dst.channels != 1 || j.dst.coff != 0)
-        return nullptr;
     const Plane* pl[3] = {&j.guide, &j.src, &j.dst};
-    for (int i = 0; i < 3; ++i)
-        if ((pl[i]->stride & 3) || (pl[i]->frame_stride & 3) || ((uintptr_t)pl[i]->ptr & 15)) return nullptr;
+    if (u8) {
+        if (j.guide.channels != 3 || (j.count != 1 && j.count != 3) || j.src.channels != j.count || j.dst.channels != j.count)
+            return nullptr;
+        for (int i = 0; i < 3; ++i)
+            if (pl[i]->coff != 0 || pl[i]->frame_stride != 0 || (pl[i]->stride & 3) || ((uintptr_t)pl[i]->ptr & 3)) return nullptr;
+        if ((int64_t)j.buf_rows * j.src.stride >= (1ll << 31)) return nullptr;
+    } else {
+        if (GF_KNOB("GF_DISABLE_C4", 0) || GF_KNOB("GF_DISABLE_FAST", 0)) return nullptr;
+        if (j.guide.channels != 3 || j.guide.coff != 0 || j.src.channels != 1 || j.src.coff != 0 || j.dst.channels != 1 || j.dst.coff != 0)
+            return nullptr;
+        for (int i = 0; i < 3; ++i)
+            if ((pl[i]->stride & 3) || (pl[i]->frame_stride & 3) || ((uintptr_t)pl[i]->ptr & 15)) return nullptr;
+    }
     if ((j.width & 3) || j.width < 128 || j.height < 4 * j.r + 2) return nullptr;
     if ((int64_t)j.buf_rows * j.guide.stride >= (1ll << 31) || (int64_t)j.out_rows * j.dst.stride >= (1ll << 31)) return nullptr;
     switch (j.r) {
-    case 4: *done = true; *name = "c4_r4"; return gf_c4_launch<4>(j);
-    case 8: *done = true; *name = "c4_r8"; return gf_c4_launch<8>(j);
-    case 12: *done = true; *name = "c4_r12"; return gf_c4_launch<12>(j);
-    case 16: *done = true; *name = "c4_r16"; return gf_c4_launch<16>(j);
+    case 4: *done = true; *name = u8 ? "c4u8_r4" : "c4_r4"; return gf_c4_launch<4, T>(j);
+    case 8: *done = true; *name = u8 ? "c4u8_r8" : "c4_r8"; return gf_c4_launch<8, T>(j);
+    case 12: *done = true; *name = u8 ? "c4u8_r12" : "c4_r12"; return gf_c4_launch<12, T>(j);
+    case 16: *done = true; *name = u8 ? "c4u8_r16" : "c4_r16"; return gf_c4_launch<16, T>(j);
     default: return nullptr;
     }
 }

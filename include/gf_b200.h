@@ -204,6 +204,16 @@ int gf_guided_gray_u8(const unsigned char* guide, const unsigned char* src, unsi
                       int64_t guide_stride, int64_t src_stride, int64_t dst_stride, int r, float eps, int border,
                       void* stream);
 
+/* The colour-guide filter of gf_guided_color on 8-bit planes (a CV_8UC3 guide; a CV_8UC1 or CV_8UC3 source and
+   destination of `src_channels` interleaved channels), with the same fused conversions: the input is x/255, the output
+   saturate_cast<uchar>(cvRound(255 q)), eps on the [0,1] scale.  Strides in ELEMENTS (= bytes), 0 = tightly packed.
+   One launch of the c4 kernel for 1 or 3 source channels.  Served by that kernel only: r in {4, 8, 12, 16},
+   width % 4 == 0, width >= 128, height >= 4r+2, rows x stride < 2^31, every plane's base address and row stride
+   4-byte aligned, dst overlapping neither input; other arguments return GF_ERR_UNSUPPORTED. */
+int gf_guided_color_u8(const unsigned char* guide3, const unsigned char* src, unsigned char* dst, int width, int height,
+                       int src_channels, int64_t guide_stride, int64_t src_stride, int64_t dst_stride,
+                       int r, float eps, int border, void* stream);
+
 /* ---- Integral/ module (SURVEY 8(f) rank 1): summed-area table of a uint8 image ----------------
    Replace hIntegral / hAligned4Integral (Integral/integral_d.h:5-8, integral_d.cu:863-930):
    integral[y*dst_stride + x] = sum of src over rows <= y and columns <= x (inclusive, W x H).
