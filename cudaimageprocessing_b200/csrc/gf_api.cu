@@ -17,6 +17,7 @@
 #include "gf_pointwise.cuh"
 #include "gf_integral.cuh"
 #include "gf_gauss.cuh"
+#include "gf_fgf.cuh"
 #include "gf_scan.cuh"
 #include "gf_rt.h"
 #ifdef GF_HAVE_FAST
@@ -37,6 +38,7 @@ namespace {
 
 thread_local std::string g_err;
 thread_local const char* g_kernel = "none";
+thread_local std::string g_kernel_fgf;       // "fgf/<low-res kernel>", the name gf_fast_guided_gray reports
 std::atomic<int64_t> g_launches{0};
 
 int fail(gf_status s, const char* fmt, ...)
@@ -1066,6 +1068,126 @@ int gf_box_filter(const float* src, float* dst, int width, int height, int chann
     g_launches++;
     g_kernel = "box";
     return GF_OK;
+}
+
+// Fast guided filter (He & Sun 2015; gf_fgf.cuh): a and b solved on I and p subsampled s times with radius r/s by the
+// library's own gray a/b job, mean_a and mean_b by the box kernel, the bilinear upsample fused into q = mean_a*I + mean_b.
+int gf_fast_guided_gray(const float* guide, const float* src, float* dst, int width, int height, int64_t guide_stride,
+                        int64_t src_stride, int64_t dst_stride, int r, float eps, int s, int border, void* stream)
+{
+    if (!guide || !src || !dst) return fail(GF_ERR_INVALID, "gf_fast_guided_gray: null pointer");
+    if (width <= 0 || height <= 0) return fail(GF_ERR_INVALID, "gf_fast_guided_gray: non-positive size %dx%d", width, height);
+    const int64_t gs = or_packed(guide_stride, width, 1), ss = or_packed(src_stride, width, 1), ds = or_packed(dst_stride, width, 1);
+    if (gs < width || ss < width || ds < width) return fail(GF_ERR_INVALID, "gf_fast_guided_gray: row stride smaller than a row");
+    if (s < 1 || s > GF_FGF_MAX_S) return fail(GF_ERR_INVALID, "gf_fast_guided_gray: subsampling factor s = %d outside [1, %d]", s, GF_FGF_MAX_S);
+    if (r < 0 || r % s != 0)
+        return fail(GF_ERR_INVALID, "gf_fast_guided_gray: r = %d must be a non-negative multiple of s = %d (the low-res radius is r/s)", r, s);
+    if (!(eps >= 0.f)) return fail(GF_ERR_INVALID, "gf_fast_guided_gray: eps must be >= 0");
+    if (border < 0 || border > 2) return fail(GF_ERR_INVALID, "gf_fast_guided_gray: unknown border mode %d", border);
+    // dst may BE an input (same pointer and stride): every full-resolution pass writes only the pixels it has just read.
+    // Planes that share a row stride may interleave their rows (columns side by side) without sharing a pixel.
+    auto partial = [&](const float* in, int64_t is) {
+        if (in == dst && is == ds) return false;
+        if (!(dst < in + (int64_t)(height - 1) * is + width && in < dst + (int64_t)(height - 1) * ds + width)) return false;
+        if (is != ds) return true;
+        const int64_t c = (((intptr_t)dst - (intptr_t)in) / (int64_t)sizeof(float) % is + is) % is;   // column offset
+        return !(c >= width && c + width <= is);
+    };
+    if (partial(guide, gs) || partial(src, ss))
+        return fail(GF_ERR_UNSUPPORTED, "gf_fast_guided_gray: dst overlaps an input without being exactly that input (same pointer and stride)");
+
+    // the low-res a/b job, refused here if run_job would refuse it: the streaming kernels plan it, or the scan path takes it
+    const int ws = div_up(width, s), hs = div_up(height, s), rl = r / s;
+    const int64_t pitch = round_up(ws, 4);                   // 16-byte rows
+    Job lo;
+    lo.width = ws; lo.height = hs; lo.buf_rows = hs; lo.out_rows = hs;
+    lo.r = rl; lo.eps = eps; lo.border = border; lo.stream = stream;
+    lo.guide = lo.src = lo.dst = lo.A = lo.B = Plane{nullptr, pitch, 0, 1, 0};
+    {
+        GenericCfg c;
+        if (plan_generic(lo, 4 * rl, 4 * rl, GfGrayModel::NQ1 + GfGrayModel::NQ2, GfGrayModel::NQ2, &c) != GF_OK && !scan_ok(lo))
+            return fail(GF_ERR_UNSUPPORTED, "gf_fast_guided_gray: no kernel runs the %dx%d low-res job at radius r/s = %d with border %d "
+                                            "(a reflecting border needs r/s below both low-res dimensions at this radius)", ws, hs, rl, border);
+    }
+    if (s == 1) {                                            // the exact filter
+        Job j;
+        j.width = width; j.height = height; j.buf_rows = height; j.out_rows = height;
+        j.r = r; j.eps = eps; j.border = border; j.stream = stream;
+        j.guide = Plane{guide, gs, 0, 1, 0};
+        j.src = Plane{src, ss, 0, 1, 0};
+        j.dst = Plane{dst, ds, 0, 1, 0};
+        j.A = j.B = Plane{nullptr, 0, 0, 1, 0};
+        const int rc = run_jobs(&j, 1);
+        if (rc == GF_OK) { g_kernel_fgf = std::string("fgf/") + g_kernel; g_kernel = g_kernel_fgf.c_str(); }
+        return rc;
+    }
+
+    const size_t plane = (size_t)pitch * hs;
+    void* scratch = nullptr;
+    if (const char* e = gf_rt_alloc_async(&scratch, 5 * plane * sizeof(float), stream))
+        return fail(GF_ERR_NOMEM, "gf_fast_guided_gray: low-res scratch (%zu bytes): %s", 5 * plane * sizeof(float), e);
+    float* Is = (float*)scratch;                             // I_s, then mean_a
+    float* ps = Is + plane;                                  // p_s, then mean_b
+    float* A = ps + plane, *B = A + plane, *Q = B + plane;   // a, b and the low-res q the a/b job also writes
+    int rc = GF_OK;
+    {
+        GfFgfDownArgs a;
+        a.I = guide; a.p = src; a.Is = Is; a.ps = ps; a.si = gs; a.sp = ss; a.sl = pitch;
+        a.width = width; a.height = height; a.ws = ws; a.hs = hs; a.s = s;
+        dim3 grid(div_up(ws, GF_FGF_DOWN_THREADS), hs < 65535 ? hs : 65535), block(GF_FGF_DOWN_THREADS);
+        auto k = gf_fgf_down_kernel;
+        GF_LAUNCH(k, grid, block, 0, stream, a);
+        if (const char* e = gf_rt_launch_error()) rc = fail(GF_ERR_CUDA, "gf_fgf_down_kernel launch: %s", e);
+        else g_launches++;
+    }
+    const char* lo_name = "none";
+    if (rc == GF_OK) {
+        lo.guide.ptr = Is; lo.src.ptr = ps; lo.dst.ptr = Q; lo.A.ptr = A; lo.B.ptr = B;
+        rc = run_job(lo);
+        lo_name = g_kernel;
+    }
+    // mean_a, mean_b: gf_box_kernel on CTAs of 128 columns and bands short enough for 16 CTAs per SM.  A CTA waits for
+    // one row load per step, so its time is (hb + 2r) load latencies: gf_box_filter's own plan (one strip of up to 1024
+    // columns, bands of at least 16 rows) measured 19-22 us a plane at 4K s = 4 and 46-58 us at 8K s = 4.  Radii that
+    // leave fewer than 32 columns go through gf_box_filter.
+    auto box = [&](const float* in, float* out) -> int {
+        const int win = 128, wc = win - 2 * rl;
+        if (wc < 32) return gf_box_filter(in, out, ws, hs, 1, pitch, pitch, rl, border, stream);
+        Job jb = lo;
+        jb.src = jb.guide = Plane{in, pitch, 0, 1, 0};
+        jb.dst = Plane{out, pitch, 0, 1, 0};
+        jb.A = jb.B = Plane{nullptr, 0, 0, 1, 0};
+        GfArgs a = mk_args(jb);
+        int sms = 148, mj = 0, mn = 0;
+        gf_rt_device_info(&sms, &mj, &mn);
+        const int nstrips = div_up(ws, wc);
+        const int hb = div_up(hs, div_up(16 * sms, nstrips));
+        a.wc = wc; a.hb = hb;
+        dim3 grid(nstrips, div_up(hs, hb), 1), block(win);
+        auto k = gf_box_kernel<1>;
+        GF_LAUNCH(k, grid, block, (win + 32) * sizeof(float), stream, a);
+        if (const char* e = gf_rt_launch_error()) return fail(GF_ERR_CUDA, "gf_box_kernel launch: %s", e);
+        g_launches++;
+        return GF_OK;
+    };
+    // I_s and p_s have been read by the a/b job (stream order): they take mean_a and mean_b
+    if (rc == GF_OK) rc = box(A, Is);
+    if (rc == GF_OK) rc = box(B, ps);
+    if (rc == GF_OK) {
+        GfFgfApplyArgs a;
+        a.I = guide; a.q = dst; a.ma = Is; a.mb = ps; a.si = gs; a.sq = ds; a.sl = pitch;
+        a.width = width; a.height = height; a.ws = ws; a.hs = hs; a.s = s;
+        const bool vec = width % 4 == 0 && gs % 4 == 0 && ds % 4 == 0 && !((uintptr_t)guide & 15) && !((uintptr_t)dst & 15);
+        const int ty = div_up(height, GF_FGF_TY);
+        dim3 grid(div_up(width, GF_FGF_TX), ty < 65535 ? ty : 65535), block(256);
+        if (vec) { auto k = gf_fgf_up_apply_kernel<true>; GF_LAUNCH(k, grid, block, 0, stream, a); }
+        else { auto k = gf_fgf_up_apply_kernel<false>; GF_LAUNCH(k, grid, block, 0, stream, a); }
+        if (const char* e = gf_rt_launch_error()) rc = fail(GF_ERR_CUDA, "gf_fgf_up_apply_kernel launch: %s", e);
+        else g_launches++;
+    }
+    gf_rt_free_async(scratch, stream);
+    if (rc == GF_OK) { g_kernel_fgf = std::string("fgf/") + lo_name; g_kernel = g_kernel_fgf.c_str(); }
+    return rc;
 }
 
 static int pointwise(int op, const float* i0, const float* i1, const float* i2, const float* i3, float* out, int width,

@@ -82,6 +82,26 @@ int gf_guided_gray(const float* guide, const float* src, float* dst, float* A, f
                    int64_t dst_stride, int64_t ab_stride, int r, float eps, int border,
                    void* stream);
 
+/* Fast guided filter (He & Sun, "Fast Guided Filter", arXiv:1505.00996): gray guide, gray source, float32, any
+   width, height, stride and alignment.  An approximation of gf_guided_gray whose full-resolution cost does not grow
+   with the radius: with hs = ceil(height/s), ws = ceil(width/s),
+     - I_s, p_s: the mean of the in-image pixels of every s x s block (only the last row and column of blocks can be
+       partial);
+     - mean_a, mean_b: the gray guided filter of gf_guided_gray on (I_s, p_s) at radius r/s, with eps and border, up to
+       its box means of a and b;
+     - q = up(mean_a) * I + up(mean_b), up = bilinear with half-pixel centres and replicated edges:
+       u = clamp((x + 0.5)/s - 0.5, 0, ws - 1), and the same for y.
+   s = 1 is gf_guided_gray.  dst may be exactly the guide or the source (same pointer and stride): in place without a
+   temporary.  Strides in floats, 0 = tightly packed.  Low-res scratch comes from the library's stream-ordered pool.
+   GF_ERR_INVALID: a null pointer, a non-positive size, a stride smaller than a row, s outside [1, 32], r < 0 or r not a
+   multiple of s, eps < 0, an unknown border.  GF_ERR_UNSUPPORTED: dst overlapping an input without being exactly it,
+   or a low-res job no kernel of gf_guided_gray runs (a reflecting border with a radius r/s that is not below both
+   low-res dimensions and too large for the streaming kernels).  Every refusal comes before anything is launched.
+   gf_last_kernel() gives "fgf/<kernel of the low-res job>". */
+int gf_fast_guided_gray(const float* guide, const float* src, float* dst, int width, int height,
+                        int64_t guide_stride, int64_t src_stride, int64_t dst_stride,
+                        int r, float eps, int s, int border, void* stream);
+
 /* Colour guide (3 interleaved channels), `src_channels` (1 or 3) source/destination channels.
    a = (Sigma + eps U)^-1 cov(I, p), b = mean(p) - a.mean(I), q = mean(a).I + mean(b). */
 int gf_guided_color(const float* guide3, const float* src, float* dst, int width, int height,
