@@ -20,6 +20,7 @@ SIGNATURES = {
     "gf_guided_gray": (c_int, [P, P, P, P, P, c_int, c_int, c_int64, c_int64, c_int64, c_int64, c_int, c_float, c_int, P]),
     "gf_guided_color": (c_int, [P, P, P, c_int, c_int, c_int, c_int64, c_int64, c_int64, c_int, c_float, c_int, P]),
     "gf_fast_guided_gray": (c_int, [P, P, P, c_int, c_int, c_int64, c_int64, c_int64, c_int, c_float, c_int, c_int, P]),
+    "gf_fast_guided_gray_u8": (c_int, [P, P, P, c_int, c_int, c_int64, c_int64, c_int64, c_int, c_float, c_int, c_int, P]),
     "gf_guided_batch": (c_int, [P, P, P, c_int, c_int, c_int, c_int, c_int64, c_int64, c_int64, c_int64, c_int64, c_int64,
                                 c_int, c_float, c_int, P]),
     "gf_guided_gray_strip": (c_int, [P, P, P, c_int, c_int, c_int, c_int, c_int, c_int, c_int64, c_int64, c_int64,

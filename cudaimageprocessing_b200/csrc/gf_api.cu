@@ -38,7 +38,7 @@ namespace {
 
 thread_local std::string g_err;
 thread_local const char* g_kernel = "none";
-thread_local std::string g_kernel_fgf;       // "fgf/<low-res kernel>", the name gf_fast_guided_gray reports
+thread_local std::string g_kernel_fgf;       // "fgf/<low-res kernel>" ("fgf_u8/..."), the name gf_fast_guided_gray(_u8) reports
 std::atomic<int64_t> g_launches{0};
 
 int fail(gf_status s, const char* fmt, ...)
@@ -1070,72 +1070,81 @@ int gf_box_filter(const float* src, float* dst, int width, int height, int chann
     return GF_OK;
 }
 
+}  // extern "C"
+
 // Fast guided filter (He & Sun 2015; gf_fgf.cuh): a and b solved on I and p subsampled s times with radius r/s by the
 // library's own gray a/b job, mean_a and mean_b by the box kernel, the bilinear upsample fused into q = mean_a*I + mean_b.
-int gf_fast_guided_gray(const float* guide, const float* src, float* dst, int width, int height, int64_t guide_stride,
-                        int64_t src_stride, int64_t dst_stride, int r, float eps, int s, int border, void* stream)
+// T = float: gf_fast_guided_gray; T = unsigned char: gf_fast_guided_gray_u8, in the integer domain (eps' = 255^2 eps, the
+// low-res planes hold 0..255; gf_fgf.cuh).  Strides are in elements.
+template <typename T>
+static int fast_guided_gray(const T* guide, const T* src, T* dst, int width, int height, int64_t guide_stride,
+                            int64_t src_stride, int64_t dst_stride, int r, float eps, int s, int border, void* stream,
+                            const char* fn, const char* tag)
 {
-    if (!guide || !src || !dst) return fail(GF_ERR_INVALID, "gf_fast_guided_gray: null pointer");
-    if (width <= 0 || height <= 0) return fail(GF_ERR_INVALID, "gf_fast_guided_gray: non-positive size %dx%d", width, height);
+    constexpr bool u8 = sizeof(T) == 1;
+    if (!guide || !src || !dst) return fail(GF_ERR_INVALID, "%s: null pointer", fn);
+    if (width <= 0 || height <= 0) return fail(GF_ERR_INVALID, "%s: non-positive size %dx%d", fn, width, height);
     const int64_t gs = or_packed(guide_stride, width, 1), ss = or_packed(src_stride, width, 1), ds = or_packed(dst_stride, width, 1);
-    if (gs < width || ss < width || ds < width) return fail(GF_ERR_INVALID, "gf_fast_guided_gray: row stride smaller than a row");
-    if (s < 1 || s > GF_FGF_MAX_S) return fail(GF_ERR_INVALID, "gf_fast_guided_gray: subsampling factor s = %d outside [1, %d]", s, GF_FGF_MAX_S);
+    if (gs < width || ss < width || ds < width) return fail(GF_ERR_INVALID, "%s: row stride smaller than a row", fn);
+    if (u8 && s == 1)
+        return fail(GF_ERR_INVALID, "%s: s = 1 is the exact filter, whose 8-bit entry is gf_guided_gray_u8", fn);
+    if (s < 1 || s > GF_FGF_MAX_S) return fail(GF_ERR_INVALID, "%s: subsampling factor s = %d outside [%d, %d]", fn, s, u8 ? 2 : 1, GF_FGF_MAX_S);
     if (r < 0 || r % s != 0)
-        return fail(GF_ERR_INVALID, "gf_fast_guided_gray: r = %d must be a non-negative multiple of s = %d (the low-res radius is r/s)", r, s);
-    if (!(eps >= 0.f)) return fail(GF_ERR_INVALID, "gf_fast_guided_gray: eps must be >= 0");
-    if (border < 0 || border > 2) return fail(GF_ERR_INVALID, "gf_fast_guided_gray: unknown border mode %d", border);
+        return fail(GF_ERR_INVALID, "%s: r = %d must be a non-negative multiple of s = %d (the low-res radius is r/s)", fn, r, s);
+    if (!(eps >= 0.f)) return fail(GF_ERR_INVALID, "%s: eps must be >= 0", fn);
+    if (border < 0 || border > 2) return fail(GF_ERR_INVALID, "%s: unknown border mode %d", fn, border);
     // dst may BE an input (same pointer and stride): every full-resolution pass writes only the pixels it has just read.
     // Planes that share a row stride may interleave their rows (columns side by side) without sharing a pixel.
-    auto partial = [&](const float* in, int64_t is) {
+    auto partial = [&](const T* in, int64_t is) {
         if (in == dst && is == ds) return false;
         if (!(dst < in + (int64_t)(height - 1) * is + width && in < dst + (int64_t)(height - 1) * ds + width)) return false;
         if (is != ds) return true;
-        const int64_t c = (((intptr_t)dst - (intptr_t)in) / (int64_t)sizeof(float) % is + is) % is;   // column offset
+        const int64_t c = (((intptr_t)dst - (intptr_t)in) / (int64_t)sizeof(T) % is + is) % is;   // column offset
         return !(c >= width && c + width <= is);
     };
     if (partial(guide, gs) || partial(src, ss))
-        return fail(GF_ERR_UNSUPPORTED, "gf_fast_guided_gray: dst overlaps an input without being exactly that input (same pointer and stride)");
+        return fail(GF_ERR_UNSUPPORTED, "%s: dst overlaps an input without being exactly that input (same pointer and stride)", fn);
 
     // the low-res a/b job, refused here if run_job would refuse it: the streaming kernels plan it, or the scan path takes it
     const int ws = div_up(width, s), hs = div_up(height, s), rl = r / s;
     const int64_t pitch = round_up(ws, 4);                   // 16-byte rows
     Job lo;
     lo.width = ws; lo.height = hs; lo.buf_rows = hs; lo.out_rows = hs;
-    lo.r = rl; lo.eps = eps; lo.border = border; lo.stream = stream;
+    lo.r = rl; lo.eps = u8 ? eps * 65025.0f : eps; lo.border = border; lo.stream = stream;
     lo.guide = lo.src = lo.dst = lo.A = lo.B = Plane{nullptr, pitch, 0, 1, 0};
     {
         GenericCfg c;
         if (plan_generic(lo, 4 * rl, 4 * rl, GfGrayModel::NQ1 + GfGrayModel::NQ2, GfGrayModel::NQ2, &c) != GF_OK && !scan_ok(lo))
-            return fail(GF_ERR_UNSUPPORTED, "gf_fast_guided_gray: no kernel runs the %dx%d low-res job at radius r/s = %d with border %d "
-                                            "(a reflecting border needs r/s below both low-res dimensions at this radius)", ws, hs, rl, border);
+            return fail(GF_ERR_UNSUPPORTED, "%s: no kernel runs the %dx%d low-res job at radius r/s = %d with border %d "
+                                            "(a reflecting border needs r/s below both low-res dimensions at this radius)", fn, ws, hs, rl, border);
     }
-    if (s == 1) {                                            // the exact filter
+    if (s == 1) {                                            // the exact filter (float only: s = 1 is refused above for u8)
         Job j;
         j.width = width; j.height = height; j.buf_rows = height; j.out_rows = height;
         j.r = r; j.eps = eps; j.border = border; j.stream = stream;
-        j.guide = Plane{guide, gs, 0, 1, 0};
-        j.src = Plane{src, ss, 0, 1, 0};
-        j.dst = Plane{dst, ds, 0, 1, 0};
+        j.guide = Plane{reinterpret_cast<const float*>(guide), gs, 0, 1, 0};
+        j.src = Plane{reinterpret_cast<const float*>(src), ss, 0, 1, 0};
+        j.dst = Plane{reinterpret_cast<const float*>(dst), ds, 0, 1, 0};
         j.A = j.B = Plane{nullptr, 0, 0, 1, 0};
         const int rc = run_jobs(&j, 1);
-        if (rc == GF_OK) { g_kernel_fgf = std::string("fgf/") + g_kernel; g_kernel = g_kernel_fgf.c_str(); }
+        if (rc == GF_OK) { g_kernel_fgf = std::string(tag) + g_kernel; g_kernel = g_kernel_fgf.c_str(); }
         return rc;
     }
 
     const size_t plane = (size_t)pitch * hs;
     void* scratch = nullptr;
     if (const char* e = gf_rt_alloc_async(&scratch, 5 * plane * sizeof(float), stream))
-        return fail(GF_ERR_NOMEM, "gf_fast_guided_gray: low-res scratch (%zu bytes): %s", 5 * plane * sizeof(float), e);
+        return fail(GF_ERR_NOMEM, "%s: low-res scratch (%zu bytes): %s", fn, 5 * plane * sizeof(float), e);
     float* Is = (float*)scratch;                             // I_s, then mean_a
     float* ps = Is + plane;                                  // p_s, then mean_b
     float* A = ps + plane, *B = A + plane, *Q = B + plane;   // a, b and the low-res q the a/b job also writes
     int rc = GF_OK;
     {
-        GfFgfDownArgs a;
+        GfFgfDownArgs<T> a;
         a.I = guide; a.p = src; a.Is = Is; a.ps = ps; a.si = gs; a.sp = ss; a.sl = pitch;
         a.width = width; a.height = height; a.ws = ws; a.hs = hs; a.s = s;
         dim3 grid(div_up(ws, GF_FGF_DOWN_THREADS), hs < 65535 ? hs : 65535), block(GF_FGF_DOWN_THREADS);
-        auto k = gf_fgf_down_kernel;
+        auto k = gf_fgf_down_kernel<T>;
         GF_LAUNCH(k, grid, block, 0, stream, a);
         if (const char* e = gf_rt_launch_error()) rc = fail(GF_ERR_CUDA, "gf_fgf_down_kernel launch: %s", e);
         else g_launches++;
@@ -1174,20 +1183,38 @@ int gf_fast_guided_gray(const float* guide, const float* src, float* dst, int wi
     if (rc == GF_OK) rc = box(A, Is);
     if (rc == GF_OK) rc = box(B, ps);
     if (rc == GF_OK) {
-        GfFgfApplyArgs a;
+        GfFgfApplyArgs<T> a;
         a.I = guide; a.q = dst; a.ma = Is; a.mb = ps; a.si = gs; a.sq = ds; a.sl = pitch;
         a.width = width; a.height = height; a.ws = ws; a.hs = hs; a.s = s;
-        const bool vec = width % 4 == 0 && gs % 4 == 0 && ds % 4 == 0 && !((uintptr_t)guide & 15) && !((uintptr_t)dst & 15);
+        const uintptr_t al = 4 * sizeof(T) - 1;             // 4 pixels per access: 16 bytes (float), 4 bytes (u8)
+        const bool vec = width % 4 == 0 && gs % 4 == 0 && ds % 4 == 0 && !((uintptr_t)guide & al) && !((uintptr_t)dst & al);
         const int ty = div_up(height, GF_FGF_TY);
         dim3 grid(div_up(width, GF_FGF_TX), ty < 65535 ? ty : 65535), block(256);
-        if (vec) { auto k = gf_fgf_up_apply_kernel<true>; GF_LAUNCH(k, grid, block, 0, stream, a); }
-        else { auto k = gf_fgf_up_apply_kernel<false>; GF_LAUNCH(k, grid, block, 0, stream, a); }
+        if (vec) { auto k = gf_fgf_up_apply_kernel<true, T>; GF_LAUNCH(k, grid, block, 0, stream, a); }
+        else { auto k = gf_fgf_up_apply_kernel<false, T>; GF_LAUNCH(k, grid, block, 0, stream, a); }
         if (const char* e = gf_rt_launch_error()) rc = fail(GF_ERR_CUDA, "gf_fgf_up_apply_kernel launch: %s", e);
         else g_launches++;
     }
     gf_rt_free_async(scratch, stream);
-    if (rc == GF_OK) { g_kernel_fgf = std::string("fgf/") + lo_name; g_kernel = g_kernel_fgf.c_str(); }
+    if (rc == GF_OK) { g_kernel_fgf = std::string(tag) + lo_name; g_kernel = g_kernel_fgf.c_str(); }
     return rc;
+}
+
+extern "C" {
+
+int gf_fast_guided_gray(const float* guide, const float* src, float* dst, int width, int height, int64_t guide_stride,
+                        int64_t src_stride, int64_t dst_stride, int r, float eps, int s, int border, void* stream)
+{
+    return fast_guided_gray(guide, src, dst, width, height, guide_stride, src_stride, dst_stride, r, eps, s, border, stream,
+                            "gf_fast_guided_gray", "fgf/");
+}
+
+int gf_fast_guided_gray_u8(const unsigned char* guide, const unsigned char* src, unsigned char* dst, int width, int height,
+                           int64_t guide_stride, int64_t src_stride, int64_t dst_stride, int r, float eps, int s, int border,
+                           void* stream)
+{
+    return fast_guided_gray(guide, src, dst, width, height, guide_stride, src_stride, dst_stride, r, eps, s, border, stream,
+                            "gf_fast_guided_gray_u8", "fgf_u8/");
 }
 
 static int pointwise(int op, const float* i0, const float* i1, const float* i2, const float* i3, float* out, int width,

@@ -22,6 +22,30 @@ static inline void gf_prefetch_l2(const void*) {}
 __device__ __forceinline__ void gf_prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
 #endif
 
+// ---- uint8 planes in the integer domain (gf_s8.cuh, gf_c4.cuh, gf_fgf.cuh): a byte is loaded as the float 0..255 and
+// q' = 255 q is stored as saturate_cast<uchar>(cvRound(q')) ------------------------------------------------------------
+__device__ __forceinline__ float gf_u8_to_f(unsigned word, int k)   // byte k of word as a float, no I2F:
+{                                                                   // 0x4B0000bb is the float 8388608 + bb
+#ifdef GF_CPU_EMU
+    return (float)((word >> (8 * k)) & 255u);
+#else
+    return __uint_as_float(__byte_perm(word, 0x4B000000u, 0x7650 + k)) - 8388608.0f;
+#endif
+}
+__device__ __forceinline__ unsigned gf_f_to_u8(float q255)
+{
+#ifdef GF_CPU_EMU
+    const int r = (int)std::nearbyint(q255);
+#else
+    const int r = __float2int_rn(q255);                // cvRound: round half to even
+#endif
+    return (unsigned)(r < 0 ? 0 : (r > 255 ? 255 : r));   // saturate_cast<uchar>
+}
+__device__ __forceinline__ float gf_ld1(const float* p) { return *p; }
+__device__ __forceinline__ float gf_ld1(const unsigned char* p) { return (float)*p; }
+__device__ __forceinline__ void gf_st1(float* p, float v) { *p = v; }
+__device__ __forceinline__ void gf_st1(unsigned char* p, float v) { *p = (unsigned char)gf_f_to_u8(v); }
+
 #define GF_REFLECT101 0
 #define GF_TRUNCATE 1
 #define GF_REFLECT 2

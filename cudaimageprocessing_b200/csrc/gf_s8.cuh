@@ -94,28 +94,8 @@ __device__ __forceinline__ void gf_st8(float* p, const float2 (&v)[4])
 // rounds, and eps becomes 255^2 eps -- so neither conversion costs an operation.  Better than free: the
 // vertical running sums of I', p', I'p', I'I' are integers below 2^24, i.e. EXACT in float32 (no drift,
 // no re-seed), and so are the lane prefixes of the window sums; only sums above 2^24 (17 x 17 x 255^2
-// = 1.9e7) round, by at most one part in 2^24.
-__device__ __forceinline__ float gf_u8_to_f(unsigned word, int k)   // byte k of word as a float, no I2F:
-{                                                                   // 0x4B0000bb is the float 8388608 + bb
-#ifdef GF_CPU_EMU
-    return (float)((word >> (8 * k)) & 255u);
-#else
-    return __uint_as_float(__byte_perm(word, 0x4B000000u, 0x7650 + k)) - 8388608.0f;
-#endif
-}
-__device__ __forceinline__ unsigned gf_f_to_u8(float q255)
-{
-#ifdef GF_CPU_EMU
-    const int r = (int)std::nearbyint(q255);
-#else
-    const int r = __float2int_rn(q255);                // cvRound: round half to even
-#endif
-    return (unsigned)(r < 0 ? 0 : (r > 255 ? 255 : r));   // saturate_cast<uchar>
-}
-__device__ __forceinline__ float gf_ld1(const float* p) { return *p; }
-__device__ __forceinline__ float gf_ld1(const unsigned char* p) { return (float)*p; }
-__device__ __forceinline__ void gf_st1(float* p, float v) { *p = v; }
-__device__ __forceinline__ void gf_st1(unsigned char* p, float v) { *p = (unsigned char)gf_f_to_u8(v); }
+// = 1.9e7) round, by at most one part in 2^24.  The byte conversions themselves (gf_u8_to_f, gf_f_to_u8,
+// gf_ld1, gf_st1) are in gf_common.cuh: the fast guided filter's uint8 build uses them too.
 __device__ __forceinline__ float gf_bits_f(unsigned u)
 {
 #ifdef GF_CPU_EMU

@@ -102,6 +102,17 @@ int gf_fast_guided_gray(const float* guide, const float* src, float* dst, int wi
                         int64_t guide_stride, int64_t src_stride, int64_t dst_stride,
                         int r, float eps, int s, int border, void* stream);
 
+/* The fast guided filter of gf_fast_guided_gray on 8-bit gray planes (CV_8UC1), with the conversions fused into its two
+   full-resolution kernels: the input is x/255, the output saturate_cast<uchar>(cvRound(255 q)) (round half to even), eps
+   on the [0,1] scale.  2 bytes of HBM traffic per pixel in each full-resolution kernel instead of 8, and no conversion
+   passes around the call.  Any width, height, stride and base alignment; strides in ELEMENTS (= bytes), 0 = tightly
+   packed.  dst may be exactly the guide or the source (same pointer and stride).  s in [2, 32] (s = 1 is the exact
+   filter: gf_guided_gray_u8), r a multiple of s.  Refusals as gf_fast_guided_gray's, before anything is launched.
+   gf_last_kernel() gives "fgf_u8/<kernel of the low-res job>". */
+int gf_fast_guided_gray_u8(const unsigned char* guide, const unsigned char* src, unsigned char* dst, int width, int height,
+                           int64_t guide_stride, int64_t src_stride, int64_t dst_stride, int r, float eps, int s, int border,
+                           void* stream);
+
 /* Colour guide (3 interleaved channels), `src_channels` (1 or 3) source/destination channels.
    a = (Sigma + eps U)^-1 cov(I, p), b = mean(p) - a.mean(I), q = mean(a).I + mean(b). */
 int gf_guided_color(const float* guide3, const float* src, float* dst, int width, int height,
