@@ -69,37 +69,52 @@ def make_inputs(h, w, kind, seed):
     return synth_pair(h, w, seed=seed, kind=kind)
 
 
-def _guarded(h, w, s, fill=None):
-    big = np.full((h + 2 * GUARD, s), np.nan, np.float32)
+def _frames(big, n, h):
+    """the (n, h + GUARD, stride) view of a guarded allocation: every frame followed by its GUARD rows"""
+    return big[GUARD:].reshape(n, h + GUARD, big.shape[1])
+
+
+def _guarded(n, h, w, s, fill=None):
+    big = np.full((GUARD + n * (h + GUARD), s), np.nan, np.float32)
     if fill is not None:
-        big[GUARD:GUARD + h, :w] = fill
+        _frames(big, n, h)[:, :h, :w] = fill
     return big
 
 
 def run_guarded(be, I, p, r, eps, border, want_ab=True, in_pad=4, dst_pad=4, ab_pad=12):
     """gf_guided_gray on planes inside NaN-filled allocations: GUARD rows above and below, `*_pad` floats of NaN after
     every row (guide and source, q, and the a / b planes each have their own row stride).  Asserts that every guard is
-    still NaN and that q, A and B are finite inside the image; returns (q, A, B), A and B None without them."""
-    h, w = I.shape
+    still NaN and that q, A and B are finite inside the image; returns (q, A, B), A and B None without them.
+    I and p of shape (n, h, w) are a batch for gf_guided_batch (no a / b planes): frame k + 1 starts GUARD NaN rows
+    after the end of frame k, and q comes back with the same shape."""
+    batch = I.ndim == 3
+    assert not (batch and want_ab), "gf_guided_batch has no a / b planes"
+    Ib, pb = (I, p) if batch else (I[None], p[None])
+    n, h, w = Ib.shape
     si, sd, sab = w + in_pad, w + dst_pad, w + ab_pad
-    host = [_guarded(h, w, si, I), _guarded(h, w, si, p), _guarded(h, w, sd)]
+    host = [_guarded(n, h, w, si, Ib), _guarded(n, h, w, si, pb), _guarded(n, h, w, sd)]
     strides = [si, si, sd]
     if want_ab:
-        host += [_guarded(h, w, sab), _guarded(h, w, sab)]
+        host += [_guarded(n, h, w, sab), _guarded(n, h, w, sab)]
         strides += [sab, sab]
     dev = [be.up(b) for b in host]
     ptrs = [be.ptr(d) + GUARD * s * 4 for d, s in zip(dev, strides)] + [None] * (5 - len(dev))
-    be.api.call("gf_guided_gray", *ptrs, w, h, si, si, sd, sab if want_ab else 0, r, eps, border, None)
+    if batch:
+        fs, fd = (h + GUARD) * si, (h + GUARD) * sd
+        be.api.call("gf_guided_batch", *ptrs[:3], n, w, h, 1, si, si, sd, fs, fs, fd, r, eps, border, None)
+    else:
+        be.api.call("gf_guided_gray", *ptrs, w, h, si, si, sd, sab if want_ab else 0, r, eps, border, None)
     be.sync()
     out = []
     for d, plane in zip(dev, "IpqAB"):
         b = be.down(d)
-        assert np.isnan(b[:GUARD]).all() and np.isnan(b[GUARD + h:]).all() and np.isnan(b[GUARD:GUARD + h, w:]).all(), \
-            f"plane {plane}: a guard was written ({be.api.last_kernel()}, {h}x{w}, r={r}, border={border})"
+        f = _frames(b, n, h)
+        assert np.isnan(b[:GUARD]).all() and np.isnan(f[:, h:]).all() and np.isnan(f[:, :h, w:]).all(), \
+            f"plane {plane}: a guard was written ({be.api.last_kernel()}, {n}x{h}x{w}, r={r}, border={border})"
         if plane in "qAB":
-            v = b[GUARD:GUARD + h, :w]
-            assert np.isfinite(v).all(), f"plane {plane}: non-finite inside the image ({be.api.last_kernel()}, {h}x{w}, r={r}, border={border})"
-            out.append(v)
+            v = f[:, :h, :w]
+            assert np.isfinite(v).all(), f"plane {plane}: non-finite inside the image ({be.api.last_kernel()}, {n}x{h}x{w}, r={r}, border={border})"
+            out.append(v if batch else v[0])
     return tuple(out) if want_ab else (out[0], None, None)
 
 
@@ -198,12 +213,17 @@ def test_ws_long_sub_bands_do_not_drift(be, knob, name):
 
 
 def test_ws_64bit_addressing(be):
+    check_64bit_addressing(be, 8, "ws_r8_k12")
+
+
+def check_64bit_addressing(be, r, name):
     """Five planes side by side in ONE allocation of 300 rows x 2^23 floats (10 GB): every plane spans more than 2^31
-    floats, so a 32-bit row offset anywhere in the kernel breaks this test.  The columns between the planes are NaN."""
+    floats, so a 32-bit row offset anywhere in the kernel breaks this test.  The columns between the planes are NaN.
+    Runs with and without the a / b planes, both through kernel `name`."""
     import torch
     if torch.cuda.mem_get_info()[0] < 12 << 30:
         pytest.skip("needs 12 GB of free device memory")
-    h, s, w, r = 300, 1 << 23, 4 * 352, 8
+    h, s, w = 300, 1 << 23, 4 * 352
     cols = [i * (w + 36) for i in range(5)]                # I, p, q, A, B
     I, p = synth_pair(h, w, seed=64)
     rq, ra, rb = C.guided_gray_f64(I, p, r, 1e-2, 0, NT, return_ab=True)
@@ -218,11 +238,11 @@ def test_ws_64bit_addressing(be):
             be.api.call("gf_guided_gray", ptr[0], ptr[1], ptr[2], ptr[3] if want_ab else None, ptr[4] if want_ab else None,
                         w, h, s, s, s, s if want_ab else 0, r, 1e-2, 0, None)
             torch.cuda.synchronize()
-            assert be.api.last_kernel() == "ws_r8_k12"
+            assert be.api.last_kernel() == name
             assert int((~torch.isnan(big)).sum()) == 5 * h * w        # nothing written outside the five planes
             q, A, B = (big[:, c:c + w].cpu().numpy() for c in cols[2:])
             eq, ea, eb = np.abs(q - rq).max(), np.abs(A - ra).max(), np.abs(B - rb).max()
-            print(f"64-bit offsets, A/B={want_ab}: kernel ws_r8_k12; |q - f64| {eq:.2e}, |a - f64| {ea:.2e}, |b - f64| {eb:.2e}")
+            print(f"64-bit offsets, A/B={want_ab}: kernel {name}; |q - f64| {eq:.2e}, |a - f64| {ea:.2e}, |b - f64| {eb:.2e}")
             assert eq <= Q_TOL and ea <= AB_TOL and eb <= AB_TOL
     finally:
         del big

@@ -121,7 +121,11 @@ def test_errors_are_loud(be):
 # ---- the tuned kernel (gf_fast.cuh) under the emulator -------------------------------------------
 @pytest.mark.parametrize("border", [0, 1, 2])
 @pytest.mark.parametrize("shape,r", [((20, 64), 1), ((24, 100), 2), ((30, 40), 3), ((20, 520), 4), ((26, 36), 5),
-                                     ((20, 48), 6), ((40, 133), 7), ((40, 600), 8), ((30, 64), 12), ((44, 500), 16)])
+                                     ((20, 48), 6), ((40, 133), 7), ((40, 600), 8), ((30, 64), 12), ((44, 500), 16),
+                                     # r = 9..15 (80 and 64 output columns per strip): several strips, partial last strip and
+                                     # lane, rows reflected more than once (r = 11, 14); r = 10 with interior warps
+                                     ((30, 184), 9), ((110, 216), 10), ((20, 240), 11), ((60, 64), 13), ((25, 133), 14),
+                                     ((66, 196), 15)])
 def test_gray_fast(be, shape, r, border, knob):
     knob(be, "GF_DISABLE_S8", 1)
     _gray_fast(be, shape, r, border)
@@ -145,6 +149,13 @@ def test_gray_fast_ab_batch_strip(be, knob):
     assert be.api.last_kernel() == "wp_r4"
     rq, ra, rb = O.guided_filter_gray(I, p, 4, 0.05, 0, np.float64, return_ab=True)
     assert np.abs(q - rq).max() <= 1e-5 and np.abs(A - ra).max() <= 1e-4 and np.abs(B - rb).max() <= 1e-4
+    # a / b at a radius the ws kernel lacks, and through the CTA-wide kernel's global-memory ring
+    for shape, r, border in (((40, 180), 11, 2), ((60, 700), 24, 1)):
+        I, p = synth_pair(*shape, seed=r, kind="structured")
+        q, A, B = be.guided_gray(I, p, r, 0.05, border, want_ab=True)
+        assert be.api.last_kernel() == (f"wp_r{r}" if r <= 16 else f"fast_r{r}")
+        rq, ra, rb = O.guided_filter_gray(I, p, r, 0.05, border, np.float64, return_ab=True)
+        assert np.abs(q - rq).max() <= 1e-5 and np.abs(A - ra).max() <= 1e-4 and np.abs(B - rb).max() <= 1e-4
     rng = np.random.default_rng(8)
     Ib = rng.random((3, 20, 36), dtype=np.float32)
     pb = rng.random((3, 20, 36), dtype=np.float32)
@@ -173,11 +184,12 @@ def test_kat_crop_u8_fast(be, knob):
 
 
 @pytest.mark.parametrize("shape,r,border", [((24, 1452), 4, 0), ((120, 400), 8, 1), ((90, 400), 7, 2), ((70, 360), 3, 0),
-                                            ((60, 1100), 16, 0), ((90, 1500), 20, 0)])
+                                            ((60, 1100), 16, 0), ((90, 1500), 20, 0), ((130, 1300), 24, 1), ((140, 1000), 32, 2)])
 def test_gray_fast_steady_path(be, shape, r, border, knob):
     knob(be, "GF_DISABLE_S8", 1)
     """wide enough for a CTA strictly inside the image and tall enough for the straight-line
-    steady-state loop (interior rows, 128-bit loads, constant normalisation) to run."""
+    steady-state loop (interior rows, 128-bit loads, constant normalisation) to run.  r = 24 and 32
+    keep their stage-2 ring in global memory (it does not fit shared memory)."""
     I, p = synth_pair(*shape, seed=51)
     q = be.guided_gray(I, p, r, 1e-2, border)
     assert be.api.last_kernel() == (f"wp_r{r}" if r <= 16 else f"fast_r{r}")
@@ -438,6 +450,32 @@ def test_run_strips_exchange_behind_the_kernel(be, border, knob):
     q1 = be.run_strips(I, p, 3, 4, 1e-2, border)
     assert be.api.launch_count() - n0 == 3
     assert np.abs(q - q1).max() <= 1e-5          # different band boundaries: running sums round differently
+
+
+def test_run_strips_destination_right_before_the_guide(be, knob):
+    """A strip's destination holds its own rows, its guide buffer 2r halo rows more on either side.  A destination that
+    ends where the guide buffer begins (one allocation) does not overlap it: the strip is still split into the main
+    job and two seam jobs, without an in-place temporary.  (The overlap test used to give the destination the buffer's
+    row count, so whether the split happened depended on where the allocator put the planes.)"""
+    from cudaimageprocessing_b200._capi import StripPeer
+    import ctypes
+    knob(be, "GF_STRIP_OVERLAP", 1)
+    knob(be, "GF_STRIP_MIN_MAIN_ROWS", 16)
+    H, w, r, border = 240, 512, 4, 2
+    y0, rows, t = 80, 80, 8                      # the middle strip of three; t = 2r halo rows above and below
+    I, p = synth_pair(H, w, seed=94, kind="structured")
+    block = be.empty((rows + t + rows + t, w))   # q, then the guide buffer; halo rows NaN until the pull
+    q, gbuf = block[:rows], block[rows:]
+    sbuf = be.empty((t + rows + t, w))
+    gbuf[t:t + rows], sbuf[t:t + rows] = I[y0:y0 + rows], p[y0:y0 + rows]
+    own = [be.up(a) for a in (I[:y0], p[:y0], I[y0 + rows - t:], p[y0 + rows - t:])]
+    up = StripPeer(be.ptr(own[0]), be.ptr(own[1]), w, w, 0, y0)
+    dn = StripPeer(be.ptr(own[2]), be.ptr(own[3]), w, w, t, H - y0 - rows)
+    n0 = be.api.launch_count()
+    be.api.call("gf_run_strips", be.ptr(gbuf), be.ptr(sbuf), be.ptr(q), w, H, y0, rows, w, w, w, r, 1e-2, border,
+                ctypes.byref(up), ctypes.byref(dn), None)
+    assert be.api.launch_count() - n0 == 3       # main + 2 seams; the emulator's pull is a memcpy
+    assert np.abs(q - O.guided_filter_gray(I, p, r, 1e-2, border, np.float64)[y0:y0 + rows]).max() <= TOL
 
 
 def test_run_strips_rejects_short_neighbours(be):
