@@ -19,7 +19,9 @@
 //     their a/b rows across the sub-band boundaries through the rings (a stream's first R rows pre-populate
 //     its partner's window, its last R rows complete its other neighbour's), so a band pays the 4R-row ramp
 //     once per CTA (at its two outer ends) instead of once per warp: only the 2R cheap vertical warm-up
-//     rows (loads + adds) remain per stream.
+//     rows (loads + adds) remain per stream;
+//   * where it fits (GfWsGeom::TMEM), a producer keeps its last 2R+1 input rows in tensor memory and reads the row that
+//     leaves its vertical window back from there: per row it loads only the entering row from L2.
 // Hand-off: monotonic row counters in shared memory (st.release / ld.acquire at CTA scope, nanosleep
 // back-off); the ring has 2R+2 rows, a producer waits only when its consumer is a full row behind.
 // Numerics: additions only inside a window (prefix + suffix, no subtraction of prefixes); the vertical
@@ -72,6 +74,15 @@ struct GfWsGeom {
     static constexpr size_t ctrl_bytes = 64 + (size_t)NS * NBAR * 8;      // 2 NS row counters + the mbarriers
     static constexpr size_t smem_bytes = (size_t)NS * ring_bytes + (ctrl_bytes + 127) / 128 * 128;
     static constexpr int MIN_SUB = R + 1;                // shortest sub-band whose neighbours can share rows with it
+    // The producer's last 2R+1 input rows (K columns of I, then K of p) in tensor memory, so that the leaving row comes
+    // back from there instead of L2.  A warp reaches only the 32 lanes of quarter warp % 4: producers k and k + 4 share
+    // one, side by side in its 512 columns.  Kernels whose history does not fit re-read the leaving row, and so do the
+    // K = 8 ones: their leaving row is two 256-bit loads, no more instructions than the LDTM + STTM that would replace them
+    // (measured at 4K r = 4 with a / b: 0.7 % slower with the history; profiles/r3_ws_tmem_ab_with_r4.jsonl).
+    static constexpr int TM_ROW = 2 * K;                 // columns of one input row
+    static constexpr int TM_COLS = (NS + 3) / 4 * KW * TM_ROW;
+    static constexpr bool TMEM = TM_COLS <= 512 && K % 8 != 0;
+    static constexpr int TM_ALLOC = TM_COLS <= 32 ? 32 : TM_COLS <= 64 ? 64 : TM_COLS <= 128 ? 128 : TM_COLS <= 256 ? 256 : 512;
 };
 
 // ---- hand-off primitives --------------------------------------------------------------------------
@@ -133,6 +144,88 @@ __device__ __forceinline__ void gf_ws_bar_wait(const unsigned long long* b, int 
         ::"r"(addr), "r"((unsigned)(phase & 1)) : "memory");
 }
 #endif
+
+// ---- tensor memory (tcgen05) ------------------------------------------------------------------------
+// Allocation by one whole warp (the address goes to shared memory), 32x32b accesses: lane i of the warp reaches TMEM
+// lane (taddr >> 16) + i, one 32-bit column per register.  A load's registers are valid after gf_tm_wait_ld.
+#ifdef GF_CPU_EMU
+#include "tmem_emu.h"          // (tests/emu: the emulator's model of a CTA's tensor memory)
+static inline void gf_tm_alloc(unsigned* dst, int ncols) { emu::tmem_alloc(dst, ncols); }
+static inline void gf_tm_dealloc(unsigned taddr, int ncols) { emu::tmem_dealloc(taddr, ncols); }
+static inline void gf_tm_st8(unsigned taddr, const float* v) { emu::tmem_st(taddr, 8, v); }
+static inline void gf_tm_st16(unsigned taddr, const float* v) { emu::tmem_st(taddr, 16, v); }
+static inline void gf_tm_ld8(unsigned taddr, float* v) { emu::tmem_ld(taddr, 8, v); }
+static inline void gf_tm_ld16(unsigned taddr, float* v) { emu::tmem_ld(taddr, 16, v); }
+static inline void gf_tm_wait_st() {}
+template <int K> static inline void gf_tm_wait_ld(float (&)[K], float (&)[K]) {}
+static inline void gf_tm_fence_before() {}
+static inline void gf_tm_fence_after() {}
+#else
+__device__ __forceinline__ void gf_tm_alloc(unsigned* dst, int ncols)
+{
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"((unsigned)__cvta_generic_to_shared(dst)), "r"(ncols) : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+}
+__device__ __forceinline__ void gf_tm_dealloc(unsigned taddr, int ncols)
+{
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
+}
+__device__ __forceinline__ void gf_tm_st8(unsigned taddr, const float* v)
+{
+    asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};"
+                 ::"r"(taddr), "f"(v[0]), "f"(v[1]), "f"(v[2]), "f"(v[3]), "f"(v[4]), "f"(v[5]), "f"(v[6]), "f"(v[7]) : "memory");
+}
+__device__ __forceinline__ void gf_tm_st16(unsigned taddr, const float* v)
+{
+    asm volatile("tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};"
+                 ::"r"(taddr), "f"(v[0]), "f"(v[1]), "f"(v[2]), "f"(v[3]), "f"(v[4]), "f"(v[5]), "f"(v[6]), "f"(v[7]),
+                 "f"(v[8]), "f"(v[9]), "f"(v[10]), "f"(v[11]), "f"(v[12]), "f"(v[13]), "f"(v[14]), "f"(v[15]) : "memory");
+}
+__device__ __forceinline__ void gf_tm_ld8(unsigned taddr, float* v)
+{
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
+                 : "=f"(v[0]), "=f"(v[1]), "=f"(v[2]), "=f"(v[3]), "=f"(v[4]), "=f"(v[5]), "=f"(v[6]), "=f"(v[7]) : "r"(taddr) : "memory");
+}
+__device__ __forceinline__ void gf_tm_ld16(unsigned taddr, float* v)
+{
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
+                 : "=f"(v[0]), "=f"(v[1]), "=f"(v[2]), "=f"(v[3]), "=f"(v[4]), "=f"(v[5]), "=f"(v[6]), "=f"(v[7]),
+                   "=f"(v[8]), "=f"(v[9]), "=f"(v[10]), "=f"(v[11]), "=f"(v[12]), "=f"(v[13]), "=f"(v[14]), "=f"(v[15]) : "r"(taddr) : "memory");
+}
+__device__ __forceinline__ void gf_tm_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
+// waits for the loads and ties their registers to the wait, so that no use of them is scheduled above it
+template <int K>
+__device__ __forceinline__ void gf_tm_wait_ld(float (&a)[K], float (&b)[K])
+{
+    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+#pragma unroll
+    for (int j = 0; j < K; ++j) asm volatile("" : "+f"(a[j]), "+f"(b[j]));
+}
+__device__ __forceinline__ void gf_tm_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
+__device__ __forceinline__ void gf_tm_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
+#endif
+// one input row of the producer's history: K columns of I, then K of p
+template <int K>
+__device__ __forceinline__ void gf_tm_st_row(unsigned taddr, const float (&vi)[K], const float (&vp)[K])
+{
+    float v[2 * K];
+#pragma unroll
+    for (int j = 0; j < K; ++j) { v[j] = vi[j]; v[K + j] = vp[j]; }
+#pragma unroll
+    for (int c = 0; c + 16 <= 2 * K; c += 16) gf_tm_st16(taddr + c, v + c);
+    if constexpr (2 * K % 16 != 0) gf_tm_st8(taddr + 2 * K / 16 * 16, v + 2 * K / 16 * 16);
+}
+template <int K>
+__device__ __forceinline__ void gf_tm_ld_row(unsigned taddr, float (&vi)[K], float (&vp)[K])
+{
+    float v[2 * K];
+#pragma unroll
+    for (int c = 0; c + 16 <= 2 * K; c += 16) gf_tm_ld16(taddr + c, v + c);
+    if constexpr (2 * K % 16 != 0) gf_tm_ld8(taddr + 2 * K / 16 * 16, v + 2 * K / 16 * 16);
+#pragma unroll
+    for (int j = 0; j < K; ++j) { vi[j] = v[j]; vp[j] = v[K + j]; }
+}
+
 __device__ __forceinline__ void gf_ws_wait(const volatile int* ctr, int need)
 {
     while (gf_ws_ld_acq(ctr) < need) gf_ws_pause();
@@ -318,12 +411,15 @@ __host__ __device__ inline void gf_ws_plan(int y0, int y1, int pen, GfWsPlan<NS>
 // each with half the dependent chain): warp 2 owns Y = (sum Ip, sum II), its window sums go into the ring slot of the
 // row (the slot is free by then); warp 1 owns X = (sum I, sum p), picks the Y sums up from the slot, solves for a, b
 // and overwrites the slot with them.
+// tm: this producer's history in tensor memory (ROLE 0 of the kernels with G::TMEM): input row t of the stream sits
+// in slot (t - t_first) mod (2R+1), where the row that leaves 2R+1 iterations later is read back.
 template <int R, int K, int NS, bool TRUNC, int EM, int ROLE>
 __device__ __forceinline__ void gf_ws_stage1(const GfWsArgs& a, const GfWsPlan<NS>& pl, int k, int lane, int64_t f, int xl,
-                                             int out_lo, int out_hi, float4* rings, volatile int* ctrl)
+                                             int out_lo, int out_hi, float4* rings, volatile int* ctrl, unsigned tm)
 {
     using G = GfWsGeom<R, K, NS>;
     constexpr int RING = G::RING, KW = G::KW;
+    constexpr bool HIST = ROLE == 0 && G::TMEM;
     const GfWsStream st = pl.s[k];
     float4* ring = rings + (size_t)k * RING * G::ROW_F4 + lane;
     const int x0 = xl + lane * K;
@@ -460,6 +556,7 @@ __device__ __forceinline__ void gf_ws_stage1(const GfWsArgs& a, const GfWsPlan<N
 #pragma unroll
             for (int q = 0; q < CH; ++q) {
                 if (t0 + q >= t_end) break;
+                if (HIST) gf_tm_st_row<K>(tm + (t0 + q - t_first) * G::TM_ROW, bI[q], bP[q]);
 #pragma unroll
                 for (int j = 0; j < K; ++j) {
                     if (ROLE != 2) { X[j].x += bI[q][j]; X[j].y += bP[q][j]; }
@@ -480,7 +577,8 @@ __device__ __forceinline__ void gf_ws_stage1(const GfWsArgs& a, const GfWsPlan<N
 #pragma unroll
         for (int j = 0; j < K; ++j) oI[j] = oP[j] = 0.f;
     }
-    // running pointers (simple streams): the rows of iteration m0 -- entering row m0+R, leaving row m0-R-1 (not used)
+    // running pointers (simple streams): the rows of iteration m0 -- entering row m0+R and, without the tensor-memory
+    // history, leaving row m0-R-1 (not used)
     const int64_t stepI = (int64_t)st.d * a.gs, stepP = (int64_t)st.d * a.ss;
     const float* pnI = gIx + (int64_t)(rbase + st.d * (st.m0 + R)) * a.gs;
     const float* pnP = gPx + (int64_t)(rbase + st.d * (st.m0 + R)) * a.ss;
@@ -501,6 +599,7 @@ __device__ __forceinline__ void gf_ws_stage1(const GfWsArgs& a, const GfWsPlan<N
     const int n_last = st.L - 1 + R;
     const int n_last_sp = st.sp >= 0 ? pl.s[st.sp].L - 1 + R : 0;
     int slot = 0;
+    int hslot = 0;                   // history slot of row m-R, the row that leaves in iteration m+1
 
 #pragma unroll 1
     for (int m = st.m0; m < st.m1; ++m) {
@@ -521,6 +620,7 @@ __device__ __forceinline__ void gf_ws_stage1(const GfWsArgs& a, const GfWsPlan<N
                 Y[j].y = fmaf(-oI[j], oI[j], fmaf(nI[j], nI[j], Y[j].y));
             }
         }
+        if (HIST) gf_tm_st_row<K>(tm + (hslot == 0 ? KW - 1 : hslot - 1) * G::TM_ROW, nI, nP);     // row m+R
         if (EM == 1 || EM == 2) {
             if (TRUNC) {
 #pragma unroll
@@ -541,19 +641,25 @@ __device__ __forceinline__ void gf_ws_stage1(const GfWsArgs& a, const GfWsPlan<N
         if (ROLE != 1 && m + GF_WS_PF + 1 < st.m1) prefetch_row(m + 1 + R + GF_WS_PF);
         const int cons_seen = ROLE != 1 ? gf_ws_ld_acq(cons_own) : 0;      // read early, needed just before the ring store
         if (m + 1 < st.m1) {
-            if (EM != 3 && simple) {       // rows never leave the image: four running row pointers, no per-row address arithmetic
-                pnI += stepI; pnP += stepP; poI += stepI; poP += stepP;
+            if (EM != 3 && simple) {       // rows never leave the image: running row pointers, no per-row address arithmetic
+                pnI += stepI; pnP += stepP;
+                if (!HIST) { poI += stepI; poP += stepP; }
                 ld_vec(pnI, nI);
                 ld_vec(pnP, nP);
-                ld_vec(poI, oI);
-                ld_vec(poP, oP);
+                if (!HIST) {
+                    ld_vec(poI, oI);
+                    ld_vec(poP, oP);
+                }
             } else {
-                const int rn = row_of(m + 1 + R), ro = row_of(m - R);
+                const int rn = row_of(m + 1 + R), ro = HIST ? 0 : row_of(m - R);
                 ld_row(gI, gIx, a.gs, rn, nI);
                 ld_row(gP, gPx, a.ss, rn, nP);
-                ld_row(gI, gIx, a.gs, ro, oI);
-                ld_row(gP, gPx, a.ss, ro, oP);
+                if (!HIST) {
+                    ld_row(gI, gIx, a.gs, ro, oI);
+                    ld_row(gP, gPx, a.ss, ro, oP);
+                }
             }
+            if (HIST) gf_tm_ld_row<K>(tm + hslot * G::TM_ROW, oI, oP);      // row m-R (waited for at the end of the iteration)
         }
         // ---- horizontal: window sums of the two quantity pairs ----
         const int idx = m - st.m0;
@@ -657,11 +763,17 @@ __device__ __forceinline__ void gf_ws_stage1(const GfWsArgs& a, const GfWsPlan<N
                 }
             }
         }
+        if (HIST) {
+            // the next iteration overwrites the slot just read: its load has to be complete (and the store is, long since)
+            gf_tm_wait_st();
+            gf_tm_wait_ld<K>(oI, oP);
+            hslot = hslot + 1 == KW ? 0 : hslot + 1;
+        }
     }
-#if GF_WS_SYNC == 2
+    // "stream finished": every own row is in the ring, and the stream is done with its tensor memory (warp 0 frees it)
+    if (HIST) gf_tm_fence_before();
     __syncwarp();
-    if (ROLE != 2 && lane == 0) gf_ws_bar_arrive(bars + k * G::NBAR + 2 * RING);        // "stream finished": every own row is in the ring
-#endif
+    if (ROLE != 2 && lane == 0) gf_ws_bar_arrive(bars + k * G::NBAR + 2 * RING);
 }
 
 // ---- stage 2: consumer warp -------------------------------------------------------------------------
@@ -806,10 +918,15 @@ __global__ void __launch_bounds__((SPLIT ? 96 : 64) * NS, 1) gf_ws_gray_kernel(c
     else { band = rem / a.nstrips; strip = rem % a.nstrips; hbw = a.hb; }
     const int y0 = a.out_y0 + band * hbw;
     const int y1 = y0 + hbw < a.out_y0 + a.out_rows ? y0 + hbw : a.out_y0 + a.out_rows;
+    constexpr bool TM = G::TMEM && !SPLIT;           // the producers keep their input rows in tensor memory
+    __shared__ unsigned tm_base;
+    if (TM && warp == 0) gf_tm_alloc(&tm_base, G::TM_ALLOC);
     if (threadIdx.x < 2 * NS) ctrl[threadIdx.x] = 0;
     for (int i = threadIdx.x; i < NS * G::NBAR; i += blockDim.x)          // (2-stream CTAs have fewer threads than barriers)
         gf_ws_bar_init(reinterpret_cast<unsigned long long*>(const_cast<int*>(ctrl) + 16) + i);
+    if (TM) gf_tm_fence_before();
     __syncthreads();
+    if (TM) gf_tm_fence_after();
     GfWsPlan<NS> pl;
     gf_ws_plan<R, NS>(y0, y1, a.pen, pl);
     // strips tile the width in steps of WOUT; the LAST one is pulled back so that its window ends exactly HALO columns
@@ -831,19 +948,29 @@ __global__ void __launch_bounds__((SPLIT ? 96 : 64) * NS, 1) gf_ws_gray_kernel(c
 #endif
     const bool in_l = xl >= 0, in_r = xl + G::WIN <= a.width;
     const int em = (in_l && in_r) ? 0 : ((xl == -G::HALO && in_r) ? 1 : ((in_l && xl + G::WIN == a.width + G::HALO) ? 2 : 3));
+    // producer k reaches the lanes of quarter k % 4; k and k + 4 split its columns
+    const unsigned tm = TM ? tm_base + ((unsigned)(32 * (k % 4)) << 16) + (unsigned)(k / 4 * G::KW * G::TM_ROW) : 0u;
 #define GF_WS_S1(ROLE)                                                                                                   \
     do {                                                                                                                 \
-        if (em == 0) gf_ws_stage1<R, K, NS, TRUNC, 0, ROLE>(a, pl, k, lane, f, xl, out_lo, out_hi, smem, ctrl);            \
-        else if (em == 1) gf_ws_stage1<R, K, NS, TRUNC, 1, ROLE>(a, pl, k, lane, f, xl, out_lo, out_hi, smem, ctrl);       \
-        else if (em == 2) gf_ws_stage1<R, K, NS, TRUNC, 2, ROLE>(a, pl, k, lane, f, xl, out_lo, out_hi, smem, ctrl);       \
-        else gf_ws_stage1<R, K, NS, TRUNC, 3, ROLE>(a, pl, k, lane, f, xl, out_lo, out_hi, smem, ctrl);                    \
+        if (em == 0) gf_ws_stage1<R, K, NS, TRUNC, 0, ROLE>(a, pl, k, lane, f, xl, out_lo, out_hi, smem, ctrl, tm);        \
+        else if (em == 1) gf_ws_stage1<R, K, NS, TRUNC, 1, ROLE>(a, pl, k, lane, f, xl, out_lo, out_hi, smem, ctrl, tm);   \
+        else if (em == 2) gf_ws_stage1<R, K, NS, TRUNC, 2, ROLE>(a, pl, k, lane, f, xl, out_lo, out_hi, smem, ctrl, tm);   \
+        else gf_ws_stage1<R, K, NS, TRUNC, 3, ROLE>(a, pl, k, lane, f, xl, out_lo, out_hi, smem, ctrl, tm);                \
     } while (0)
     if (SPLIT) {
         if (part == 0) GF_WS_S1(1);
         else if (part == 1) GF_WS_S1(2);
         else gf_ws_stage2<R, K, NS, TRUNC>(a, pl, k, lane, f, xl, out_lo, out_hi, smem, ctrl);
     } else {
-        if (part == 0) GF_WS_S1(0);
+        if (part == 0) {
+            GF_WS_S1(0);
+            if (TM && warp == 0) {     // free the history once every producer of the CTA (k < pl.n; the others returned) has finished
+                const unsigned long long* bars = reinterpret_cast<const unsigned long long*>(const_cast<const int*>(ctrl) + 16);
+                for (int s = 0; s < pl.n; ++s) gf_ws_bar_wait(bars + s * G::NBAR + 2 * G::RING, 0);
+                gf_tm_fence_after();
+                gf_tm_dealloc(tm_base, G::TM_ALLOC);
+            }
+        }
         else gf_ws_stage2<R, K, NS, TRUNC>(a, pl, k, lane, f, xl, out_lo, out_hi, smem, ctrl);
     }
 #undef GF_WS_S1
