@@ -45,6 +45,7 @@ SIGNATURES = {
     "gf_host_free": (c_int, [P]),
     "gf_guided_gray_u8": (c_int, [P, P, P, c_int, c_int, c_int64, c_int64, c_int64, c_int, c_float, c_int, P]),
     "gf_guided_color_u8": (c_int, [P, P, P, c_int, c_int, c_int, c_int64, c_int64, c_int64, c_int, c_float, c_int, P]),
+    "gf_guided_per_channel_u8": (c_int, [P, P, P, c_int, c_int, c_int, c_int64, c_int64, c_int64, c_int, c_float, c_int, P]),
     "gf_gaussian_gray": (c_int, [P, P, c_int, c_int, c_int64, c_int64, c_int, ctypes.c_double, P]),
     "gf_integral_u8_i32": (c_int, [P, P, P, c_int, c_int, c_int64, c_int64, P]),
     "gf_integral_u8_i64": (c_int, [P, P, P, c_int, c_int, c_int64, c_int64, P]),

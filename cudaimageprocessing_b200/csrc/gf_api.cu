@@ -23,9 +23,10 @@
 #ifdef GF_HAVE_FAST
 #include "gf_fast.cuh"
 #include "gf_wp.cuh"
-// the big kernel families live in their own translation units (gf_tu_s8.cu, gf_tu_ws.cu, gf_tu_c4.cu, gf_tu_c4u8.cu) so
-// that the library builds in parallel
+// the big kernel families live in their own translation units (gf_tu_s8.cu, gf_tu_s8pc.cu, gf_tu_ws.cu, gf_tu_c4.cu,
+// gf_tu_c4u8.cu) so that the library builds in parallel
 const char* gf_s8_try_x(const Job& j, bool* done, const char** name, bool u8);
+const char* gf_s8pc_try_x(const Job& j, bool* done, const char** name);
 const char* gf_ws_try_x(const Job& j, bool* done, const char** name);
 const char* gf_c4_try_x(const Job& j, bool* done, const char** name);
 const char* gf_c4u8_try_x(const Job& j, bool* done, const char** name);
@@ -622,6 +623,45 @@ int gf_guided_gray_u8(const unsigned char* guide, const unsigned char* src, unsi
     return GF_OK;
 #else
     return fail(GF_ERR_UNSUPPORTED, "gf_guided_gray_u8: built without the tuned kernels");
+#endif
+}
+
+int gf_guided_per_channel_u8(const unsigned char* guide, const unsigned char* src, unsigned char* dst, int width, int height,
+                             int guide_channels, int64_t guide_stride, int64_t src_stride, int64_t dst_stride, int r, float eps,
+                             int border, void* stream)
+{
+#ifdef GF_HAVE_FAST
+    if (guide_channels != 1 && guide_channels != 3) return fail(GF_ERR_UNSUPPORTED, "Do not support channel: %d, 3", guide_channels);
+    Job j;
+    j.count = 3;                            // one launch: the frames of the s8 kernel are the source channels
+    j.width = width; j.height = height; j.buf_rows = height; j.out_rows = height;
+    j.r = r; j.eps = eps; j.border = border; j.stream = stream;
+    // Plane carries float*: the u8 planes are reinterpreted, every stride is in ELEMENTS (= bytes here)
+    j.guide = Plane{reinterpret_cast<const float*>(guide), or_packed(guide_stride, width, guide_channels), 0, guide_channels, 0};
+    j.src = Plane{reinterpret_cast<const float*>(src), or_packed(src_stride, width, 3), 0, 3, 0};
+    j.dst = Plane{reinterpret_cast<const float*>(dst), or_packed(dst_stride, width, 3), 0, 3, 0};
+    j.A = j.B = Plane{nullptr, 0, 0, 1, 0};
+    if (int rc = check_common(j)) return rc;
+    {   // any overlap of the output with an input, not just equal pointers (byte ranges: the planes hold unsigned char)
+        auto ov = [&](const unsigned char* a, int64_t sa, const unsigned char* b, int64_t sb) {
+            return a < b + (int64_t)height * sb && b < a + (int64_t)height * sa;
+        };
+        if (ov(dst, j.dst.stride, guide, j.guide.stride) || ov(dst, j.dst.stride, src, j.src.stride))
+            return fail(GF_ERR_UNSUPPORTED, "gf_guided_per_channel_u8: in-place filtering is not supported");
+    }
+    bool done = false;
+    const char* name = nullptr;
+    const char* e = gf_s8pc_try_x(j, &done, &name);
+    if (!done)
+        return fail(GF_ERR_UNSUPPORTED, "gf_guided_per_channel_u8 needs r in {1..8,16}, width >= 64, width and height >= 4r+2, "
+                                        "rows x stride < 2^31, 8-byte aligned planes and row strides and, for the TRUNCATE border, "
+                                        "width %% 8 == 0 and >= 256");
+    if (e) return fail(GF_ERR_CUDA, "%s launch: %s", name, e);
+    g_launches++;
+    g_kernel = name;
+    return GF_OK;
+#else
+    return fail(GF_ERR_UNSUPPORTED, "gf_guided_per_channel_u8: built without the tuned kernels");
 #endif
 }
 

@@ -88,19 +88,6 @@ struct GfC4Ctx {
     unsigned selA, selB;                             // uint8 only: byte selectors of the src words (gf_c4_expand)
 };
 
-// Byte permute (PRMT): byte n of the result is byte (s >> 4n) & 7 of the 8 bytes y:x.
-__device__ __forceinline__ unsigned gf_prmt(unsigned x, unsigned y, unsigned s)
-{
-#ifdef GF_CPU_EMU
-    const unsigned long long v = ((unsigned long long)y << 32) | x;
-    unsigned r = 0;
-    for (int n = 0; n < 4; ++n) r |= (unsigned)((v >> (8 * ((s >> (4 * n)) & 7))) & 255u) << (8 * n);
-    return r;
-#else
-    return __byte_perm(x, y, s);
-#endif
-}
-
 // uint8 build: a raw row (vi[0..2]: the 12 guide bytes; vp[0..2]: the src words, as float bit patterns) -> floats 0..255.
 // The src pixels are gathered into one word first: 1 channel: bytes 0..3 of vp[0] (= vp[1]); 3 channels: pixel j,
 // channel ch is byte 3j + ch of the 12 bytes, i.e. byte ch, 3 + ch of (vp[0], vp[1]) and 2 + ch, 5 + ch of (vp[1], vp[2]).

@@ -135,6 +135,52 @@ __device__ __forceinline__ void gf_st8(unsigned char* p, const float2 (&v)[4])
     t.y = gf_f_to_u8(v[2].x) | (gf_f_to_u8(v[2].y) << 8) | (gf_f_to_u8(v[3].x) << 16) | (gf_f_to_u8(v[3].y) << 24);
     *reinterpret_cast<uint2*>(p) = t;
 }
+
+// Byte permute (PRMT): byte n of the result is byte (s >> 4n) & 7 of the 8 bytes y:x.
+__device__ __forceinline__ unsigned gf_prmt(unsigned x, unsigned y, unsigned s)
+{
+#ifdef GF_CPU_EMU
+    const unsigned long long v = ((unsigned long long)y << 32) | x;
+    unsigned r = 0;
+    for (int n = 0; n < 4; ++n) r |= (unsigned)((v >> (8 * ((s >> (4 * n)) & 7))) & 255u) << (8 * n);
+    return r;
+#else
+    return __byte_perm(x, y, s);
+#endif
+}
+
+// 3 interleaved channels (gf_guided_per_channel_u8): a lane's 8 pixels are 24 bytes at an 8-byte aligned address, loaded
+// with three 8-byte loads and kept RAW in v[0..2]; gf_u8_pick3 gathers the 8 bytes of one channel into v[0], where
+// gf_u8_expand finds the bytes of a 1-channel row.  Pixel k, channel ch is byte 3k + ch of the 24: per 4 pixels (3 words
+// w0 w1 w2) bytes ch, 3 + ch of w0:w1 (selector selA) and bytes 2 + ch, 5 + ch of w1:w2 (selB), merged by 0x7610.
+__device__ __forceinline__ void gf_ld24(const unsigned char* p, float2 (&v)[4])
+{
+    const uint2* q = reinterpret_cast<const uint2*>(p);
+    const uint2 t0 = q[0], t1 = q[1], t2 = q[2];
+    v[0] = make_float2(gf_bits_f(t0.x), gf_bits_f(t0.y));
+    v[1] = make_float2(gf_bits_f(t1.x), gf_bits_f(t1.y));
+    v[2] = make_float2(gf_bits_f(t2.x), gf_bits_f(t2.y));
+    v[3] = make_float2(0.f, 0.f);
+}
+__device__ __forceinline__ void gf_u8_pick3(float2 (&v)[4], unsigned selA, unsigned selB)
+{
+    unsigned w[6];
+#pragma unroll
+    for (int i = 0; i < 3; ++i) { w[2 * i] = gf_f_bits(v[i].x); w[2 * i + 1] = gf_f_bits(v[i].y); }
+    const unsigned x = gf_prmt(gf_prmt(w[0], w[1], selA), gf_prmt(w[1], w[2], selB), 0x7610u);
+    const unsigned y = gf_prmt(gf_prmt(w[3], w[4], selA), gf_prmt(w[4], w[5], selB), 0x7610u);
+    v[0] = make_float2(gf_bits_f(x), gf_bits_f(y));
+}
+// ... and stores the lane's 8 bytes of its channel one by one (p points at channel ch of the lane's first pixel): the
+// other channels of the same pixels are other CTAs' frames.
+__device__ __forceinline__ void gf_st8x3(unsigned char* p, const float2 (&v)[4])
+{
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        p[6 * i] = (unsigned char)gf_f_to_u8(v[i].x);
+        p[6 * i + 3] = (unsigned char)gf_f_to_u8(v[i].y);
+    }
+}
 __device__ __forceinline__ float2 gf_neg2(float2 a) { return make_float2(-a.x, -a.y); }
 __device__ __forceinline__ float2 gf_dup2(float a) { return make_float2(a, a); }
 
@@ -203,9 +249,15 @@ struct GfS8Geom {
     static constexpr size_t ring_bytes = (size_t)KW * SLOT_F2 * 8;
 };
 
-template <int R, class T = float>
+// GC, PC: interleaved channels of the guide and of src / dst.  GC = PC = 1 is every planar build; PC = 3 (uint8 only,
+// gf_guided_per_channel_u8) filters channel ch = frame index of 3-channel src / dst with a gray (GC = 1) guide or with
+// the guide's channel ch (GC = 3).
+template <int R, class T = float, int GC = 1, int PC = 1>
 struct GfS8Ctx {
     const T* gI; const T* gP; T* gQ;     // frame bases at (row buf_y0 / out_y0, this lane's first column)
+                                         // (PC = 3: gI, gP at its first pixel's byte 0, gQ at its byte ch)
+    int ch;                                          // PC = 3 only: the channel (frame) this warp filters
+    unsigned selA, selB;                             // PC = 3 only: byte selectors of channel ch (gf_u8_pick3)
     int gs, ss, ds;                                  // row strides; (rows * stride) fits 31 bits (host check)
     float2* ring;                                    // this lane's cell of ring row 0
     int lane, x0, width, height, border, buf_y0, buf_ylast, out_y0, yi0;
@@ -249,46 +301,59 @@ __device__ __forceinline__ float gf_s8_rcp(float d)
 // 2 generic per-column border map (any border, any width; slow, rarely needed); 4 TRUNCATE border
 // (the class API): pixels outside the image contribute nothing and every mean divides by the number of
 // in-image pixels of its window (guided_filter_d.cu:251-262) -- zero-filled loads, per-pixel counts.
-template <int MODE, int R, class T>
-__device__ __forceinline__ void gf_s8_ld(const GfS8Ctx<R, T>& c, const T* rowp, float2 (&v)[4], float& sc)
+// P: interleaved channels of the plane rowp belongs to (GC or PC); column offsets are in pixels of P elements, and a
+// scalar of a 3-channel plane is byte ch of its pixel.
+template <int P, class T>
+__device__ __forceinline__ void gf_ld8p(const T* p, float2 (&v)[4])
 {
+    if constexpr (P == 3) gf_ld24(p, v);
+    else gf_ld8(p, v);
+}
+template <int MODE, int P = 1, int R, class T, int GC, int PC>
+__device__ __forceinline__ void gf_s8_ld(const GfS8Ctx<R, T, GC, PC>& c, const T* rowp, float2 (&v)[4], float& sc)
+{
+    const int cho = P == 3 ? c.ch : 0;
     if (MODE == 3) {
         // RAW mirror data: the permutation is applied where the row is consumed (gf_s8_fix), one iteration later --
         // selects right behind the loads would make the warp wait for them here and expose the memory latency
-        gf_ld8(rowp + c.vofs, v);
+        gf_ld8p<P>(rowp + P * c.vofs, v);
         sc = 0.f;                                       // only the lanes outside the image need the scalar (a predicated
-        if (c.out_l || c.out_r) sc = gf_ld1(rowp + c.sofs);   // load: 1-2 wavefronts instead of 8 for the whole warp)
+        if (c.out_l || c.out_r) sc = gf_ld1(rowp + P * c.sofs + cho);   // load: 1-2 wavefronts instead of 8 for the whole warp)
     } else if (MODE == 4) {
         if (c.lane_in) {
-            gf_ld8(rowp, v);
+            gf_ld8p<P>(rowp, v);
         } else {
 #pragma unroll
             for (int i = 0; i < 4; ++i) v[i] = make_float2(0.f, 0.f);
         }
     } else if (MODE != 2 || c.vec_ok) {
-        gf_ld8(rowp, v);
+        gf_ld8p<P>(rowp, v);
     } else {
 #pragma unroll
-        for (int i = 0; i < 4; ++i) v[i] = make_float2(gf_ld1(rowp + c.sx[2 * i]), gf_ld1(rowp + c.sx[2 * i + 1]));
+        for (int i = 0; i < 4; ++i) v[i] = make_float2(gf_ld1(rowp + P * c.sx[2 * i] + cho), gf_ld1(rowp + P * c.sx[2 * i + 1] + cho));
     }
 }
 
 // MODE 3: raw mirror data -> the lane's 8 columns
 //   left of the image:  column -8k+j <- column 8k-j   = {sc, e7, e6, .., e1}
 //   right of the image: column W+8m+j <- W-2-8m-j     = {e6, e5, .., e0, sc}
-template <int MODE, int R, class T>
-__device__ __forceinline__ void gf_s8_fix(const GfS8Ctx<R, T>& c, float2 (&v)[4], float sc)
+template <int MODE, int P = 1, int R, class T, int GC, int PC>
+__device__ __forceinline__ void gf_s8_fix(const GfS8Ctx<R, T, GC, PC>& c, float2 (&v)[4], float sc)
 {
     if (sizeof(T) == 1) {                               // uint8 build: the vector part of the row is still raw bytes
+        auto expand = [&](float2 (&u)[4]) {
+            if constexpr (P == 3) gf_u8_pick3(u, c.selA, c.selB);
+            gf_u8_expand(u);
+        };
         if (MODE == 2) {                                // (lanes that gathered column by column already hold floats)
             float2 t[4] = {v[0], v[1], v[2], v[3]};
-            gf_u8_expand(t);
+            expand(t);
 #pragma unroll
             for (int i = 0; i < 4; ++i) v[i] = c.vec_ok ? t[i] : v[i];
         } else if (MODE == 4) {
-            if (c.lane_in) gf_u8_expand(v);
+            if (c.lane_in) expand(v);
         } else {
-            gf_u8_expand(v);
+            expand(v);
         }
     }
     if (MODE != 3) return;
@@ -306,8 +371,8 @@ __device__ __forceinline__ void gf_s8_fix(const GfS8Ctx<R, T>& c, float2 (&v)[4]
 
 // Row y (any integer) of both planes: REFLECT borders map the row index; MODE 4 (TRUNCATE) rows outside
 // the image are zeros.
-template <int MODE, int R, class T>
-__device__ __forceinline__ void gf_s8_ld_row(const GfS8Ctx<R, T>& c, int y, float2 (&vI)[4], float2 (&vP)[4], float& scI, float& scP)
+template <int MODE, int R, class T, int GC, int PC>
+__device__ __forceinline__ void gf_s8_ld_row(const GfS8Ctx<R, T, GC, PC>& c, int y, float2 (&vI)[4], float2 (&vP)[4], float& scI, float& scP)
 {
     if (MODE == 4) {
         if (y < 0 || y > c.buf_ylast) {
@@ -316,14 +381,14 @@ __device__ __forceinline__ void gf_s8_ld_row(const GfS8Ctx<R, T>& c, int y, floa
             return;
         }
         const int o = y - c.buf_y0;
-        gf_s8_ld<MODE>(c, c.gI + o * c.gs, vI, scI);
-        gf_s8_ld<MODE>(c, c.gP + o * c.ss, vP, scP);
+        gf_s8_ld<MODE, GC>(c, c.gI + o * c.gs, vI, scI);
+        gf_s8_ld<MODE, PC>(c, c.gP + o * c.ss, vP, scP);
     } else {
         int rn = gf_s8_map_y(y, c.height, c.border);
         rn = rn > c.buf_ylast ? c.buf_ylast : rn;
         const int o = rn - c.buf_y0;
-        gf_s8_ld<MODE>(c, c.gI + o * c.gs, vI, scI);
-        gf_s8_ld<MODE>(c, c.gP + o * c.ss, vP, scP);
+        gf_s8_ld<MODE, GC>(c, c.gI + o * c.gs, vI, scI);
+        gf_s8_ld<MODE, PC>(c, c.gP + o * c.ss, vP, scP);
     }
 }
 
@@ -336,8 +401,8 @@ __device__ __forceinline__ float gf_s8_cnt_y(int y, int height)
 }
 
 // c = f, f = 0: f holds exactly the rows of the current window, summed without a subtraction
-template <int R, class T>
-__device__ __forceinline__ void gf_s8_reseed1(GfS8Ctx<R, T>& c)
+template <int R, class T, int GC, int PC>
+__device__ __forceinline__ void gf_s8_reseed1(GfS8Ctx<R, T, GC, PC>& c)
 {
     if (!GF_S8_RESEED1 || sizeof(T) != 4) return;
 #pragma unroll
@@ -346,8 +411,8 @@ __device__ __forceinline__ void gf_s8_reseed1(GfS8Ctx<R, T>& c)
         c.fI[i] = c.fP[i] = c.fIP[i] = c.fII[i] = make_float2(0.f, 0.f);
     }
 }
-template <int R, class T>
-__device__ __forceinline__ void gf_s8_reseed2(GfS8Ctx<R, T>& c)
+template <int R, class T, int GC, int PC>
+__device__ __forceinline__ void gf_s8_reseed2(GfS8Ctx<R, T, GC, PC>& c)
 {
     if (!GF_S8_RESEED2) return;
 #pragma unroll
@@ -362,8 +427,8 @@ __device__ __forceinline__ void gf_s8_reseed2(GfS8Ctx<R, T>& c)
 // stage 1 of input row yi = yi0 + t.  ONE copy of this code per strip mode serves the whole band
 // (instruction-cache footprint): ramp-up is data, not code -- the first a, b row (t = 2R) and the
 // first "old" row are zeros, and while `full` is false the ring is written but not subtracted.
-template <int R, int MODE, class T>
-__device__ __forceinline__ void gf_s8_iter(GfS8Ctx<R, T>& c, int t, int slot, bool full)
+template <int R, int MODE, class T, int GC, int PC>
+__device__ __forceinline__ void gf_s8_iter(GfS8Ctx<R, T, GC, PC>& c, int t, int slot, bool full)
 {
     using G = GfS8Geom<R>;
     constexpr int KW = G::KW, VL = G::VL;
@@ -374,8 +439,8 @@ __device__ __forceinline__ void gf_s8_iter(GfS8Ctx<R, T>& c, int t, int slot, bo
     // ================= phase B, part 1: vertical sums of row yi =================
     // (first, so that the loads of the next iteration can be issued right away and have a whole
     // iteration to land)
-    gf_s8_fix<MODE>(c, c.nI, c.sc[0]); gf_s8_fix<MODE>(c, c.nP, c.sc[1]);
-    gf_s8_fix<MODE>(c, c.oI, c.sc[2]); gf_s8_fix<MODE>(c, c.oP, c.sc[3]);
+    gf_s8_fix<MODE, GC>(c, c.nI, c.sc[0]); gf_s8_fix<MODE, PC>(c, c.nP, c.sc[1]);
+    gf_s8_fix<MODE, GC>(c, c.oI, c.sc[2]); gf_s8_fix<MODE, PC>(c, c.oP, c.sc[3]);
     float2 gI[4];
 #pragma unroll
     for (int i = 0; i < 4; ++i) gI[i] = c.oI[i];
@@ -403,9 +468,14 @@ __device__ __forceinline__ void gf_s8_iter(GfS8Ctx<R, T>& c, int t, int slot, bo
             if (rp <= c.buf_ylast) {
                 const int op = rp - c.buf_y0;
                 constexpr int LINE = 128 / (int)sizeof(T);      // elements per 128-byte line
-                if (lane * LINE < 256) {
-                    gf_prefetch_l2(c.gI + op * c.gs + (LINE - 8) * lane);
-                    gf_prefetch_l2(c.gP + op * c.ss + (LINE - 8) * lane);
+                if (GC == PC) {
+                    if (lane * LINE < 256 * PC) {
+                        gf_prefetch_l2(c.gI + op * c.gs + (LINE - 8 * GC) * lane);
+                        gf_prefetch_l2(c.gP + op * c.ss + (LINE - 8 * PC) * lane);
+                    }
+                } else {                                    // a gray guide spans 1/3 of the lines of a 3-channel source
+                    if (lane * LINE < 256 * GC) gf_prefetch_l2(c.gI + op * c.gs + (LINE - 8 * GC) * lane);
+                    if (lane * LINE < 256 * PC) gf_prefetch_l2(c.gP + op * c.ss + (LINE - 8 * PC) * lane);
                 }
             }
         }
@@ -457,12 +527,19 @@ __device__ __forceinline__ void gf_s8_iter(GfS8Ctx<R, T>& c, int t, int slot, bo
             T* pq = c.gQ + (yo - c.out_y0) * c.ds;
             if (c.out_lane && !(GF_S8_ABL & 8)) {
                 if (!XMAP || c.vec_ok) {
-                    gf_st8(pq, q);
+                    if constexpr (PC == 3) gf_st8x3(pq, q);
+                    else gf_st8(pq, q);
                 } else {
 #pragma unroll
                     for (int i = 0; i < 4; ++i) {
-                        if (c.x0 + 2 * i >= 0 && c.x0 + 2 * i < c.width) gf_st1(pq + 2 * i, q[i].x);
-                        if (c.x0 + 2 * i + 1 >= 0 && c.x0 + 2 * i + 1 < c.width) gf_st1(pq + 2 * i + 1, q[i].y);
+                        // (written out for PC = 1: an index scaled by 1 reorders the planar builds' code)
+                        if constexpr (PC == 1) {
+                            if (c.x0 + 2 * i >= 0 && c.x0 + 2 * i < c.width) gf_st1(pq + 2 * i, q[i].x);
+                            if (c.x0 + 2 * i + 1 >= 0 && c.x0 + 2 * i + 1 < c.width) gf_st1(pq + 2 * i + 1, q[i].y);
+                        } else {
+                            if (c.x0 + 2 * i >= 0 && c.x0 + 2 * i < c.width) gf_st1(pq + PC * (2 * i), q[i].x);
+                            if (c.x0 + 2 * i + 1 >= 0 && c.x0 + 2 * i + 1 < c.width) gf_st1(pq + PC * (2 * i + 1), q[i].y);
+                        }
                     }
                 }
             }
@@ -522,8 +599,8 @@ __device__ __forceinline__ void gf_s8_iter(GfS8Ctx<R, T>& c, int t, int slot, bo
 // Warm-up rows t in [0, 2R): vertical accumulation only.  Nothing else is going on, so a single
 // row in flight would expose the full DRAM latency 2R times; rows are loaded CH at a time instead.
 // On entry nI/nP hold row yi0 (t = 0); on exit they hold row yi0 + 2R.
-template <int R, int MODE, class T>
-__device__ __forceinline__ void gf_s8_warmup(GfS8Ctx<R, T>& c)
+template <int R, int MODE, class T, int GC, int PC>
+__device__ __forceinline__ void gf_s8_warmup(GfS8Ctx<R, T, GC, PC>& c)
 {
     constexpr int CH = 4, NROWS = 2 * R;
     float2 bI[CH][4], bP[CH][4];
@@ -538,7 +615,7 @@ __device__ __forceinline__ void gf_s8_warmup(GfS8Ctx<R, T>& c)
 #pragma unroll
         for (int k = 0; k < CH; ++k) {
             if (t0 + k < NROWS) {
-                gf_s8_fix<MODE>(c, c.nI, c.sc[0]); gf_s8_fix<MODE>(c, c.nP, c.sc[1]);
+                gf_s8_fix<MODE, GC>(c, c.nI, c.sc[0]); gf_s8_fix<MODE, PC>(c, c.nP, c.sc[1]);
                 c.sc[0] = bsI[k]; c.sc[1] = bsP[k];
 #pragma unroll
                 for (int i = 0; i < 4; ++i) {
@@ -556,8 +633,8 @@ __device__ __forceinline__ void gf_s8_warmup(GfS8Ctx<R, T>& c)
 // The row loop of one band: 2R warm-up rows, then iterations t = 2R .. steps in periods of 2R+1
 // (= ring length = re-seed period; the inner loop is straight-line code, `slot` is its counter).
 // The last iteration only needs its phase A; its phase B works on clamped rows and is discarded.
-template <int R, int MODE, class T>
-__device__ __forceinline__ void gf_s8_band(GfS8Ctx<R, T>& c, int steps)
+template <int R, int MODE, class T, int GC, int PC>
+__device__ __forceinline__ void gf_s8_band(GfS8Ctx<R, T, GC, PC>& c, int steps)
 {
     constexpr int KW = 2 * R + 1;
     gf_s8_warmup<R, MODE>(c);
@@ -579,14 +656,15 @@ __device__ __forceinline__ void gf_s8_band(GfS8Ctx<R, T>& c, int steps)
 // Strip geometry: strip s outputs columns [s * WOUT, (s + 1) * WOUT) and reads 2 * H1 lanes of halo
 // on either side.  Strips that overhang the image use mirror loads (MODE 3: REFLECT101,
 // width % 8 == 0), clipped counts (MODE 4: TRUNCATE) or the generic per-column border map (MODE 2).
-template <int R, int MINB, class T>
+// GC, PC: see GfS8Ctx.
+template <int R, int MINB, class T, int GC = 1, int PC = 1>
 __global__ void __launch_bounds__(32, MINB) gf_s8_gray_kernel(const GF_GRID_CONSTANT GfWpArgs a)
 {
     using G = GfS8Geom<R>;
     constexpr int H1 = G::H1, KW = G::KW, VL = G::VL;
     GF_DYN_SMEM(float, smem);
     auto run = [&](int64_t f, int strip, int yo0, int yo1) {
-    GfS8Ctx<R, T> c;
+    GfS8Ctx<R, T, GC, PC> c;
     c.lane = threadIdx.x & 31;
     const int xl = strip * G::WOUT - 2 * H1 * 8, lane_lo = 2 * H1;
     int mode = 0;
@@ -599,8 +677,14 @@ __global__ void __launch_bounds__(32, MINB) gf_s8_gray_kernel(const GF_GRID_CONS
     }
     c.x0 = xl + 8 * c.lane;
     // (GfWpArgs carries the planes as float*; T = unsigned char builds reinterpret them, strides are in elements)
-    c.gI = reinterpret_cast<const T*>(a.guide) + f * a.gfs + c.x0; c.gP = reinterpret_cast<const T*>(a.src) + f * a.sfs + c.x0;
-    c.gQ = reinterpret_cast<T*>(a.dst) + f * a.dfs + c.x0;
+    c.gI = reinterpret_cast<const T*>(a.guide) + f * a.gfs + GC * c.x0; c.gP = reinterpret_cast<const T*>(a.src) + f * a.sfs + PC * c.x0;
+    c.gQ = reinterpret_cast<T*>(a.dst) + f * a.dfs + PC * c.x0;
+    if constexpr (PC == 3) {                             // frame f is channel f of the interleaved planes (frame strides 0)
+        c.ch = (int)f;
+        c.gQ += f;
+        c.selA = (unsigned)f | (3u + (unsigned)f) << 4;
+        c.selB = (2u + (unsigned)f) << 8 | (5u + (unsigned)f) << 12;
+    }
     c.gs = (int)a.gs; c.ss = (int)a.ss; c.ds = (int)a.ds;
     c.ring_lane = c.lane >= lane_lo && c.lane < lane_lo + VL;
     c.out_lane = c.ring_lane && c.x0 < a.width;
@@ -635,16 +719,16 @@ __global__ void __launch_bounds__(32, MINB) gf_s8_gray_kernel(const GF_GRID_CONS
     const int steps = (yo1 - yo0) + 4 * R;
     const int o0 = gf_s8_map_y(c.yi0, a.height, a.border) - a.buf_y0;       // row of iteration 0
     if (mode == 2) {
-        gf_s8_ld<2>(c, c.gI + o0 * c.gs, c.nI, c.sc[0]); gf_s8_ld<2>(c, c.gP + o0 * c.ss, c.nP, c.sc[1]);
+        gf_s8_ld<2, GC>(c, c.gI + o0 * c.gs, c.nI, c.sc[0]); gf_s8_ld<2, PC>(c, c.gP + o0 * c.ss, c.nP, c.sc[1]);
         gf_s8_band<R, 2>(c, steps);
     } else if (mode == 3) {
-        gf_s8_ld<3>(c, c.gI + o0 * c.gs, c.nI, c.sc[0]); gf_s8_ld<3>(c, c.gP + o0 * c.ss, c.nP, c.sc[1]);
+        gf_s8_ld<3, GC>(c, c.gI + o0 * c.gs, c.nI, c.sc[0]); gf_s8_ld<3, PC>(c, c.gP + o0 * c.ss, c.nP, c.sc[1]);
         gf_s8_band<R, 3>(c, steps);
     } else if (mode == 4) {
         gf_s8_ld_row<4>(c, c.yi0, c.nI, c.nP, c.sc[0], c.sc[1]);
         gf_s8_band<R, 4>(c, steps);
     } else {
-        gf_s8_ld<0>(c, c.gI + o0 * c.gs, c.nI, c.sc[0]); gf_s8_ld<0>(c, c.gP + o0 * c.ss, c.nP, c.sc[1]);
+        gf_s8_ld<0, GC>(c, c.gI + o0 * c.gs, c.nI, c.sc[0]); gf_s8_ld<0, PC>(c, c.gP + o0 * c.ss, c.nP, c.sc[1]);
         gf_s8_band<R, 0>(c, steps);
     }
     };
@@ -697,7 +781,7 @@ static inline long gf_tape_plan(GfWpArgs& a, int r, long slots, int hb_min, int 
 }
 
 #ifndef GF_S8_NO_TRY     // (translation units that only need the helpers above: gf_tu_ws.cu, gf_tu_c4.cu, gf_api.cu)
-template <int R, class T = float>
+template <int R, class T = float, int GC = 1, int PC = 1>
 static const char* gf_s8_launch(const Job& j)
 {
     using G = GfS8Geom<R>;
@@ -760,19 +844,59 @@ static const char* gf_s8_launch(const Job& j)
     dim3 grid((unsigned)items), block(32);
     constexpr int FIT = (int)((size_t)228 * 1024 / (G::ring_bytes + 1024));
     constexpr int MINB = FIT > 7 ? 7 : (FIT < 1 ? 1 : FIT);
-    auto k = gf_s8_gray_kernel<R, MINB, T>;
+    auto k = gf_s8_gray_kernel<R, MINB, T, GC, PC>;
     if (const char* e = gf_rt_set_smem(k, smem)) return e;
     GF_LAUNCH(k, grid, block, smem, j.stream, a);
     return gf_rt_launch_error();
 }
 
+// The geometry every s8 launch needs, whatever its planes hold.
+static bool gf_s8_geometry_ok(const Job& j)
+{
+    if (j.border == GF_TRUNCATE && ((j.width & 7) || j.width < 256)) return false;
+    // row offsets inside a frame are 32-bit in the kernel
+    if ((int64_t)j.buf_rows * j.guide.stride >= (1ll << 31) || (int64_t)j.buf_rows * j.src.stride >= (1ll << 31) ||
+        (int64_t)j.out_rows * j.dst.stride >= (1ll << 31))
+        return false;
+    // single reflections only, and at least one full warp window of columns
+    return j.height >= 4 * j.r + 2 && j.width >= 4 * j.r + 2 && j.width >= 64;
+}
+
+#if defined(GF_S8_PER_CHANNEL_TRY) || defined(GF_CPU_EMU)
+// gf_guided_per_channel_u8 (its own translation unit, gf_tu_s8pc.cu; the emulator build, one unit per kernel family,
+// compiles it into gf_tu_s8.cu): uint8 planes, src / dst of 3 interleaved channels that are the 3 frames of the launch
+// (count = 3, frame strides 0), the guide gray (shared by the frames) or 3 channels (frame f filtered with guide channel f).  Every plane's base and row stride 8-byte aligned: a lane's 8 pixels are one
+// 8-byte load of a gray plane and three of a 3-channel plane.
+static const char* gf_s8_per_channel_try(const Job& j, bool* done, const char** name)
+{
+    *done = false;
+    const int gc = j.guide.channels;
+    if (j.color || j.A.ptr || j.count != 3 || (gc != 1 && gc != 3) || j.src.channels != 3 || j.dst.channels != 3) return nullptr;
+    const Plane* pl[3] = {&j.guide, &j.src, &j.dst};
+    for (int i = 0; i < 3; ++i)
+        if (pl[i]->coff != 0 || pl[i]->frame_stride != 0 || (pl[i]->stride & 7) || ((uintptr_t)pl[i]->ptr & 7)) return nullptr;
+    if (!gf_s8_geometry_ok(j)) return nullptr;
+    switch (j.r * 4 + gc) {
+#define GF_S8_CASE(RR)                                                                                                         \
+    case 4 * RR + 1: *done = true; *name = "s8u8_g1c3_r" #RR; return gf_s8_launch<RR, unsigned char, 1, 3>(j);           \
+    case 4 * RR + 3: *done = true; *name = "s8u8_g3c3_r" #RR; return gf_s8_launch<RR, unsigned char, 3, 3>(j);
+#ifdef GF_CPU_EMU
+    GF_S8_CASE(4) GF_S8_CASE(7) GF_S8_CASE(8) GF_S8_CASE(16)
+#else      // the radii of gf_guided_gray_u8
+    GF_S8_CASE(1) GF_S8_CASE(2) GF_S8_CASE(3) GF_S8_CASE(4) GF_S8_CASE(5) GF_S8_CASE(6) GF_S8_CASE(7) GF_S8_CASE(8) GF_S8_CASE(16)
+#endif
+#undef GF_S8_CASE
+    default: return nullptr;
+    }
+}
+#endif
+#ifndef GF_S8_PER_CHANNEL_TRY
 // u8 = true: the planes hold unsigned char (Plane::ptr reinterpreted, strides in elements): uint8 in,
 // uint8 out, conversions fused into the loads and stores (gf_guided_gray_u8).
 static const char* gf_s8_try(const Job& j, bool* done, const char** name, bool u8 = false)
 {
     *done = false;
     if (j.color || j.A.ptr) return nullptr;
-    if (j.border == GF_TRUNCATE && ((j.width & 7) || j.width < 256)) return nullptr;
     if (!u8 && (GF_KNOB("GF_DISABLE_S8", 0) || GF_KNOB("GF_DISABLE_FAST", 0))) return nullptr;
     const Plane* pl[3] = {&j.guide, &j.src, &j.dst};
     const uintptr_t amask = u8 ? 7 : 31;                  // one 8-byte / 32-byte vector per lane and row
@@ -780,12 +904,7 @@ static const char* gf_s8_try(const Job& j, bool* done, const char** name, bool u
         if (pl[i]->channels != 1 || pl[i]->coff != 0 || (pl[i]->stride & 7) || (pl[i]->frame_stride & 7) ||
             ((uintptr_t)pl[i]->ptr & amask))
             return nullptr;
-    // row offsets inside a frame are 32-bit in the kernel
-    if ((int64_t)j.buf_rows * j.guide.stride >= (1ll << 31) || (int64_t)j.buf_rows * j.src.stride >= (1ll << 31) ||
-        (int64_t)j.out_rows * j.dst.stride >= (1ll << 31))
-        return nullptr;
-    // single reflections only, and at least one full warp window of columns
-    if (j.height < 4 * j.r + 2 || j.width < 4 * j.r + 2 || j.width < 64) return nullptr;
+    if (!gf_s8_geometry_ok(j)) return nullptr;
     if (u8) {
         switch (j.r) {
 #define GF_S8_CASE(RR) case RR: *done = true; *name = "s8u8_r" #RR; return gf_s8_launch<RR, unsigned char>(j);
@@ -810,5 +929,6 @@ static const char* gf_s8_try(const Job& j, bool* done, const char** name, bool u
     default: return nullptr;
     }
 }
+#endif  // !GF_S8_PER_CHANNEL_TRY
 #endif  // GF_S8_NO_TRY
 #endif  // GF_NO_HOST

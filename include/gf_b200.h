@@ -235,6 +235,20 @@ int gf_guided_gray_u8(const unsigned char* guide, const unsigned char* src, unsi
                       int64_t guide_stride, int64_t src_stride, int64_t dst_stride, int r, float eps, int border,
                       void* stream);
 
+/* The gray guided filter of gf_guided_gray_u8 on every channel of an 8-bit 3-channel image (CV_8UC3 src and dst):
+   guide_channels = 1 filters each source channel with the one gray guide (the class API's (1,3) mode,
+   GuidedFilter::init(w, h, 1, 3)); guide_channels = 3 filters source channel c with guide channel c (the (3,3) mode).
+   Channel c of dst is byte for byte what gf_guided_gray_u8 gives on the planes of channel c: the input is x/255, eps
+   on the [0,1] scale, the output saturate_cast<uchar>(cvRound(255 q)); any border.  Strides in ELEMENTS (= bytes),
+   0 = tightly packed (3 width, guide_channels width).  One launch of the s8 kernel, whose frames are the source
+   channels; gf_last_kernel() gives "s8u8_g1c3_r<r>" or "s8u8_g3c3_r<r>".  Served by that kernel only: r in {1..8, 16},
+   width >= 64, width and height >= 4r+2, every plane's base address and row stride 8-byte aligned, rows x stride
+   < 2^31, for TRUNCATE width % 8 == 0 and width >= 256, dst overlapping neither input; other arguments return
+   GF_ERR_UNSUPPORTED (guide_channels not 1 or 3 too), before anything is launched. */
+int gf_guided_per_channel_u8(const unsigned char* guide, const unsigned char* src, unsigned char* dst, int width, int height,
+                             int guide_channels, int64_t guide_stride, int64_t src_stride, int64_t dst_stride,
+                             int r, float eps, int border, void* stream);
+
 /* The colour-guide filter of gf_guided_color on 8-bit planes (a CV_8UC3 guide; a CV_8UC1 or CV_8UC3 source and
    destination of `src_channels` interleaved channels), with the same fused conversions: the input is x/255, the output
    saturate_cast<uchar>(cvRound(255 q)), eps on the [0,1] scale.  Strides in ELEMENTS (= bytes), 0 = tightly packed.
