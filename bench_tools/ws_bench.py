@@ -96,16 +96,6 @@ def main():
         jobs = [(e, c) for c in ((3840, 2160, 8), (7680, 4320, 8), (1920, 1080, 8), (16384, 8192, 8)) for e in (ws(12), ws(8), {"GF_WS": "0"})]
         jobs += [(ws(12), (3840, 2160, 8, 1)), (ws(12), (3840, 2160, 8, 2)), (ws(12), (3840, 2160, 16)), (ws(8), (3840, 2160, 16)),
                  ({"GF_WS": "0"}, (3840, 2160, 16)), (ws(12), (3840, 2160, 7)), (ws(8), (3840, 2160, 4)), ({"GF_WS": "0"}, (3840, 2160, 4))]
-    if len(sys.argv) > 1 and sys.argv[1] == "--split":         # producer split on / off, edge band weight
-        jobs = []
-        for c in ((3840, 2160, 8), (7680, 4320, 8), (1920, 1080, 8), (16384, 8192, 8)):
-            for k in (12, 8):
-                for sp in (0, 1):
-                    jobs.append(({"GF_WS": "1", "GF_WS_K": str(k), "GF_WS_SPLIT1": str(sp)}, c))
-        for pct in (100, 120, 150):
-            jobs.append(({"GF_WS": "1", "GF_WS_K": "12", "GF_WS_SPLIT1": "1", "GF_WS_EDGE_PCT": str(pct)}, (3840, 2160, 8)))
-        jobs += [({"GF_WS": "1", "GF_WS_SPLIT1": "1"}, (3840, 2160, 16)), ({"GF_WS": "1", "GF_WS_SPLIT1": "1", "GF_WS_K": "8"}, (3840, 2160, 16)),
-                 ({"GF_WS": "1", "GF_WS_SPLIT1": "1"}, (3840, 2160, 4)), ({"GF_WS": "1", "GF_WS_SPLIT1": "1"}, (3840, 2160, 8, 1))]
     extra_args = []
     if len(sys.argv) > 1 and sys.argv[1] == "--ab":            # jobs that write the a / b planes (hGuidedFilter through the shim)
         extra_args = ["--ab"]

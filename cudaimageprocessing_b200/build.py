@@ -65,7 +65,7 @@ def _compile_and_link(out: str, defines: list[str]) -> tuple[int, str]:
 
 
 def build_variant(name: str, defines: list[str]) -> str:
-    """Developer tool: a differently configured build (e.g. -DGF_S8_NEWTON=0) next to the product
+    """Developer tool: a differently configured build (e.g. -DGF_WS_TIMING) next to the product
     library, for A/B timing through GF_LIB_PATH (bench_tools/ab.py).  Never loaded by default."""
     out = os.path.join(PKG, name)
     rc, text = _compile_and_link(out, defines)

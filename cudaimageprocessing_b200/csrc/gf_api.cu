@@ -817,33 +817,6 @@ __global__ void __launch_bounds__(256) gf_halo_pull_kernel(const GfHaloPullArgs 
 #endif
 
 // ---- row strips with the halo exchange inside the call (SURVEY 8(b): gf_run_strips) ------------------------
-#ifndef GF_CPU_EMU
-namespace {
-// one side stream + fork/join events per device for the interior bands of gf_run_strips; the lock covers the enqueue
-struct StripSide {
-    std::mutex mu;
-    cudaStream_t s = nullptr;
-    cudaEvent_t e0 = nullptr, e1 = nullptr;
-    bool init = false;
-};
-StripSide g_strip_side[64];
-std::mutex g_strip_side_mu;
-StripSide* strip_side()
-{
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return nullptr;
-    StripSide* sd = &g_strip_side[dev];
-    std::lock_guard<std::mutex> lock(g_strip_side_mu);
-    if (!sd->init) {
-        if (cudaStreamCreateWithFlags(&sd->s, cudaStreamNonBlocking) != cudaSuccess) return nullptr;
-        if (cudaEventCreateWithFlags(&sd->e0, cudaEventDisableTiming) != cudaSuccess) return nullptr;
-        if (cudaEventCreateWithFlags(&sd->e1, cudaEventDisableTiming) != cudaSuccess) return nullptr;
-        sd->init = true;
-    }
-    return sd;
-}
-}  // namespace
-#endif
 static void strip_halo_rows(int global_height, int y0, int rows, int r, int* top, int* bot)
 {
     *top = y0 > 0 ? (2 * r < y0 ? 2 * r : y0) : 0;
@@ -897,8 +870,9 @@ int gf_run_strips(float* guide_buf, float* src_buf, float* dst, int width, int g
         add(guide_buf + off * gs, gs, down->guide, down->guide_stride, down->top, bot);
         add(src_buf + off * ss, ss, down->src, down->src_stride, down->top, bot);
     }
-    auto pull = [&](void* on) -> int {
-        if (nreg == 0) return GF_OK;
+    // The pull goes first on the caller's stream, then the whole strip in one launch.  (Filtering the rows that read no
+    // halo while the pull runs measured slower: DESIGN.md section 6.)
+    if (nreg > 0) {
 #ifndef GF_CPU_EMU
         for (int i = nreg; i < 4; ++i) { pa.dst[i] = nullptr; pa.src[i] = nullptr; pa.dstride[i] = pa.sstride[i] = 0; pa.rows[i] = 0; }
         pa.width = width;
@@ -910,7 +884,7 @@ int gf_run_strips(float* guide_buf, float* src_buf, float* dst, int width, int g
         gf_rt_device_info(&sms, &mj, &mn);
         dim3 grid(sms, nreg), block(256);
         auto k = gf_halo_pull_kernel;
-        GF_LAUNCH(k, grid, block, 0, on, pa);
+        GF_LAUNCH(k, grid, block, 0, stream, pa);
         if (const char* le = gf_rt_launch_error()) return fail(GF_ERR_CUDA, "gf_run_strips: halo pull kernel: %s", le);
         g_launches++;
 #else
@@ -918,59 +892,8 @@ int gf_run_strips(float* guide_buf, float* src_buf, float* dst, int width, int g
             for (int y = 0; y < pa.rows[i]; ++y)
                 std::memcpy(pa.dst[i] + y * pa.dstride[i], pa.src[i] + y * pa.sstride[i], (size_t)width * sizeof(float));
 #endif
-        return GF_OK;
-    };
-    Job j = strip_job(guide_buf, src_buf, dst, width, global_height, y0 - top, top + rows + bot, y0, rows, gs, ss, dst_stride, r, eps, border, stream);
-    // OPTION GF_STRIP_OVERLAP=1 (off by default: measured slower): exchange off the critical path.  Only the first and the
-    // last 2r OUTPUT rows of the strip read halo rows, so the strip is filtered in three jobs: rows [2r, rows-2r) on the
-    // caller's stream at once; the pull and then the two 2r-row seam jobs on a side stream.
-    // Measured (32768-column strips of 4096 rows, r = 16; profiles/r2_strip_overlap_8gpu.jsonl, r2_strip_phases.jsonl):
-    //   8 GPUs   pull-then-launch 0.967 ms   this option 0.992 ms
-    //   1 GPU, neighbours faked on the same GPU: main job alone 0.913 ms, both seam jobs alone 0.099 ms, main + seams
-    //   together 0.947 ms, everything 0.956 ms, against 0.932 ms for pull-then-launch.
-    // The seam jobs pay a 4r-row ramp for 2r output rows (4.5 % more row iterations), and the slots the main job leaves
-    // idle (s8_r16 keeps 4 warps per SM: 171 column strips x 3 bands = 513 of 592) are not free: a fourth warp on an SM
-    // slows the other three (profiles/r2_s8_residency.jsonl), so hiding a 0.02-0.04 ms pull costs 0.034 ms.  The other
-    // split that was tried -- first and last BAND of every column strip after the pull, the middle bands before it --
-    // lost by more (1.02-1.04 ms): with 3 bands per strip two of them wait for the pull.
-    const int cut_top = (up && top > 0) ? 2 * r : 0, cut_bot = (down && bot > 0) ? 2 * r : 0;
-    const int min_main = GF_KNOB("GF_STRIP_MIN_MAIN_ROWS", 16 * r + 64);
-    if (nreg > 0 && GF_KNOB("GF_STRIP_OVERLAP", 0) && rows - cut_top - cut_bot >= min_main && check_common(j) == GF_OK &&
-        !overlaps(j.dst, j.out_rows, j.guide, j.buf_rows, 1) && !overlaps(j.dst, j.out_rows, j.src, j.buf_rows, 1)) {
-        const int64_t dstr = or_packed(dst_stride, width, 1);
-        void* side = stream;
-#ifndef GF_CPU_EMU
-        StripSide* sd = strip_side();
-        if (!sd) return fail(GF_ERR_CUDA, "gf_run_strips: side stream");
-        std::lock_guard<std::mutex> lock(sd->mu);
-        side = sd->s;
-        if (cudaEventRecord(sd->e0, (cudaStream_t)stream) != cudaSuccess || cudaStreamWaitEvent(sd->s, sd->e0, 0) != cudaSuccess)
-            return fail(GF_ERR_CUDA, "gf_run_strips: fork");
-#endif
-        auto part = [&](int first, int n, void* on) -> int {       // output rows [first, first + n) of the strip
-            if (n <= 0) return GF_OK;
-            Job p = j;
-            p.out_y0 = y0 + first; p.out_rows = n; p.stream = on;
-            p.dst.ptr = dst + (int64_t)first * dstr;
-            return run_jobs(&p, 1);
-        };
-#ifdef GF_STRIP_DEBUG   // timing builds only (bench_tools/strip_phases.py): parts can be left out, the pixels are then WRONG
-        const int skip = GF_KNOB("GF_STRIP_DEBUG_SKIP", 0);      // 1 no main job, 2 no pull, 4 no seam jobs
-#else
-        const int skip = 0;
-#endif
-        int rc = (skip & 1) ? GF_OK : part(cut_top, rows - cut_top - cut_bot, stream);
-        if (rc == GF_OK && !(skip & 2)) rc = pull(side);
-        if (rc == GF_OK && !(skip & 4)) rc = part(0, cut_top, side);
-        if (rc == GF_OK && !(skip & 4)) rc = part(rows - cut_bot, cut_bot, side);
-#ifndef GF_CPU_EMU
-        // join even after an error: the caller's stream must not run ahead of what was already queued on the side stream
-        if (cudaEventRecord(sd->e1, sd->s) != cudaSuccess || cudaStreamWaitEvent((cudaStream_t)stream, sd->e1, 0) != cudaSuccess)
-            return rc ? rc : fail(GF_ERR_CUDA, "gf_run_strips: join");
-#endif
-        return rc;
     }
-    if (int rc = pull(stream)) return rc;
+    Job j = strip_job(guide_buf, src_buf, dst, width, global_height, y0 - top, top + rows + bot, y0, rows, gs, ss, dst_stride, r, eps, border, stream);
     return run_jobs(&j, 1);
 }
 

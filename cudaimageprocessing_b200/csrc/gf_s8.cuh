@@ -28,26 +28,6 @@
 #pragma once
 #include "gf_wp.cuh"
 
-#ifndef GF_S8_NEWTON
-#define GF_S8_NEWTON 1        // one Newton step after MUFU.RCP
-#endif
-#ifndef GF_S8_RESEED2
-#define GF_S8_RESEED2 1       // re-seed the stage-2 running sums from pure additions every 2R+1 rows
-#endif
-#ifndef GF_S8_RESEED1
-#define GF_S8_RESEED1 1       // same for the four stage-1 column sums
-#endif
-// Developer ablations (timing experiments only -- results are WRONG with any of them set):
-#ifndef GF_S8_ABL
-#define GF_S8_ABL 0           // bit 0: no shuffles, bit 1: no ring traffic, bit 2: no steady-state loads, bit 3: no stores
-#endif
-#if GF_S8_ABL & 1
-#define GF_S8_SHFL_UP(v, d) (v)
-#define GF_S8_SHFL_DOWN(v, d) (v)
-#else
-#define GF_S8_SHFL_UP(v, d) __shfl_up_sync(0xffffffffu, v, d)
-#define GF_S8_SHFL_DOWN(v, d) __shfl_down_sync(0xffffffffu, v, d)
-#endif
 #ifndef GF_S8_EDGE_PCT
 #define GF_S8_EDGE_PCT 85     // band height of the two edge strips (mirror loads, clipped counts, column map), % of the interior strips'
 #endif
@@ -204,7 +184,7 @@ __device__ __forceinline__ void gf_s8_window_m8(const float2 (&c)[4], float2 (&w
     // totals of the following lanes: tn[d] = T(l+d)
     float tn[2 * M];
 #pragma unroll
-    for (int d = 1; d <= 2 * M - 1; ++d) tn[d] = GF_S8_SHFL_DOWN(p[7], d);
+    for (int d = 1; d <= 2 * M - 1; ++d) tn[d] = __shfl_down_sync(0xffffffffu, p[7], d);
     float e = tn[1];
 #pragma unroll
     for (int d = 2; d <= 2 * M - 1; ++d) e += tn[d];
@@ -215,9 +195,9 @@ __device__ __forceinline__ void gf_s8_window_m8(const float2 (&c)[4], float2 (&w
     a[1] = x[1] + a[2]; a[0] = t01 + a[2];
     float l[8], r[8];
 #pragma unroll
-    for (int j = 0; j < 8; ++j) l[j] = GF_S8_SHFL_UP(a[j], M);
+    for (int j = 0; j < 8; ++j) l[j] = __shfl_up_sync(0xffffffffu, a[j], M);
 #pragma unroll
-    for (int j = 0; j < 7; ++j) r[j] = GF_S8_SHFL_DOWN(p[j], M);
+    for (int j = 0; j < 7; ++j) r[j] = __shfl_down_sync(0xffffffffu, p[j], M);
     r[7] = tn[M];
 #pragma unroll
     for (int i = 0; i < 4; ++i) w[i] = gf_add2(make_float2(l[2 * i], l[2 * i + 1]), make_float2(r[2 * i], r[2 * i + 1]));
@@ -400,11 +380,13 @@ __device__ __forceinline__ float gf_s8_cnt_y(int y, int height)
     return (float)(hi - lo + 1 > 0 ? hi - lo + 1 : 1);
 }
 
+// Every 2R+1 rows the running sums restart from sums of pure additions (reseed1: the four stage-1 column sums,
+// reseed2: the stage-2 sums), so that their drift does not grow with the band height.
 // c = f, f = 0: f holds exactly the rows of the current window, summed without a subtraction
 template <int R, class T, int GC, int PC>
 __device__ __forceinline__ void gf_s8_reseed1(GfS8Ctx<R, T, GC, PC>& c)
 {
-    if (!GF_S8_RESEED1 || sizeof(T) != 4) return;
+    if (sizeof(T) != 4) return;
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
         c.cI[i] = c.fI[i]; c.cP[i] = c.fP[i]; c.cIP[i] = c.fIP[i]; c.cII[i] = c.fII[i];
@@ -414,7 +396,6 @@ __device__ __forceinline__ void gf_s8_reseed1(GfS8Ctx<R, T, GC, PC>& c)
 template <int R, class T, int GC, int PC>
 __device__ __forceinline__ void gf_s8_reseed2(GfS8Ctx<R, T, GC, PC>& c)
 {
-    if (!GF_S8_RESEED2) return;
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
         c.sA[i] = c.fA[i]; c.sB[i] = c.fB[i];
@@ -450,7 +431,7 @@ __device__ __forceinline__ void gf_s8_iter(GfS8Ctx<R, T, GC, PC>& c, int t, int 
         c.cP[i] = gf_add2(c.cP[i], gf_sub2(c.nP[i], c.oP[i]));
         c.cIP[i] = gf_fma2(gf_neg2(c.oI[i]), c.oP[i], gf_fma2(c.nI[i], c.nP[i], c.cIP[i]));
         c.cII[i] = gf_fma2(gf_neg2(c.oI[i]), c.oI[i], gf_fma2(c.nI[i], c.nI[i], c.cII[i]));
-        if (GF_S8_RESEED1 && sizeof(T) == 4) {       // (uint8 build: integer sums below 2^24 are exact)
+        if (sizeof(T) == 4) {       // (uint8 build: integer sums below 2^24 are exact)
             c.fI[i] = gf_add2(c.fI[i], c.nI[i]);
             c.fP[i] = gf_add2(c.fP[i], c.nP[i]);
             c.fIP[i] = gf_fma2(c.nI[i], c.nP[i], c.fIP[i]);
@@ -458,25 +439,23 @@ __device__ __forceinline__ void gf_s8_iter(GfS8Ctx<R, T, GC, PC>& c, int t, int 
         }
     }
     // rows of the next iteration, consumed at the top of it
-    if (!(GF_S8_ABL & 4)) {
-        gf_s8_ld_row<MODE>(c, yi + 1, c.nI, c.nP, c.sc[0], c.sc[1]);
-        gf_s8_ld_row<MODE>(c, yi + 1 - KW, c.oI, c.oP, c.sc[2], c.sc[3]);
-        if (GF_S8_PF > 0 && MODE <= 1 && lane < 8) {
-            // L2 prefetch hint a few rows ahead: 8 lanes x one 128-byte line = the warp's 256 columns.
-            // (Measured: +3% over no hint; a hint per 32-byte sector from all 32 lanes is 10% SLOWER.)
-            const int rp = yi + 1 + GF_S8_PF;
-            if (rp <= c.buf_ylast) {
-                const int op = rp - c.buf_y0;
-                constexpr int LINE = 128 / (int)sizeof(T);      // elements per 128-byte line
-                if (GC == PC) {
-                    if (lane * LINE < 256 * PC) {
-                        gf_prefetch_l2(c.gI + op * c.gs + (LINE - 8 * GC) * lane);
-                        gf_prefetch_l2(c.gP + op * c.ss + (LINE - 8 * PC) * lane);
-                    }
-                } else {                                    // a gray guide spans 1/3 of the lines of a 3-channel source
-                    if (lane * LINE < 256 * GC) gf_prefetch_l2(c.gI + op * c.gs + (LINE - 8 * GC) * lane);
-                    if (lane * LINE < 256 * PC) gf_prefetch_l2(c.gP + op * c.ss + (LINE - 8 * PC) * lane);
+    gf_s8_ld_row<MODE>(c, yi + 1, c.nI, c.nP, c.sc[0], c.sc[1]);
+    gf_s8_ld_row<MODE>(c, yi + 1 - KW, c.oI, c.oP, c.sc[2], c.sc[3]);
+    if (GF_S8_PF > 0 && MODE <= 1 && lane < 8) {
+        // L2 prefetch hint a few rows ahead: 8 lanes x one 128-byte line = the warp's 256 columns.
+        // (Measured: +3% over no hint; a hint per 32-byte sector from all 32 lanes is 10% SLOWER.)
+        const int rp = yi + 1 + GF_S8_PF;
+        if (rp <= c.buf_ylast) {
+            const int op = rp - c.buf_y0;
+            constexpr int LINE = 128 / (int)sizeof(T);      // elements per 128-byte line
+            if (GC == PC) {
+                if (lane * LINE < 256 * PC) {
+                    gf_prefetch_l2(c.gI + op * c.gs + (LINE - 8 * GC) * lane);
+                    gf_prefetch_l2(c.gP + op * c.ss + (LINE - 8 * PC) * lane);
                 }
+            } else {                                    // a gray guide spans 1/3 of the lines of a 3-channel source
+                if (lane * LINE < 256 * GC) gf_prefetch_l2(c.gI + op * c.gs + (LINE - 8 * GC) * lane);
+                if (lane * LINE < 256 * PC) gf_prefetch_l2(c.gP + op * c.ss + (LINE - 8 * PC) * lane);
             }
         }
     }
@@ -485,7 +464,7 @@ __device__ __forceinline__ void gf_s8_iter(GfS8Ctx<R, T, GC, PC>& c, int t, int 
         float2 hA[4], hB[4];
         gf_s8_window<R>(c.va, hA, lane);
         gf_s8_window<R>(c.vb, hB, lane);
-        if (c.ring_lane && !(GF_S8_ABL & 2)) {
+        if (c.ring_lane) {
             float2* s = c.ring + slot * G::SLOT_F2;
             if (full) {
 #pragma unroll
@@ -500,10 +479,8 @@ __device__ __forceinline__ void gf_s8_iter(GfS8Ctx<R, T, GC, PC>& c, int t, int 
 #pragma unroll
             for (int i = 0; i < 4; ++i) { s[i * VL] = hA[i]; s[(4 + i) * VL] = hB[i]; }
         }
-        if (GF_S8_RESEED2) {
 #pragma unroll
-            for (int i = 0; i < 4; ++i) { c.fA[i] = gf_add2(c.fA[i], hA[i]); c.fB[i] = gf_add2(c.fB[i], hB[i]); }
-        }
+        for (int i = 0; i < 4; ++i) { c.fA[i] = gf_add2(c.fA[i], hA[i]); c.fB[i] = gf_add2(c.fB[i], hB[i]); }
         if (full) {                                     // q of row yo = yi-1-2R; its guide row is oI
             const int yo = yi - 1 - 2 * R;
             float2 q[4];
@@ -525,7 +502,7 @@ __device__ __forceinline__ void gf_s8_iter(GfS8Ctx<R, T, GC, PC>& c, int t, int 
                 }
             }
             T* pq = c.gQ + (yo - c.out_y0) * c.ds;
-            if (c.out_lane && !(GF_S8_ABL & 8)) {
+            if (c.out_lane) {
                 if (!XMAP || c.vec_ok) {
                     if constexpr (PC == 3) gf_st8x3(pq, q);
                     else gf_st8(pq, q);
@@ -584,10 +561,8 @@ __device__ __forceinline__ void gf_s8_iter(GfS8Ctx<R, T, GC, PC>& c, int t, int 
             const float2 nnum = gf_fma2(hI[i], hP[i], gf_mul2(hIP[i], mN));           // -(numerator)
             const float2 nden = gf_fma2(hI[i], hI[i], gf_fma2(hII[i], mN, mE));       // -(denominator) < 0
             float2 rc = make_float2(gf_s8_rcp(nden.x), gf_s8_rcp(nden.y));
-            if (GF_S8_NEWTON) {
-                const float2 e = gf_fma2(gf_neg2(nden), rc, gf_dup2(1.0f));
-                rc = gf_fma2(e, rc, rc);
-            }
+            const float2 e = gf_fma2(gf_neg2(nden), rc, gf_dup2(1.0f));     // one Newton step after MUFU.RCP
+            rc = gf_fma2(e, rc, rc);
             const float2 aa = gf_mul2(nnum, rc);
             const float2 bn = gf_fma2(gf_neg2(aa), hI[i], hP[i]);                      // N * b
             c.va[i] = aa;

@@ -22,30 +22,17 @@
 //     rows (loads + adds) remain per stream;
 //   * where it fits (GfWsGeom::TMEM), a producer keeps its last 2R+1 input rows in tensor memory and reads the row that
 //     leaves its vertical window back from there: per row it loads only the entering row from L2.
-// Hand-off: monotonic row counters in shared memory (st.release / ld.acquire at CTA scope, nanosleep
-// back-off); the ring has 2R+2 rows, a producer waits only when its consumer is a full row behind.
+// Hand-off: one mbarrier per ring slot (producer -> consumer: the row is in the slot) and a monotonic
+// consumed-rows counter in shared memory (consumer -> producer); the ring has 2R+2 rows, a producer waits
+// only when its consumer is a full row behind.
 // Numerics: additions only inside a window (prefix + suffix, no subtraction of prefixes); the vertical
 // sums slide (add the entering row, subtract the leaving one) over at most GF_WS_MAX_SUB rows per stream
 // before the band is cut (random-walk drift ~1e-7 per 100 rows on [0,1] data; measured in the tests).
-// Borders: the vertical rule is a row map (TRUNCATE: zero rows + counts); horizontally, lanes that lie
-// (partly) outside the image gather their columns through a per-lane column map (the first and last
-// strip only), so mirrored inputs give mirrored a, b and nothing else changes.
+// Borders: the vertical rule is a row map (TRUNCATE: zero rows + counts); horizontally, the first and the
+// last strip mirror the producer's column sums across lanes (gf_ws_mirror), so mirrored inputs give
+// mirrored a, b and nothing else changes.
 #pragma once
 #include "gf_s8.cuh"
-
-#ifndef GF_WS_NEWTON
-#define GF_WS_NEWTON 1       // one Newton step after MUFU.RCP in the a/b solve
-#endif
-#ifndef GF_WS_SPLIT
-#define GF_WS_SPLIT 0        // prefix / suffix chains of the window sums in two halves: measured 1-2 % SLOWER (r2_ws_variants.jsonl)
-#endif
-#ifndef GF_WS_PF
-#define GF_WS_PF 0           // rows ahead for an L2 prefetch hint of the entering row; measured 4-6 % SLOWER at 4K/8K
-                             // (profiles/r2_ws_variants.jsonl), so off
-#endif
-#ifndef GF_WS_NORM2
-#define GF_WS_NORM2 1        // two-term reciprocal of the pixel count (see GfNorm)
-#endif
 
 struct GfWsArgs {
     const float* guide; const float* src; float* dst; float* A; float* B;
@@ -70,8 +57,11 @@ struct GfWsGeom {
     static constexpr int RING = 2 * R + 2;               // a/b rows per stream
     static constexpr int ROW_F4 = (K / 2) * 32;          // float4 per ring row: [pair of columns][lane] = (a0, b0, a1, b1)
     static constexpr size_t ring_bytes = (size_t)RING * ROW_F4 * 16;
-    static constexpr int NBAR = 2 * RING + 1;            // mbarriers per stream: row ready + products ready per ring slot, "stream finished"
-    static constexpr size_t ctrl_bytes = 64 + (size_t)NS * NBAR * 8;      // 2 NS row counters + the mbarriers
+    // control block: 2 NS ints (ctrl[2k + 1]: stream k's consumed-rows counter), then NBAR mbarriers per stream (row ready
+    // per ring slot, RING spare, "stream finished").  ctrl[2k] and the spare barriers are unused; they keep the layout
+    // the kernels were tuned with.
+    static constexpr int NBAR = 2 * RING + 1;
+    static constexpr size_t ctrl_bytes = 64 + (size_t)NS * NBAR * 8;
     static constexpr size_t smem_bytes = (size_t)NS * ring_bytes + (ctrl_bytes + 127) / 128 * 128;
     static constexpr int MIN_SUB = R + 1;                // shortest sub-band whose neighbours can share rows with it
     // The producer's last 2R+1 input rows (K columns of I, then K of p) in tensor memory, so that the leaving row comes
@@ -86,17 +76,12 @@ struct GfWsGeom {
 };
 
 // ---- hand-off primitives --------------------------------------------------------------------------
-// GF_WS_SYNC: how a consumer learns that an a/b row is in the ring.
-//   2 (default)  one mbarrier per ring slot (phase = use count of the slot): the producer's lane 0 arrives
-//                (release at CTA scope, no MEMBAR), consumers sleep in mbarrier.try_wait (hardware wake-up);
-//   1            monotonic row counter, st.release / ld.acquire, consumers spin;
-//   0            same counter with a nanosleep back-off (first version: the sleep quantum turned out to be
-//                longer than a row, profiles/r2_ws_sync_variants.jsonl).
-// The consumed-rows counter (consumer -> producer) is a counter in every variant: a producer reads it once
-// per row and practically never has to wait (the consumer releases a ring row as soon as it is in registers).
-#ifndef GF_WS_SYNC
-#define GF_WS_SYNC 2
-#endif
+// A consumer learns that an a/b row is in the ring from one mbarrier per ring slot (phase = use count of the
+// slot): the producer's lane 0 arrives (release at CTA scope, no MEMBAR), consumers sleep in mbarrier.try_wait
+// (hardware wake-up).  Row counters with st.release / ld.acquire, spinning or with a nanosleep back-off, timed
+// the same and were removed (DESIGN.md section 3.3).
+// The consumed-rows counter (consumer -> producer) is a plain counter: a producer reads it once per row and
+// practically never has to wait (the consumer releases a ring row as soon as it is in registers).
 #ifdef GF_CPU_EMU
 static inline int gf_ws_ld_acq(const volatile int* p) { return *p; }
 static inline void gf_ws_st_rel(volatile int* p, int v) { *p = v; }
@@ -119,12 +104,7 @@ __device__ __forceinline__ void gf_ws_st_rel(volatile int* p, int v)
 {
     asm volatile("st.release.cta.shared.s32 [%0], %1;" ::"r"((unsigned)__cvta_generic_to_shared(const_cast<int*>(p))), "r"(v) : "memory");
 }
-__device__ __forceinline__ void gf_ws_pause()
-{
-#if GF_WS_SYNC == 0
-    __nanosleep(32);
-#endif
-}
+__device__ __forceinline__ void gf_ws_pause() {}
 __device__ __forceinline__ void gf_ws_bar_init(unsigned long long* b)
 {
     asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"((unsigned)__cvta_generic_to_shared(b)) : "memory");
@@ -235,30 +215,21 @@ __device__ __forceinline__ void gf_ws_publish(volatile int* ctr, int val, int la
     __syncwarp();                       // every lane's ring accesses are ordered before lane 0's release
     if (lane == 0) gf_ws_st_rel(ctr, val);
 }
-// row `idx` (count from the stream's first own row) of a stream is in its ring
-template <int RING>
-__device__ __forceinline__ void gf_ws_row_ready(volatile int* prod, unsigned long long* bars, int idx, int slot, int lane)
+// the a/b row in ring slot `slot` of a stream is complete
+__device__ __forceinline__ void gf_ws_row_ready(unsigned long long* bars, int slot, int lane)
 {
-#if GF_WS_SYNC == 2
     __syncwarp();
     if (lane == 0) gf_ws_bar_arrive(bars + slot);
-#else
-    gf_ws_publish(prod, idx + 1, lane);
-#endif
 }
 // `last_rows`: the row is one of the LAST rows of another stream (the neighbour across a shared end).  A slot
 // barrier only tells phase p from p-1 (one parity bit): a consumer that arrives while that producer is still more
 // than a ring behind would take the completion of phase p-1 for phase p.  Those rows wait for the producer's
 // "stream finished" barrier instead (its last row is the first one needed anyway).
 template <int RING>
-__device__ __forceinline__ void gf_ws_row_wait(const volatile int* prod, const unsigned long long* bars, int idx, bool last_rows)
+__device__ __forceinline__ void gf_ws_row_wait(const unsigned long long* bars, int idx, bool last_rows)
 {
-#if GF_WS_SYNC == 2
     if (last_rows) gf_ws_bar_wait(bars + 2 * RING, 0);
     else gf_ws_bar_wait(bars + idx % RING, idx / RING);
-#else
-    gf_ws_wait(prod, idx + 1);
-#endif
 }
 
 // ---- (2R+1)-window sums of K adjacent columns per lane, on packed quantity pairs --------------------
@@ -280,30 +251,12 @@ template <int K, int R>
 __device__ __forceinline__ void gf_ws_window(const float2 (&v)[K], float2 (&w)[K])
 {
     float2 P[K], S[K];
-#if GF_WS_SPLIT
-    // two half-length chains per direction instead of one (dependency depth K/2 + 1 instead of K - 1; K/2 more
-    // additions): a lone producer warp per scheduler otherwise waits on FADD2 latency at every step
-    constexpr int HF = K / 2;
-    P[0] = v[0];
-    P[HF] = v[HF];
-#pragma unroll
-    for (int j = 1; j < HF; ++j) { P[j] = gf_add2(P[j - 1], v[j]); P[HF + j] = gf_add2(P[HF + j - 1], v[HF + j]); }
-#pragma unroll
-    for (int j = HF; j < K; ++j) P[j] = gf_add2(P[j], P[HF - 1]);
-    S[K - 1] = v[K - 1];
-    S[HF - 1] = v[HF - 1];
-#pragma unroll
-    for (int j = 1; j < HF; ++j) { S[K - 1 - j] = gf_add2(S[K - j], v[K - 1 - j]); S[HF - 1 - j] = gf_add2(S[HF - j], v[HF - 1 - j]); }
-#pragma unroll
-    for (int j = 0; j < HF; ++j) S[j] = gf_add2(S[j], S[HF]);
-#else
     P[0] = v[0];
 #pragma unroll
     for (int j = 1; j < K; ++j) P[j] = gf_add2(P[j - 1], v[j]);
     S[K - 1] = v[K - 1];
 #pragma unroll
     for (int j = K - 2; j >= 0; --j) S[j] = gf_add2(S[j + 1], v[j]);
-#endif
     constexpr int CM = (R + K - 1) / K;      // farthest lane a window reaches
     // cumulative totals of the c nearest lanes on either side (only when R > K)
     float2 TL[CM + 1], TR[CM + 1];
@@ -407,19 +360,15 @@ __host__ __device__ inline void gf_ws_plan(int y0, int y1, int pen, GfWsPlan<NS>
 // ---- stage 1: producer warp -------------------------------------------------------------------------
 // EM: 0 the strip window lies inside the image, 1 it overhangs the left edge by exactly HALO columns, 2 the right
 // edge by exactly HALO (the last strip is placed that way), 3 anything else: per-column map + gathered loads.
-// ROLE: 0 one producer warp per stream; 1 / 2 the producer split over TWO warps (3 warps per scheduler instead of 2,
-// each with half the dependent chain): warp 2 owns Y = (sum Ip, sum II), its window sums go into the ring slot of the
-// row (the slot is free by then); warp 1 owns X = (sum I, sum p), picks the Y sums up from the slot, solves for a, b
-// and overwrites the slot with them.
-// tm: this producer's history in tensor memory (ROLE 0 of the kernels with G::TMEM): input row t of the stream sits
-// in slot (t - t_first) mod (2R+1), where the row that leaves 2R+1 iterations later is read back.
-template <int R, int K, int NS, bool TRUNC, int EM, int ROLE>
+// tm: this producer's history in tensor memory (kernels with G::TMEM): input row t of the stream sits in slot
+// (t - t_first) mod (2R+1), where the row that leaves 2R+1 iterations later is read back.
+template <int R, int K, int NS, bool TRUNC, int EM>
 __device__ __forceinline__ void gf_ws_stage1(const GfWsArgs& a, const GfWsPlan<NS>& pl, int k, int lane, int64_t f, int xl,
                                              int out_lo, int out_hi, float4* rings, volatile int* ctrl, unsigned tm)
 {
     using G = GfWsGeom<R, K, NS>;
     constexpr int RING = G::RING, KW = G::KW;
-    constexpr bool HIST = ROLE == 0 && G::TMEM;
+    constexpr bool HIST = G::TMEM;
     const GfWsStream st = pl.s[k];
     float4* ring = rings + (size_t)k * RING * G::ROW_F4 + lane;
     const int x0 = xl + lane * K;
@@ -459,19 +408,6 @@ __device__ __forceinline__ void gf_ws_stage1(const GfWsArgs& a, const GfWsPlan<N
         rr = rr < 0 ? 0 : (rr > rows_hi ? rows_hi : rr);
         return rr;
     };
-    // L2 prefetch hint for the row that enters GF_WS_PF iterations from now: one 128-byte line per lane and plane
-    auto prefetch_row = [&](int t) {
-        if (GF_WS_PF == 0 || EM == 3) return;
-        if (lane * 32 < G::WIN) {
-            int rr = row_of(t);
-            if (!simple) { if (TRUNC && rr < 0) return; }
-            const int64_t c0 = (int64_t)xl + lane * 32;
-            if (c0 >= 0 && c0 + 32 <= a.width) {
-                gf_prefetch_l2(gI + (int64_t)rr * a.gs + c0);
-                gf_prefetch_l2(gP + (int64_t)rr * a.ss + c0);
-            }
-        }
-    };
     // the K columns of this lane from a row pointer that already points at the lane's first column
     auto ld_vec = [&](const float* rp, float (&v)[K]) {
             if (EM == 1 || EM == 2) {      // edge strip: groups outside the image are not read (their sums are mirrored in)
@@ -505,6 +441,8 @@ __device__ __forceinline__ void gf_ws_stage1(const GfWsArgs& a, const GfWsPlan<N
         }
         const int64_t ro = (int64_t)rr * stride;
         if (vec) {
+            // the loads of ld_vec, written out: a call to ld_vec here (as a lambda or a function, in any arrangement of
+            // the branches tried) costs the K = 8 TRUNCATE kernels 16 more instructions
             const float* rp = planex + ro;
             if (EM == 1 || EM == 2) {      // edge strip: groups outside the image are not read (their sums are mirrored in)
 #pragma unroll
@@ -559,11 +497,9 @@ __device__ __forceinline__ void gf_ws_stage1(const GfWsArgs& a, const GfWsPlan<N
                 if (HIST) gf_tm_st_row<K>(tm + (t0 + q - t_first) * G::TM_ROW, bI[q], bP[q]);
 #pragma unroll
                 for (int j = 0; j < K; ++j) {
-                    if (ROLE != 2) { X[j].x += bI[q][j]; X[j].y += bP[q][j]; }
-                    if (ROLE != 1) {
-                        Y[j].x = fmaf(bI[q][j], bP[q][j], Y[j].x);
-                        Y[j].y = fmaf(bI[q][j], bI[q][j], Y[j].y);
-                    }
+                    X[j].x += bI[q][j]; X[j].y += bP[q][j];
+                    Y[j].x = fmaf(bI[q][j], bP[q][j], Y[j].x);
+                    Y[j].y = fmaf(bI[q][j], bI[q][j], Y[j].y);
                 }
             }
         }
@@ -592,7 +528,6 @@ __device__ __forceinline__ void gf_ws_stage1(const GfWsArgs& a, const GfWsPlan<N
     const float Nf = (float)(KW * KW);
     const float epsNN = a.eps * Nf * Nf;
     const GfNorm nk = gf_norm_make(Nf);
-    volatile int* prod = ctrl + 2 * k;
     unsigned long long* bars = reinterpret_cast<unsigned long long*>(const_cast<int*>(ctrl) + 16);
     const volatile int* cons_own = ctrl + 2 * k + 1;
     const volatile int* cons_sp = ctrl + 2 * (st.sp >= 0 ? st.sp : k) + 1;
@@ -604,21 +539,17 @@ __device__ __forceinline__ void gf_ws_stage1(const GfWsArgs& a, const GfWsPlan<N
 #pragma unroll 1
     for (int m = st.m0; m < st.m1; ++m) {
         // ---- vertical: row m+R enters, row m-R-1 leaves ----
-        if (ROLE != 2) {
 #pragma unroll
-            for (int c = 0; c < K / 2; ++c) {      // (entering - leaving) on the column pairs the loads deliver: FADD2
-                const float2 dI = gf_sub2(make_float2(nI[2 * c], nI[2 * c + 1]), make_float2(oI[2 * c], oI[2 * c + 1]));
-                const float2 dP = gf_sub2(make_float2(nP[2 * c], nP[2 * c + 1]), make_float2(oP[2 * c], oP[2 * c + 1]));
-                X[2 * c].x += dI.x; X[2 * c + 1].x += dI.y;
-                X[2 * c].y += dP.x; X[2 * c + 1].y += dP.y;
-            }
+        for (int c = 0; c < K / 2; ++c) {      // (entering - leaving) on the column pairs the loads deliver: FADD2
+            const float2 dI = gf_sub2(make_float2(nI[2 * c], nI[2 * c + 1]), make_float2(oI[2 * c], oI[2 * c + 1]));
+            const float2 dP = gf_sub2(make_float2(nP[2 * c], nP[2 * c + 1]), make_float2(oP[2 * c], oP[2 * c + 1]));
+            X[2 * c].x += dI.x; X[2 * c + 1].x += dI.y;
+            X[2 * c].y += dP.x; X[2 * c + 1].y += dP.y;
         }
-        if (ROLE != 1) {
 #pragma unroll
-            for (int j = 0; j < K; ++j) {
-                Y[j].x = fmaf(-oI[j], oP[j], fmaf(nI[j], nP[j], Y[j].x));
-                Y[j].y = fmaf(-oI[j], oI[j], fmaf(nI[j], nI[j], Y[j].y));
-            }
+        for (int j = 0; j < K; ++j) {
+            Y[j].x = fmaf(-oI[j], oP[j], fmaf(nI[j], nP[j], Y[j].x));
+            Y[j].y = fmaf(-oI[j], oI[j], fmaf(nI[j], nI[j], Y[j].y));
         }
         if (HIST) gf_tm_st_row<K>(tm + (hslot == 0 ? KW - 1 : hslot - 1) * G::TM_ROW, nI, nP);     // row m+R
         if (EM == 1 || EM == 2) {
@@ -629,17 +560,16 @@ __device__ __forceinline__ void gf_ws_stage1(const GfWsArgs& a, const GfWsPlan<N
             } else {
                 constexpr int CL0 = 2 * G::HALO, CR0 = 2 * (G::WIN - G::HALO - 1);
                 if (a.border == GF_REFLECT) {
-                    if (EM == 1) { if (ROLE != 2) gf_ws_mirror<K, CL0 - 1>(X, lane, oob); if (ROLE != 1) gf_ws_mirror<K, CL0 - 1>(Y, lane, oob); }
-                    else { if (ROLE != 2) gf_ws_mirror<K, CR0 + 1>(X, lane, oob); if (ROLE != 1) gf_ws_mirror<K, CR0 + 1>(Y, lane, oob); }
+                    if (EM == 1) { gf_ws_mirror<K, CL0 - 1>(X, lane, oob); gf_ws_mirror<K, CL0 - 1>(Y, lane, oob); }
+                    else { gf_ws_mirror<K, CR0 + 1>(X, lane, oob); gf_ws_mirror<K, CR0 + 1>(Y, lane, oob); }
                 } else {
-                    if (EM == 1) { if (ROLE != 2) gf_ws_mirror<K, CL0>(X, lane, oob); if (ROLE != 1) gf_ws_mirror<K, CL0>(Y, lane, oob); }
-                    else { if (ROLE != 2) gf_ws_mirror<K, CR0>(X, lane, oob); if (ROLE != 1) gf_ws_mirror<K, CR0>(Y, lane, oob); }
+                    if (EM == 1) { gf_ws_mirror<K, CL0>(X, lane, oob); gf_ws_mirror<K, CL0>(Y, lane, oob); }
+                    else { gf_ws_mirror<K, CR0>(X, lane, oob); gf_ws_mirror<K, CR0>(Y, lane, oob); }
                 }
             }
         }
         // ---- rows of the next iteration (a whole iteration to land) ----
-        if (ROLE != 1 && m + GF_WS_PF + 1 < st.m1) prefetch_row(m + 1 + R + GF_WS_PF);
-        const int cons_seen = ROLE != 1 ? gf_ws_ld_acq(cons_own) : 0;      // read early, needed just before the ring store
+        const int cons_seen = gf_ws_ld_acq(cons_own);      // read early, needed just before the ring store
         if (m + 1 < st.m1) {
             if (EM != 3 && simple) {       // rows never leave the image: running row pointers, no per-row address arithmetic
                 pnI += stepI; pnP += stepP;
@@ -664,36 +594,8 @@ __device__ __forceinline__ void gf_ws_stage1(const GfWsArgs& a, const GfWsPlan<N
         // ---- horizontal: window sums of the two quantity pairs ----
         const int idx = m - st.m0;
         float2 hX[K], hY[K];
-        if (ROLE != 2) gf_ws_window<K, R>(X, hX);
-        if (ROLE != 1) gf_ws_window<K, R>(Y, hY);
-        if (ROLE == 2) {
-            // products warp: wait until every consumer is done with the row the slot held, park the Y sums in it
-            if (idx >= RING) {
-                const int mm = m - RING;
-                const int use = mm + KW < n_last ? mm + KW : n_last;
-                if (cons_seen < use + R + 1) gf_ws_wait(cons_own, use + R + 1);
-                if (st.sp >= 0 && mm < R) {
-                    const int usep = 2 * R - mm < n_last_sp ? 2 * R - mm : n_last_sp;
-                    gf_ws_wait(cons_sp, usep + R + 1);
-                }
-            }
-            float4* rp = ring + slot * G::ROW_F4;
-#pragma unroll
-            for (int c = 0; c < K / 2; ++c) rp[c * 32] = make_float4(hY[2 * c].x, hY[2 * c].y, hY[2 * c + 1].x, hY[2 * c + 1].y);
-            __syncwarp();
-            if (lane == 0) gf_ws_bar_arrive(bars + k * G::NBAR + RING + slot);
-            slot = slot + 1 == RING ? 0 : slot + 1;
-            continue;
-        }
-        if (ROLE == 1) {
-            gf_ws_bar_wait(bars + k * G::NBAR + RING + slot, idx / RING);
-            const float4* rp = ring + slot * G::ROW_F4;
-#pragma unroll
-            for (int c = 0; c < K / 2; ++c) {
-                const float4 t = rp[c * 32];
-                hY[2 * c] = make_float2(t.x, t.y); hY[2 * c + 1] = make_float2(t.z, t.w);
-            }
-        }
+        gf_ws_window<K, R>(X, hX);
+        gf_ws_window<K, R>(Y, hY);
         // ---- a = (N S_Ip - S_I S_p) / (N S_II - S_I^2 + eps N^2),  bN = S_p - a S_I  (b = bN / N) ----
         float av[K], bv[K];
         if (TRUNC) {
@@ -724,13 +626,13 @@ __device__ __forceinline__ void gf_ws_stage1(const GfWsArgs& a, const GfWsPlan<N
                 const float2 t = gf_fma2(cN, hY[j], cE);
                 const float2 u = gf_fma2(make_float2(-hX[j].x, -hX[j].x), make_float2(hX[j].y, hX[j].x), t);
                 float rc = gf_s8_rcp(u.y);
-                if (GF_WS_NEWTON) rc = fmaf(fmaf(-u.y, rc, 1.0f), rc, rc);
+                rc = fmaf(fmaf(-u.y, rc, 1.0f), rc, rc);
                 av[j] = u.x * rc;
                 bv[j] = fmaf(-av[j], hX[j].x, hX[j].y);
             }
         }
         // ---- the ring slot of row m held row m-RING: every consumer of that row must be done with it ----
-        if (ROLE == 0 && idx >= RING) {
+        if (idx >= RING) {
             const int mm = m - RING;
             const int use = mm + KW < n_last ? mm + KW : n_last;          // last step of the own consumer that reads row mm
             if (cons_seen < use + R + 1) gf_ws_wait(cons_own, use + R + 1);
@@ -744,7 +646,7 @@ __device__ __forceinline__ void gf_ws_stage1(const GfWsArgs& a, const GfWsPlan<N
 #pragma unroll
             for (int c = 0; c < K / 2; ++c) rp[c * 32] = make_float4(av[2 * c], bv[2 * c], av[2 * c + 1], bv[2 * c + 1]);
         }
-        gf_ws_row_ready<RING>(prod, bars + k * G::NBAR, idx, slot, lane);
+        gf_ws_row_ready(bars + k * G::NBAR, slot, lane);
         slot = slot + 1 == RING ? 0 : slot + 1;
         // ---- optional A / B planes (hGuidedFilter's d_A, d_B): own territory rows, output columns ----
         if (a.A != nullptr && m >= 0 && m < st.L) {
@@ -773,7 +675,7 @@ __device__ __forceinline__ void gf_ws_stage1(const GfWsArgs& a, const GfWsPlan<N
     // "stream finished": every own row is in the ring, and the stream is done with its tensor memory (warp 0 frees it)
     if (HIST) gf_tm_fence_before();
     __syncwarp();
-    if (ROLE != 2 && lane == 0) gf_ws_bar_arrive(bars + k * G::NBAR + 2 * RING);
+    if (lane == 0) gf_ws_bar_arrive(bars + k * G::NBAR + 2 * RING);
 }
 
 // ---- stage 2: consumer warp -------------------------------------------------------------------------
@@ -804,15 +706,14 @@ __device__ __forceinline__ void gf_ws_stage2(const GfWsArgs& a, const GfWsPlan<N
     volatile int* cons = ctrl + 2 * k + 1;
     const int ep_last = st.ep >= 0 ? pl.s[st.ep].L - 1 - pl.s[st.ep].m0 + st.L : 0;    // ring index of row n >= L in the end partner: ep_last - n
 
-    // ring row and producer counter of stream-local a/b row n
+    // ring row and barriers of stream-local a/b row n
     const unsigned long long* bars = reinterpret_cast<const unsigned long long*>(const_cast<const int*>(ctrl) + 16);
-    auto resolve = [&](int n, const float4*& base, const volatile int*& prod, const unsigned long long*& bar, int& idx) {
+    auto resolve = [&](int n, const float4*& base, const unsigned long long*& bar, int& idx) {
         int t = k;
         idx = n - st.m0;
         if (n < 0 && st.sp >= 0) { t = st.sp; idx = -1 - n; }              // (a shared start: the partner's m0 is 0)
         else if (n >= st.L && st.ep >= 0) { t = st.ep; idx = ep_last - n; }
         base = rings + (t * RING + idx % RING) * G::ROW_F4 + lane;
-        prod = ctrl + 2 * t;
         bar = bars + t * G::NBAR;
     };
     const int64_t stepG = (int64_t)st.d * a.gs, stepQ = (int64_t)st.d * a.ds;
@@ -837,15 +738,15 @@ __device__ __forceinline__ void gf_ws_stage2(const GfWsArgs& a, const GfWsPlan<N
     const int n_last = st.L - 1 + R;
 #pragma unroll 1
     for (int n = -R; n <= n_last; ++n) {
-        const float4* nb; const volatile int* np; const unsigned long long* nbar; int ni;
-        resolve(n, nb, np, nbar, ni);
-        gf_ws_row_wait<RING>(np, nbar, ni, n >= st.L && st.ep >= 0);
+        const float4* nb; const unsigned long long* nbar; int ni;
+        resolve(n, nb, nbar, ni);
+        gf_ws_row_wait<RING>(nbar, ni, n >= st.L && st.ep >= 0);
         float4 nw[K / 2];
 #pragma unroll
         for (int c = 0; c < K / 2; ++c) nw[c] = nb[c * 32];
         if (n - KW >= -R) {
-            const float4* ob; const volatile int* op; const unsigned long long* obar; int oi;
-            resolve(n - KW, ob, op, obar, oi);
+            const float4* ob; const unsigned long long* obar; int oi;
+            resolve(n - KW, ob, obar, oi);
 #pragma unroll
             for (int c = 0; c < K / 2; ++c) {
                 const float4 o = ob[c * 32];
@@ -879,7 +780,7 @@ __device__ __forceinline__ void gf_ws_stage2(const GfWsArgs& a, const GfWsPlan<N
         } else {
 #pragma unroll
             for (int j = 0; j < K; ++j) {
-                const float2 m = GF_WS_NORM2 ? gf_fma2(W[j], nh, gf_mul2(W[j], nl)) : gf_mul2(W[j], nh);
+                const float2 m = gf_fma2(W[j], nh, gf_mul2(W[j], nl));
                 q[j] = fmaf(m.x, g[j], m.y);
             }
         }
@@ -895,10 +796,9 @@ __device__ __forceinline__ void gf_ws_stage2(const GfWsArgs& a, const GfWsPlan<N
 }
 
 // ---- kernel: one CTA = one (frame, strip, band) ---------------------------------------------------------
-// SPLIT = false: warps [0, NS) produce, [NS, 2 NS) consume.  SPLIT = true: [0, NS) sums + solve, [NS, 2 NS) products,
-// [2 NS, 3 NS) consume (warp w, NS + w, 2 NS + w of a 4-stream CTA share a scheduler).
-template <int R, int K, int NS, bool TRUNC, bool SPLIT>
-__global__ void __launch_bounds__((SPLIT ? 96 : 64) * NS, 1) gf_ws_gray_kernel(const GF_GRID_CONSTANT GfWsArgs a)
+// Warps [0, NS) produce, [NS, 2 NS) consume.
+template <int R, int K, int NS, bool TRUNC>
+__global__ void __launch_bounds__(64 * NS, 1) gf_ws_gray_kernel(const GF_GRID_CONSTANT GfWsArgs a)
 {
     using G = GfWsGeom<R, K, NS>;
     GF_DYN_SMEM(float4, smem);
@@ -918,7 +818,7 @@ __global__ void __launch_bounds__((SPLIT ? 96 : 64) * NS, 1) gf_ws_gray_kernel(c
     else { band = rem / a.nstrips; strip = rem % a.nstrips; hbw = a.hb; }
     const int y0 = a.out_y0 + band * hbw;
     const int y1 = y0 + hbw < a.out_y0 + a.out_rows ? y0 + hbw : a.out_y0 + a.out_rows;
-    constexpr bool TM = G::TMEM && !SPLIT;           // the producers keep their input rows in tensor memory
+    constexpr bool TM = G::TMEM;           // the producers keep their input rows in tensor memory
     __shared__ unsigned tm_base;
     if (TM && warp == 0) gf_tm_alloc(&tm_base, G::TM_ALLOC);
     if (threadIdx.x < 2 * NS) ctrl[threadIdx.x] = 0;
@@ -950,50 +850,24 @@ __global__ void __launch_bounds__((SPLIT ? 96 : 64) * NS, 1) gf_ws_gray_kernel(c
     const int em = (in_l && in_r) ? 0 : ((xl == -G::HALO && in_r) ? 1 : ((in_l && xl + G::WIN == a.width + G::HALO) ? 2 : 3));
     // producer k reaches the lanes of quarter k % 4; k and k + 4 split its columns
     const unsigned tm = TM ? tm_base + ((unsigned)(32 * (k % 4)) << 16) + (unsigned)(k / 4 * G::KW * G::TM_ROW) : 0u;
-#define GF_WS_S1(ROLE)                                                                                                   \
-    do {                                                                                                                 \
-        if (em == 0) gf_ws_stage1<R, K, NS, TRUNC, 0, ROLE>(a, pl, k, lane, f, xl, out_lo, out_hi, smem, ctrl, tm);        \
-        else if (em == 1) gf_ws_stage1<R, K, NS, TRUNC, 1, ROLE>(a, pl, k, lane, f, xl, out_lo, out_hi, smem, ctrl, tm);   \
-        else if (em == 2) gf_ws_stage1<R, K, NS, TRUNC, 2, ROLE>(a, pl, k, lane, f, xl, out_lo, out_hi, smem, ctrl, tm);   \
-        else gf_ws_stage1<R, K, NS, TRUNC, 3, ROLE>(a, pl, k, lane, f, xl, out_lo, out_hi, smem, ctrl, tm);                \
-    } while (0)
-    if (SPLIT) {
-        if (part == 0) GF_WS_S1(1);
-        else if (part == 1) GF_WS_S1(2);
-        else gf_ws_stage2<R, K, NS, TRUNC>(a, pl, k, lane, f, xl, out_lo, out_hi, smem, ctrl);
-    } else {
-        if (part == 0) {
-            GF_WS_S1(0);
-            if (TM && warp == 0) {     // free the history once every producer of the CTA (k < pl.n; the others returned) has finished
-                const unsigned long long* bars = reinterpret_cast<const unsigned long long*>(const_cast<const int*>(ctrl) + 16);
-                for (int s = 0; s < pl.n; ++s) gf_ws_bar_wait(bars + s * G::NBAR + 2 * G::RING, 0);
-                gf_tm_fence_after();
-                gf_tm_dealloc(tm_base, G::TM_ALLOC);
-            }
+    if (part == 0) {
+        if (em == 0) gf_ws_stage1<R, K, NS, TRUNC, 0>(a, pl, k, lane, f, xl, out_lo, out_hi, smem, ctrl, tm);
+        else if (em == 1) gf_ws_stage1<R, K, NS, TRUNC, 1>(a, pl, k, lane, f, xl, out_lo, out_hi, smem, ctrl, tm);
+        else if (em == 2) gf_ws_stage1<R, K, NS, TRUNC, 2>(a, pl, k, lane, f, xl, out_lo, out_hi, smem, ctrl, tm);
+        else gf_ws_stage1<R, K, NS, TRUNC, 3>(a, pl, k, lane, f, xl, out_lo, out_hi, smem, ctrl, tm);
+        if (TM && warp == 0) {     // free the history once every producer of the CTA (k < pl.n; the others returned) has finished
+            const unsigned long long* bars = reinterpret_cast<const unsigned long long*>(const_cast<const int*>(ctrl) + 16);
+            for (int s = 0; s < pl.n; ++s) gf_ws_bar_wait(bars + s * G::NBAR + 2 * G::RING, 0);
+            gf_tm_fence_after();
+            gf_tm_dealloc(tm_base, G::TM_ALLOC);
         }
-        else gf_ws_stage2<R, K, NS, TRUNC>(a, pl, k, lane, f, xl, out_lo, out_hi, smem, ctrl);
     }
-#undef GF_WS_S1
+    else gf_ws_stage2<R, K, NS, TRUNC>(a, pl, k, lane, f, xl, out_lo, out_hi, smem, ctrl);
 }
 
 // ---- host side --------------------------------------------------------------------------------------
 #ifndef GF_NO_HOST
 // Longest sub-band a stream walks with sliding (add / subtract) vertical sums before the band is cut.
-// Whether gf_guided_gray & co. take this kernel when they can (option GF_WS overrides)
-#ifndef GF_WS_DEFAULT
-#define GF_WS_DEFAULT 0
-#endif
-// Producer split over two warps (option GF_WS_SPLIT1 overrides)
-#ifndef GF_WS_SPLIT1_DEFAULT
-#define GF_WS_SPLIT1_DEFAULT 0
-#endif
-#ifndef GF_WS_WITH_SPLIT1
-#ifdef GF_CPU_EMU
-#define GF_WS_WITH_SPLIT1 1
-#else
-#define GF_WS_WITH_SPLIT1 0
-#endif
-#endif
 #ifndef GF_WS_MAX_SUB
 #define GF_WS_MAX_SUB 512
 #endif
@@ -1059,28 +933,10 @@ static const char* gf_ws_launch(const Job& j)
     }
     a.hb = bd.hb; a.nbands = bd.nbands; a.hb_e = bd.hb_e; a.nbands_e = bd.nbands_e;
     const long items = (a.nbands_e > 0 ? 2L * a.nbands_e + (long)(a.nstrips - 2) * a.nbands : (long)a.nstrips * a.nbands) * j.count;
-    // The split-producer kernels (measured 20-90 % slower, DESIGN.md section 3.3) are compiled only into the emulator
-    // build (their hand-off logic stays under test) and into -DGF_WS_WITH_SPLIT1=1 experiment builds.
-#if GF_WS_WITH_SPLIT1
-    const bool split = GF_KNOB("GF_WS_SPLIT1", GF_WS_SPLIT1_DEFAULT) != 0;
-#else
-    const bool split = false;
-#endif
-    dim3 grid((unsigned)items), block((split ? 96 : 64) * NS);
-    const char* e;
-#define GF_WS_GO(TR, SP)                                                        \
-    do {                                                                        \
-        auto kf = gf_ws_gray_kernel<R, K, NS, TR, SP>;                          \
-        if ((e = gf_rt_set_smem(kf, G::smem_bytes))) return e;                  \
-        GF_LAUNCH(kf, grid, block, G::smem_bytes, j.stream, a);                 \
-    } while (0)
-#if GF_WS_WITH_SPLIT1
-    if (j.border == GF_TRUNCATE) { if (split) GF_WS_GO(true, true); else GF_WS_GO(true, false); }
-    else { if (split) GF_WS_GO(false, true); else GF_WS_GO(false, false); }
-#else
-    if (j.border == GF_TRUNCATE) GF_WS_GO(true, false); else GF_WS_GO(false, false);
-#endif
-#undef GF_WS_GO
+    dim3 grid((unsigned)items), block(64 * NS);
+    auto kf = j.border == GF_TRUNCATE ? gf_ws_gray_kernel<R, K, NS, true> : gf_ws_gray_kernel<R, K, NS, false>;
+    if (const char* e = gf_rt_set_smem(kf, G::smem_bytes)) return e;
+    GF_LAUNCH(kf, grid, block, G::smem_bytes, j.stream, a);
     return gf_rt_launch_error();
 }
 
@@ -1093,7 +949,7 @@ static const char* gf_ws_try(const Job& j, bool* done, const char** name)
     // ... and single frames of up to 12 Mpx at r = 8 (the headline shape: 62.4 us against 65.7 us at 4K, 35.5 against 37.1 at
     // 1080p; above that size gf_s8's steady state wins: 8K 192 vs 170 us, profiles/r2_ws_matrix_final.jsonl, r2_ws_pen.jsonl)
     const bool small_r8 = j.r == 8 && j.count == 1 && (int64_t)j.width * j.out_rows <= 12000000;
-    if (j.color || !GF_KNOB("GF_WS", (j.A.ptr || small_r8) ? 1 : GF_WS_DEFAULT) || GF_KNOB("GF_DISABLE_FAST", 0) ||
+    if (j.color || !GF_KNOB("GF_WS", (j.A.ptr || small_r8) ? 1 : 0) || GF_KNOB("GF_DISABLE_FAST", 0) ||
         GF_KNOB("GF_DISABLE_S8", 0))          // (GF_DISABLE_S8 = "first-generation kernels only" in the differential tests)
         return nullptr;
     const int force_k = GF_KNOB("GF_WS_K", 0);

@@ -474,27 +474,13 @@ def test_host_entry_and_dropin_program(be, tmp_path):
 @pytest.mark.parametrize("world,r", [(2, 8), (3, 16), (5, 4)])
 def test_run_strips_one_gpu(be, world, r):
     """gf_run_strips with every "rank" on this one GPU (peer pointers = plain device pointers): the halo pull, the
-    strip geometry and the stitched result -- the multi-GPU form of the same call runs in tests/test_gpu_dist.py."""
+    strip geometry and the stitched result -- the multi-GPU form of the same call runs in tests/test_gpu_dist.py.
+    Two launches per rank: the halo pull, then the whole strip."""
     I, p = synth_pair(1500, 1408, seed=23)
+    n0 = be.api.launch_count()
     q = be.run_strips(I, p, world, r, 1e-2, 0)
+    assert be.api.launch_count() - n0 == 2 * world
     assert np.abs(q - C.guided_gray_f64(I, p, r, 1e-2, 0, NT)).max() <= TOL
-
-
-def test_run_strips_exchange_behind_the_kernel(be, knob):
-    """gf_run_strips with GF_STRIP_OVERLAP=1: the rows that read no halo on the caller's stream at once, the pull and the
-    2r seam rows on a side stream (three launches per rank instead of two); same pixels as pull-then-launch to the
-    rounding of the running sums."""
-    I, p = synth_pair(2400, 2048, seed=24)
-    knob(be, "GF_STRIP_OVERLAP", 1)
-    n0 = be.api.launch_count()
-    q = be.run_strips(I, p, 2, 16, 1e-2, 0)
-    assert be.api.launch_count() - n0 == 6
-    knob(be, "GF_STRIP_OVERLAP", 0)
-    n0 = be.api.launch_count()
-    q1 = be.run_strips(I, p, 2, 16, 1e-2, 0)
-    assert be.api.launch_count() - n0 == 4
-    assert np.abs(q - q1).max() <= 1e-5
-    assert np.abs(q - C.guided_gray_f64(I, p, 16, 1e-2, 0, NT)).max() <= TOL
 
 
 def test_large_radius_4k_scan_path(be, knob):

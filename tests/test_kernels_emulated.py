@@ -375,12 +375,9 @@ def test_class_run_planar_path(be, knob):
     ((60, 480), 4, 1, 8),
     ((40, 728), 4, 0, 8),
 ])
-@pytest.mark.parametrize("split", [0, 1])
-def test_gray_ws(be, shape, r, border, k, split, knob):
-    """split = 1: the producer of every stream is two warps (sums + solve / products) that meet in the ring slot."""
+def test_gray_ws(be, shape, r, border, k, knob):
     knob(be, "GF_WS", 1)
     knob(be, "GF_WS_K", k)
-    knob(be, "GF_WS_SPLIT1", split)
     I, p = synth_pair(*shape, seed=81, kind="structured")
     w = shape[1]
     q, A, B = be.guided_gray(I, p, r, 1e-2, border, want_ab=True, pad=(-w) % 8 if k % 8 == 0 else 0)   # K = 8: 32-byte rows
@@ -428,39 +425,21 @@ def test_gray_ws_strip_and_batch(be, knob):
 @pytest.mark.parametrize("world,border", [(2, 0), (3, 1), (4, 2)])
 def test_run_strips_pulls_halos(be, world, border):
     """gf_run_strips (SURVEY 8(b)): every rank's buffers hold its own rows only; the call pulls the 2r halo rows out of
-    the neighbours' buffers and filters the strip -- the stitched result equals the single-image result."""
+    the neighbours' buffers and filters the strip -- the stitched result equals the single-image result.  One launch
+    per rank: the pull, then the whole strip (the emulator's pull is a memcpy)."""
     I, p = synth_pair(97, 130, seed=91, kind="structured")
+    n0 = be.api.launch_count()
     q = be.run_strips(I, p, world, 3, 1e-2, border)
+    assert be.api.launch_count() - n0 == world
     assert np.abs(q - O.guided_filter_gray(I, p, 3, 1e-2, border, np.float64)).max() <= TOL
 
 
-@pytest.mark.parametrize("border", [0, 1, 2])
-def test_run_strips_exchange_behind_the_kernel(be, border, knob):
-    """gf_run_strips with GF_STRIP_OVERLAP=1: rows that read no halo are filtered at once, the 2r seam rows at either
-    end after the pull (three jobs instead of one) -- same result as the single image and as pull-then-launch."""
-    knob(be, "GF_STRIP_OVERLAP", 1)
-    knob(be, "GF_STRIP_MIN_MAIN_ROWS", 16)       # the 80-row strips of this test count as tall
-    I, p = synth_pair(240, 512, seed=93, kind="structured")
-    n0 = be.api.launch_count()
-    q = be.run_strips(I, p, 3, 4, 1e-2, border)
-    assert be.api.launch_count() - n0 == 7       # (main + seam) + (main + 2 seams) + (main + seam); the emulator's pull is a memcpy
-    assert np.abs(q - O.guided_filter_gray(I, p, 4, 1e-2, border, np.float64)).max() <= TOL
-    knob(be, "GF_STRIP_OVERLAP", 0)              # the sequential form: pull, then one launch
-    n0 = be.api.launch_count()
-    q1 = be.run_strips(I, p, 3, 4, 1e-2, border)
-    assert be.api.launch_count() - n0 == 3
-    assert np.abs(q - q1).max() <= 1e-5          # different band boundaries: running sums round differently
-
-
-def test_run_strips_destination_right_before_the_guide(be, knob):
+def test_run_strips_destination_ending_where_the_guide_begins(be):
     """A strip's destination holds its own rows, its guide buffer 2r halo rows more on either side.  A destination that
-    ends where the guide buffer begins (one allocation) does not overlap it: the strip is still split into the main
-    job and two seam jobs, without an in-place temporary.  (The overlap test used to give the destination the buffer's
-    row count, so whether the split happened depended on where the allocator put the planes.)"""
+    ends where the guide buffer begins (one allocation) does not overlap it: the strip is filtered in one launch (the
+    emulator's pull is a memcpy) and its rows equal the single-image result."""
     from cudaimageprocessing_b200._capi import StripPeer
     import ctypes
-    knob(be, "GF_STRIP_OVERLAP", 1)
-    knob(be, "GF_STRIP_MIN_MAIN_ROWS", 16)
     H, w, r, border = 240, 512, 4, 2
     y0, rows, t = 80, 80, 8                      # the middle strip of three; t = 2r halo rows above and below
     I, p = synth_pair(H, w, seed=94, kind="structured")
@@ -474,7 +453,7 @@ def test_run_strips_destination_right_before_the_guide(be, knob):
     n0 = be.api.launch_count()
     be.api.call("gf_run_strips", be.ptr(gbuf), be.ptr(sbuf), be.ptr(q), w, H, y0, rows, w, w, w, r, 1e-2, border,
                 ctypes.byref(up), ctypes.byref(dn), None)
-    assert be.api.launch_count() - n0 == 3       # main + 2 seams; the emulator's pull is a memcpy
+    assert be.api.launch_count() - n0 == 1
     assert np.abs(q - O.guided_filter_gray(I, p, r, 1e-2, border, np.float64)[y0:y0 + rows]).max() <= TOL
 
 
