@@ -1038,6 +1038,53 @@ int gf_box_filter(const float* src, float* dst, int width, int height, int chann
 
 }  // extern "C"
 
+// Does dst (rows of dn elements, row stride ds) share memory with the input `in` (rows of in_n elements, stride is)
+// without being exactly that input (same pointer, stride and row length)?  Planes that share a row stride may interleave
+// their rows (columns side by side) without sharing an element.
+template <typename T>
+static bool fgf_partial_overlap(const T* in, int64_t is, int64_t in_n, const T* dst, int64_t ds, int64_t dn, int height)
+{
+    if (in == dst && is == ds && in_n == dn) return false;
+    if (!(dst < in + (int64_t)(height - 1) * is + in_n && in < dst + (int64_t)(height - 1) * ds + dn)) return false;
+    if (is != ds) return true;
+    const int64_t c = (((intptr_t)dst - (intptr_t)in) / (int64_t)sizeof(T) % is + is) % is;   // column offset
+    return !(c >= in_n && c + dn <= is);
+}
+
+// mean_a, mean_b of the fast filters: gf_box_kernel over `frames` low-res planes of `ch` interleaved channels (1 or 4), on
+// CTAs of 128 columns and bands short enough for 16 CTAs per SM.  A CTA waits for one row load per step, so its time is
+// (hb + 2r) load latencies: gf_box_filter's own plan (one strip of up to 1024 columns, bands of at least 16 rows)
+// measured 19-22 us a plane at 4K s = 4 and 46-58 us at 8K s = 4.  Radii that leave fewer than 32 columns go through
+// gf_box_filter, one call per plane.
+static int fgf_box(const float* in, float* out, int w, int h, int ch, int64_t stride, int64_t plane, int frames, int r,
+                   int border, void* stream)
+{
+    const int win = 128, wc = win - 2 * r;
+    if (wc < 32) {
+        for (int f = 0; f < frames; ++f)
+            if (int rc = gf_box_filter(in + f * plane, out + f * plane, w, h, ch, stride, stride, r, border, stream)) return rc;
+        return GF_OK;
+    }
+    Job jb;
+    jb.width = w; jb.height = h; jb.buf_rows = h; jb.out_rows = h;
+    jb.r = r; jb.border = border; jb.stream = stream;
+    jb.src = jb.guide = Plane{in, stride, plane, ch, 0};
+    jb.dst = Plane{out, stride, plane, ch, 0};
+    jb.A = jb.B = Plane{nullptr, 0, 0, 1, 0};
+    GfArgs a = mk_args(jb);
+    int sms = 148, mj = 0, mn = 0;
+    gf_rt_device_info(&sms, &mj, &mn);
+    const int nstrips = div_up(w, wc);
+    const int hb = div_up(h, div_up(16 * sms, nstrips * frames));
+    a.wc = wc; a.hb = hb;
+    dim3 grid(nstrips, div_up(h, hb), frames), block(win);
+    if (ch == 1) { auto k = gf_box_kernel<1>; GF_LAUNCH(k, grid, block, (win + 32) * sizeof(float), stream, a); }
+    else { auto k = gf_box_kernel<4>; GF_LAUNCH(k, grid, block, 4 * (win + 32) * sizeof(float), stream, a); }
+    if (const char* e = gf_rt_launch_error()) return fail(GF_ERR_CUDA, "gf_box_kernel launch: %s", e);
+    g_launches++;
+    return GF_OK;
+}
+
 // Fast guided filter (He & Sun 2015; gf_fgf.cuh): a and b solved on I and p subsampled s times with radius r/s by the
 // library's own gray a/b job, mean_a and mean_b by the box kernel, the bilinear upsample fused into q = mean_a*I + mean_b.
 // T = float: gf_fast_guided_gray; T = unsigned char: gf_fast_guided_gray_u8, in the integer domain (eps' = 255^2 eps, the
@@ -1059,16 +1106,8 @@ static int fast_guided_gray(const T* guide, const T* src, T* dst, int width, int
         return fail(GF_ERR_INVALID, "%s: r = %d must be a non-negative multiple of s = %d (the low-res radius is r/s)", fn, r, s);
     if (!(eps >= 0.f)) return fail(GF_ERR_INVALID, "%s: eps must be >= 0", fn);
     if (border < 0 || border > 2) return fail(GF_ERR_INVALID, "%s: unknown border mode %d", fn, border);
-    // dst may BE an input (same pointer and stride): every full-resolution pass writes only the pixels it has just read.
-    // Planes that share a row stride may interleave their rows (columns side by side) without sharing a pixel.
-    auto partial = [&](const T* in, int64_t is) {
-        if (in == dst && is == ds) return false;
-        if (!(dst < in + (int64_t)(height - 1) * is + width && in < dst + (int64_t)(height - 1) * ds + width)) return false;
-        if (is != ds) return true;
-        const int64_t c = (((intptr_t)dst - (intptr_t)in) / (int64_t)sizeof(T) % is + is) % is;   // column offset
-        return !(c >= width && c + width <= is);
-    };
-    if (partial(guide, gs) || partial(src, ss))
+    // dst may BE an input (same pointer and stride): every full-resolution pass writes only the pixels it has just read
+    if (fgf_partial_overlap(guide, gs, width, dst, ds, width, height) || fgf_partial_overlap(src, ss, width, dst, ds, width, height))
         return fail(GF_ERR_UNSUPPORTED, "%s: dst overlaps an input without being exactly that input (same pointer and stride)", fn);
 
     // the low-res a/b job, refused here if run_job would refuse it: the streaming kernels plan it, or the scan path takes it
@@ -1107,7 +1146,7 @@ static int fast_guided_gray(const T* guide, const T* src, T* dst, int width, int
     int rc = GF_OK;
     {
         GfFgfDownArgs<T> a;
-        a.I = guide; a.p = src; a.Is = Is; a.ps = ps; a.si = gs; a.sp = ss; a.sl = pitch;
+        a.I = guide; a.p = src; a.Is = Is; a.ps = ps; a.si = gs; a.sp = ss; a.sl = pitch; a.sls = pitch; a.spl = 0;
         a.width = width; a.height = height; a.ws = ws; a.hs = hs; a.s = s;
         dim3 grid(div_up(ws, GF_FGF_DOWN_THREADS), hs < 65535 ? hs : 65535), block(GF_FGF_DOWN_THREADS);
         auto k = gf_fgf_down_kernel<T>;
@@ -1121,33 +1160,9 @@ static int fast_guided_gray(const T* guide, const T* src, T* dst, int width, int
         rc = run_job(lo);
         lo_name = g_kernel;
     }
-    // mean_a, mean_b: gf_box_kernel on CTAs of 128 columns and bands short enough for 16 CTAs per SM.  A CTA waits for
-    // one row load per step, so its time is (hb + 2r) load latencies: gf_box_filter's own plan (one strip of up to 1024
-    // columns, bands of at least 16 rows) measured 19-22 us a plane at 4K s = 4 and 46-58 us at 8K s = 4.  Radii that
-    // leave fewer than 32 columns go through gf_box_filter.
-    auto box = [&](const float* in, float* out) -> int {
-        const int win = 128, wc = win - 2 * rl;
-        if (wc < 32) return gf_box_filter(in, out, ws, hs, 1, pitch, pitch, rl, border, stream);
-        Job jb = lo;
-        jb.src = jb.guide = Plane{in, pitch, 0, 1, 0};
-        jb.dst = Plane{out, pitch, 0, 1, 0};
-        jb.A = jb.B = Plane{nullptr, 0, 0, 1, 0};
-        GfArgs a = mk_args(jb);
-        int sms = 148, mj = 0, mn = 0;
-        gf_rt_device_info(&sms, &mj, &mn);
-        const int nstrips = div_up(ws, wc);
-        const int hb = div_up(hs, div_up(16 * sms, nstrips));
-        a.wc = wc; a.hb = hb;
-        dim3 grid(nstrips, div_up(hs, hb), 1), block(win);
-        auto k = gf_box_kernel<1>;
-        GF_LAUNCH(k, grid, block, (win + 32) * sizeof(float), stream, a);
-        if (const char* e = gf_rt_launch_error()) return fail(GF_ERR_CUDA, "gf_box_kernel launch: %s", e);
-        g_launches++;
-        return GF_OK;
-    };
     // I_s and p_s have been read by the a/b job (stream order): they take mean_a and mean_b
-    if (rc == GF_OK) rc = box(A, Is);
-    if (rc == GF_OK) rc = box(B, ps);
+    if (rc == GF_OK) rc = fgf_box(A, Is, ws, hs, 1, pitch, 0, 1, rl, border, stream);
+    if (rc == GF_OK) rc = fgf_box(B, ps, ws, hs, 1, pitch, 0, 1, rl, border, stream);
     if (rc == GF_OK) {
         GfFgfApplyArgs<T> a;
         a.I = guide; a.q = dst; a.ma = Is; a.mb = ps; a.si = gs; a.sq = ds; a.sl = pitch;
@@ -1181,6 +1196,118 @@ int gf_fast_guided_gray_u8(const unsigned char* guide, const unsigned char* src,
 {
     return fast_guided_gray(guide, src, dst, width, height, guide_stride, src_stride, dst_stride, r, eps, s, border, stream,
                             "gf_fast_guided_gray_u8", "fgf_u8/");
+}
+
+// Fast guided filter with a colour guide (gf_fgf.cuh): I_s (3 channels) and p_s (C planes) by gf_fgf_down_kernel, a and b
+// of every low-res pixel by gf_fgf_color_ab_kernel, their box means by gf_box_kernel<4> with the source channels as
+// frames, and gf_fgf_up_apply_color_kernel.  Four launches for any C.
+int gf_fast_guided_color(const float* guide, const float* src, float* dst, int width, int height, int C, int64_t guide_stride,
+                         int64_t src_stride, int64_t dst_stride, int r, float eps, int s, int border, void* stream)
+{
+    const char* fn = "gf_fast_guided_color";
+    if (C != 1 && C != 3) return fail(GF_ERR_UNSUPPORTED, "%s: Do not support channel: 3, %d", fn, C);
+    if (!guide || !src || !dst) return fail(GF_ERR_INVALID, "%s: null pointer", fn);
+    if (width <= 0 || height <= 0) return fail(GF_ERR_INVALID, "%s: non-positive size %dx%d", fn, width, height);
+    const int64_t gs = or_packed(guide_stride, width, 3), ss = or_packed(src_stride, width, C), ds = or_packed(dst_stride, width, C);
+    if (gs < 3 * (int64_t)width || ss < (int64_t)C * width || ds < (int64_t)C * width)
+        return fail(GF_ERR_INVALID, "%s: row stride smaller than a row", fn);
+    if (s < 1 || s > GF_FGF_MAX_S) return fail(GF_ERR_INVALID, "%s: subsampling factor s = %d outside [1, %d]", fn, s, GF_FGF_MAX_S);
+    if (r < 0 || r % s != 0)
+        return fail(GF_ERR_INVALID, "%s: r = %d must be a non-negative multiple of s = %d (the low-res radius is r/s)", fn, r, s);
+    if (!(eps >= 0.f)) return fail(GF_ERR_INVALID, "%s: eps must be >= 0", fn);
+    if (border < 0 || border > 2) return fail(GF_ERR_INVALID, "%s: unknown border mode %d", fn, border);
+    // dst may BE the source, or with C = 3 the guide (same pointer and stride): the down kernel alone reads the source,
+    // and the apply kernel reads the guide of a pixel before it writes that pixel
+    if (fgf_partial_overlap(guide, gs, 3 * (int64_t)width, dst, ds, (int64_t)C * width, height) ||
+        fgf_partial_overlap(src, ss, (int64_t)C * width, dst, ds, (int64_t)C * width, height))
+        return fail(GF_ERR_UNSUPPORTED, "%s: dst overlaps an input without being exactly the source or, with 3 source channels, "
+                                        "the guide (same pointer and stride)", fn);
+    Job j;
+    j.width = width; j.height = height; j.buf_rows = height; j.out_rows = height;
+    j.r = r; j.eps = eps; j.border = border; j.stream = stream; j.color = true;
+    j.guide = Plane{guide, gs, 0, 3, 0};
+    j.A = j.B = Plane{nullptr, 0, 0, 1, 0};
+    if (s == 1) {                                            // the exact filter: gf_guided_color
+        GenericCfg c;
+        if (plan_generic(j, 4 * r, 4 * r, GfColorModel::NQ1 + GfColorModel::NQ2, GfColorModel::NQ2, &c) != GF_OK)
+            return fail(GF_ERR_UNSUPPORTED, "%s: s = 1 runs gf_guided_color, whose kernels do not take r = %d at width %d", fn, r, width);
+        Job js[3];
+        for (int k = 0; k < C; ++k) {
+            js[k] = j;
+            js[k].src = Plane{src, ss, 0, C, k};
+            js[k].dst = Plane{dst, ds, 0, C, k};
+        }
+        const int rc = run_jobs(js, C);
+        if (rc == GF_OK) { g_kernel_fgf = std::string("fgfc/") + g_kernel; g_kernel = g_kernel_fgf.c_str(); }
+        return rc;
+    }
+    const int ws = div_up(width, s), hs = div_up(height, s), rl = r / s;
+    if (rl > GF_FGF_MAX_RL)
+        return fail(GF_ERR_UNSUPPORTED, "%s: the low-res radius r/s = %d is above %d, the most the low-res kernels take", fn, rl, GF_FGF_MAX_RL);
+
+    // pool scratch, 16-byte rows: I_s (3 channels), the C planes of p_s, then per channel a 4-channel plane of (a, b) and
+    // one of their box means
+    const int64_t p3 = round_up(3 * ws, 4), p1 = round_up(ws, 4), p4 = 4 * (int64_t)ws;
+    const int64_t n_is = p3 * hs, n_ps = p1 * hs, n_ab = p4 * hs;
+    const size_t bytes = (size_t)(n_is + C * (n_ps + 2 * n_ab)) * sizeof(float);
+    void* scratch = nullptr;
+    if (const char* e = gf_rt_alloc_async(&scratch, bytes, stream)) return fail(GF_ERR_NOMEM, "%s: low-res scratch (%zu bytes): %s", fn, bytes, e);
+    float* Is = (float*)scratch;
+    float* ps = Is + n_is;
+    float* AB = ps + C * n_ps;
+    float* M = AB + C * n_ab;
+    int sms = 148, mj = 0, mn = 0;
+    gf_rt_device_info(&sms, &mj, &mn);
+    int rc = GF_OK;
+    {
+        GfFgfDownArgs<float> a;
+        a.I = guide; a.p = src; a.Is = Is; a.ps = ps; a.si = gs; a.sp = ss; a.sl = p1; a.sls = p3; a.spl = n_ps;
+        a.width = width; a.height = height; a.ws = ws; a.hs = hs; a.s = s;
+        dim3 grid(div_up(ws, GF_FGF_DOWN_THREADS), hs < 65535 ? hs : 65535), block(GF_FGF_DOWN_THREADS);
+        if (C == 1) { auto k = gf_fgf_down_kernel<float, 3, 1>; GF_LAUNCH(k, grid, block, 0, stream, a); }
+        else { auto k = gf_fgf_down_kernel<float, 3, 3>; GF_LAUNCH(k, grid, block, 0, stream, a); }
+        if (const char* e = gf_rt_launch_error()) rc = fail(GF_ERR_CUDA, "gf_fgf_down_kernel launch: %s", e);
+        else g_launches++;
+    }
+    if (rc == GF_OK) {   // a and b: CTAs of 128 low-res columns, bands short enough for 16 CTAs per SM, as fgf_box plans
+        Job lo;
+        lo.width = ws; lo.height = hs; lo.buf_rows = hs; lo.out_rows = hs;
+        lo.r = rl; lo.eps = eps; lo.border = border; lo.stream = stream; lo.color = true;
+        lo.guide = Plane{Is, p3, 0, 3, 0};
+        lo.src = Plane{ps, p1, n_ps, 1, 0};
+        lo.dst = Plane{AB, p4, n_ab, 4, 0};
+        lo.A = lo.B = Plane{nullptr, 0, 0, 1, 0};
+        GfArgs a = mk_args(lo);
+        const int wc = GF_FGF_AB_THREADS - 2 * rl, nstrips = div_up(ws, wc);
+        const int hb = div_up(hs, div_up(16 * sms, nstrips * C));
+        a.wc = wc; a.hb = hb;
+        dim3 grid(nstrips, div_up(hs, hb), C), block(GF_FGF_AB_THREADS);
+        auto k = gf_fgf_color_ab_kernel;
+        GF_LAUNCH(k, grid, block, 0, stream, a);
+        if (const char* e = gf_rt_launch_error()) rc = fail(GF_ERR_CUDA, "gf_fgf_color_ab_kernel launch: %s", e);
+        else g_launches++;
+    }
+    if (rc == GF_OK) rc = fgf_box(AB, M, ws, hs, 4, p4, n_ab, C, rl, border, stream);
+    if (rc == GF_OK) {
+        GfFgfApplyColorArgs a;
+        a.I = guide; a.q = dst; a.m = M; a.si = gs; a.sq = ds; a.sl = p4; a.pl = n_ab;
+        a.width = width; a.height = height; a.ws = ws; a.hs = hs; a.s = s;
+        const bool vec = width % 4 == 0 && gs % 4 == 0 && ds % 4 == 0 && !((uintptr_t)guide & 15) && !((uintptr_t)dst & 15);
+        const int ty = div_up(height, GF_FGF_TY);
+        dim3 grid(div_up(width, GF_FGF_TX), ty < 65535 ? ty : 65535), block(256);
+        if (C == 1) {
+            if (vec) { auto k = gf_fgf_up_apply_color_kernel<true, 1>; GF_LAUNCH(k, grid, block, 0, stream, a); }
+            else { auto k = gf_fgf_up_apply_color_kernel<false, 1>; GF_LAUNCH(k, grid, block, 0, stream, a); }
+        } else {
+            if (vec) { auto k = gf_fgf_up_apply_color_kernel<true, 3>; GF_LAUNCH(k, grid, block, 0, stream, a); }
+            else { auto k = gf_fgf_up_apply_color_kernel<false, 3>; GF_LAUNCH(k, grid, block, 0, stream, a); }
+        }
+        if (const char* e = gf_rt_launch_error()) rc = fail(GF_ERR_CUDA, "gf_fgf_up_apply_color_kernel launch: %s", e);
+        else g_launches++;
+    }
+    gf_rt_free_async(scratch, stream);
+    if (rc == GF_OK) g_kernel = "fgfc/color_ab";
+    return rc;
 }
 
 static int pointwise(int op, const float* i0, const float* i1, const float* i2, const float* i3, float* out, int width,

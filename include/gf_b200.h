@@ -113,6 +113,30 @@ int gf_fast_guided_gray_u8(const unsigned char* guide, const unsigned char* src,
                            int64_t guide_stride, int64_t src_stride, int64_t dst_stride, int r, float eps, int s, int border,
                            void* stream);
 
+/* The fast guided filter with a colour guide: a 3-channel interleaved float32 guide (CV_32FC3) and a source and
+   destination of src_channels = 1 or 3 interleaved channels, any width, height, stride and alignment.  An approximation
+   of gf_guided_color whose full-resolution cost does not grow with the radius: with hs = ceil(height/s), ws =
+   ceil(width/s),
+     - I_s (3 channels), p_s (src_channels channels): the per-channel mean of the in-image pixels of every s x s block;
+     - for every source channel c: a (3-vector) and b of the colour guided filter of gf_guided_color on (I_s, p_s[c]) at
+       radius r/s, with eps and border, and mean_a (3 planes), mean_b their box means at radius r/s with that border;
+     - q_c = sum_k up(mean_a_k) * I_k + up(mean_b), up the bilinear upsample of gf_fast_guided_gray.
+   s = 1 is gf_guided_color, and the call runs it.  Four kernel launches for s >= 2 whatever src_channels is (the source
+   channels are frames of each launch).  dst may be exactly the source, and with src_channels = 3 exactly the guide
+   (same pointer and stride), so guide == src == dst filters an image in place without a temporary.  Strides in floats,
+   0 = tightly packed (3 width for the guide, src_channels width for src and dst).  Low-res scratch comes from the
+   library's stream-ordered pool.
+   GF_ERR_INVALID: a null pointer, a non-positive size, a stride smaller than a row, s outside [1, 32], r < 0 or r not a
+   multiple of s, eps < 0 or NaN, an unknown border.  GF_ERR_UNSUPPORTED: src_channels not 1 or 3; dst overlapping an
+   input without being exactly the source or (src_channels = 3) the guide; s >= 2 with r/s > 48 (the low-res kernels run
+   CTAs of 128 low-res columns, at least 32 of them outputs beside the 2 r/s halo columns); s = 1 with r > 248 and
+   width + 4r > 1024 (the radius gf_guided_color's streaming kernel cannot hold).  Every refusal comes before anything is
+   allocated or launched.  gf_last_kernel() gives "fgfc/color_ab" (the low-res a/b kernel), for s = 1 "fgfc/" followed
+   by the kernel gf_guided_color ran. */
+int gf_fast_guided_color(const float* guide3, const float* src, float* dst, int width, int height, int src_channels,
+                         int64_t guide_stride, int64_t src_stride, int64_t dst_stride,
+                         int r, float eps, int s, int border, void* stream);
+
 /* Colour guide (3 interleaved channels), `src_channels` (1 or 3) source/destination channels.
    a = (Sigma + eps U)^-1 cov(I, p), b = mean(p) - a.mean(I), q = mean(a).I + mean(b). */
 int gf_guided_color(const float* guide3, const float* src, float* dst, int width, int height,
